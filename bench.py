@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- converged MPC solves/sec of the batched solver (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (cold-start guess kernel + persistent solver kernel) over
@@ -15,12 +15,16 @@ e2e     = same metric through the host-pointer C ABI call (igt_solve_host): pinn
           H2D of the inputs and D2H of x, u, cost, viol, status, iters inside the timed region
 --impl reference: the reference's own solver (CasADi/IPOPT) cannot run offline, so this arm times
           the oracle's fp64 C restatement of the same NLP/algorithm on all host cores.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned (x, u, cost,
+          viol, status, iters) as DIR/<name>.npy in float64, so that two builds can be compared output
+          for output on the same seeded inputs (see dump_outputs).
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -59,7 +63,7 @@ def make_problems(name, rank, world=1, scaling=None):
     scaling = scaling or default_scaling
     strong = scaling == "strong"
     seed = {"cfg4_frenet_65536": 4}.get(name, 2026) + (0 if strong else 1000 * rank)      # SURVEY 8(d): seeds 2026+sc / 4
-    cache = os.path.join("/tmp", "igt_bench_%s_s%d.npz" % (name, seed))
+    cache = os.path.join(tempfile.gettempdir(), "igt_bench_%s_s%d.npz" % (name, seed))
     if os.path.exists(cache):
         d = np.load(cache)
         arrs = [d["x0"], d["up"], d["cv"], d["ob"], d["ctx"]]
@@ -86,6 +90,24 @@ def random_mlp(hidden=(128, 128), seed=2026):
     layers = [torch.nn.Linear(dims[i], dims[i + 1], dtype=torch.double) for i in range(len(dims) - 1)]
     weights = [(l.weight.detach().numpy().copy(), l.bias.detach().numpy().copy()) for l in layers]
     return dict(weights=weights, Wn=np.eye(6), mu_f=np.zeros(6), sigma_t=1.0, mu_t=0.0)
+
+
+DUMP_BYTES = 64 * 10**6     # --dump-outputs writes at most this much, .npy headers included
+
+
+def dump_outputs(out, directory):
+    """Write the solver's outputs (x[B,N+1,7], u[B,N,2], cost, viol, status, iters) as <directory>/<name>.npy in
+    float64.  When all B problems do not fit in DUMP_BYTES, the same fixed, seeded sample of problems is kept in every
+    array, and problem_index.npy says which ones they are."""
+    arrs = {k: v.cpu().numpy() for k, v in out.items()}
+    B = len(arrs["cost"])
+    row_bytes = 8 * (sum(a[0].size for a in arrs.values()) + 1)               # + 1: the problem's index
+    keep = min(B, (DUMP_BYTES - 128 * (len(arrs) + 1)) // row_bytes)
+    idx = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "problem_index.npy"), idx.astype(np.float64))
+    for name, a in arrs.items():
+        np.save(os.path.join(directory, name + ".npy"), a[idx].astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -197,7 +219,11 @@ def main():
     ap.add_argument("--no-closed-loop", action="store_true")
     ap.add_argument("--scaling", default=None, choices=["weak", "strong"],
                     help="default: the workload's own (cfg4 = strong: 65536 states in total, sharded)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -291,6 +317,8 @@ def main():
     dev_ms = float(sum(step_ms))
     status = out["status"].cpu().numpy()
     iters = out["iters"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     conv_per_step = int((status == 0).sum())
     acc_per_step = int((status == 6).sum())
     dev_ms_max, conv_all, iters_all, B_all = sharding.reduce_counters(dev_ms, conv_per_step, iters.sum(), B, device=dev)
@@ -312,7 +340,7 @@ def main():
     hin_np = [a.numpy() for a in hin]
     h2d = sum(a.nbytes for a in hin_np) + (hctx.numpy().nbytes if hctx is not None else 0)
     d2h = sum(v.nbytes for v in hout_np.values())
-    e2e_steps = max(3, min(args.steps, 5))
+    e2e_steps = args.steps
     solver.solve_batch(*hin_np, nn_ctx=None if hctx is None else hctx.numpy(), out=hout_np)
     barrier()
     t0 = time.perf_counter()

@@ -28,6 +28,33 @@ def test_workload_table_and_sharded_problem_sets():
     assert bench.WORKLOADS["cfg4_frenet_65536"][4] == "strong" and bench.WORKLOADS[bench.DEFAULT_WORKLOAD][1] == 32768
 
 
+def test_dump_outputs_full_and_sampled(tmp_path, monkeypatch):
+    import torch
+    B, N = 50, 10
+    g = torch.Generator().manual_seed(1)
+    out = dict(x=torch.randn(B, N + 1, 7, generator=g, dtype=torch.float64), u=torch.randn(B, N, 2, generator=g, dtype=torch.float64),
+               cost=torch.randn(B, generator=g, dtype=torch.float64), viol=torch.rand(B, generator=g, dtype=torch.float64),
+               status=torch.arange(B, dtype=torch.int32) % 7, iters=torch.arange(B, dtype=torch.int32) + 5)
+    names = ["x", "u", "cost", "viol", "status", "iters", "problem_index"]
+    bench.dump_outputs(out, str(tmp_path / "full"))
+    for k in names[:-1]:
+        a = np.load(tmp_path / "full" / (k + ".npy"))
+        assert a.dtype == np.float64 and np.array_equal(a, out[k].numpy().astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "full" / "problem_index.npy"), np.arange(B))
+    row_bytes = 8 * ((N + 1) * 7 + N * 2 + 5)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20 * row_bytes + 128 * len(names))
+    for d in ("a", "b"):
+        bench.dump_outputs(out, str(tmp_path / d))
+    idx = np.load(tmp_path / "a" / "problem_index.npy")
+    assert len(idx) == 20 and np.all(np.diff(idx) > 0)
+    assert sum(os.path.getsize(tmp_path / "a" / (k + ".npy")) for k in names) <= bench.DUMP_BYTES
+    for k in names:
+        a, b = np.load(tmp_path / "a" / (k + ".npy")), np.load(tmp_path / "b" / (k + ".npy"))
+        assert np.array_equal(a, b)                                       # the same seeded sample every time
+        if k != "problem_index":
+            assert np.array_equal(a, out[k].numpy()[idx.astype(int)])
+
+
 def test_reference_arm_prints_one_json_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=600, cwd=ROOT)
