@@ -16,6 +16,7 @@ MAX_CINF, MAX_LAYERS = 128, 5
 PREC_F32, PREC_F64 = 0, 1
 STATUS_NAMES = {0: "converged", 1: "max_iter", 2: "x0_infeasible", 3: "reg_limit", 4: "line_search",
                 5: "stalled_infeasible", 6: "acceptable"}
+EPISODE_GT_MPC, EPISODE_OBCA = 1, 2   # mode bits of igt_episode_run_host
 STATUS_OK = (0, 6)      # converged, or stopped within the reference's own IPOPT tolerances (igt_mpc.h: IGT_STATUS_ACCEPTABLE)
 
 _dp = C.POINTER(C.c_double)

@@ -8,13 +8,14 @@
 //   warm start         previous inputs shifted by one                         common/utils.py:354-363
 //   plant              next state = x_sol[:, 1]                               evaluate.py:491-510
 //   brake fallback     a = a_min if v > 0 else 0, previous steering           evaluate.py:511-545
+//   OBCA mode          the obstacle's heading forecast as well                mpc.py:250-253 (MPC_Planner.update_predictions)
 // Same arithmetic as igt_mpc_int_b200/episode.py (the host-side numpy driver this replaces for large E).
 #pragma once
 #include "solver_core.cuh"
 
 namespace igt {
 
-constexpr int ROUTE_DESC = 12;   // x0, y0, t0x, t0y, sgn, b0, b1, r, exit_axis (0: x, 1: y, -1: none), exit_coord, pad, pad
+constexpr int ROUTE_DESC = 12;   // x0, y0, t0x, t0y, sgn, b0, b1, r, exit_axis (0: x, 1: y, -1: none), exit_coord, th0, flip
 
 // lane-centre (x, y) at arc length s (igt_mpc_int_b200/geometry.frenet2global_xy; closed form of common/utils.py:532-586)
 __host__ __device__ inline void route_xy(const double *rd, double s, double *x, double *y)
@@ -36,6 +37,17 @@ __host__ __device__ inline void route_xy(const double *rd, double s, double *x, 
     else if (rd[8] == 1.0) *y = rd[9];
 }
 
+// path heading at arc length s (the third output of igt_mpc_int_b200/geometry.frenet2global; geometry.route_heading):
+// th0 before the arc, th0 + sgn phi on it, th0 + sgn pi/2 after it.  th0 = rd[10] is stored rather than recovered from
+// (t0x, t0y) with atan2, so host and device headings are the same bits.
+__host__ __device__ inline double route_heading(const double *rd, double s)
+{
+    const double th0 = rd[10], sgn = rd[4], b0 = rd[5], b1 = rd[6], r = rd[7];
+    if (sgn == 0.0 || s < b0) return th0;
+    if (s <= b1) return th0 + sgn * ((s - b0) / r);
+    return th0 + sgn * (M_PI / 2);
+}
+
 struct EpisodeBufs {
     double *z, *u_prev;            // [B,7] [B,2] current state and last applied input
     const double *curv, *rd, *enc; // [B,3] [B,ROUTE_DESC] [B]
@@ -44,6 +56,7 @@ struct EpisodeBufs {
     int *prev_ok;                  // [B] the solve of the previous step succeeded
     double *z_cl, *u_cl;           // records [E,2,T+1,7] [E,2,T,2]
     int *solved;                   // [E,2,T]
+    double *obs_psi;               // [B,N+1] obstacle heading forecast (OBCA mode only, else null)
 };
 
 #ifdef __CUDACC__
@@ -56,6 +69,10 @@ __device__ inline void ca_step(double s, double v, double a, double dt, double *
 
 // before the solve of step t: thread b builds vehicle b's obstacle forecast (= forecast of vehicle b ^ 1), value-network
 // context, warm start.  px / pu: the plans of step t-1 (solver outputs [B,N+1,7] / [B,N,2]).
+// OBCA: also the obstacle's heading forecast eb.obs_psi[b, 0..N] (igt_mpc_int_b200/episode.py states the convention):
+// constant acceleration -- k = 0 the current psi, k >= 1 the route heading at s_k; V2V -- k < N the plan's psi at k + 1,
+// k = N the route heading at the extra step's s; abs() on routes 32 / 41 (rd[11]); 0 for a filtered obstacle.
+template <bool OBCA>
 __global__ void episode_pre_kernel(EpisodeBufs eb, int B, int N, double dt, int t, int gt, const double *px, const double *pu)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -63,30 +80,39 @@ __global__ void episode_pre_kernel(EpisodeBufs eb, int B, int N, double dt, int 
     const int o = b ^ 1;
     const double *zo = eb.z + 7 * o, *zb = eb.z + 7 * b, *rdo = eb.rd + ROUTE_DESC * o;
     double *obs = eb.obs + (long)b * (N + 1) * 2;
+    double *psi = OBCA ? eb.obs_psi + (long)b * (N + 1) : nullptr;
     double sN, vN;
     if (t > 0 && eb.prev_ok[o]) {                                  // V2V: the other vehicle's plan of t-1, shifted by one
         const double *pxo = px + (long)o * (N + 1) * 7, *puo = pu + (long)o * N * 2;
         for (int k = 0; k < N; k++) { obs[2 * k] = pxo[(k + 1) * 7 + IX]; obs[2 * k + 1] = pxo[(k + 1) * 7 + IY]; }
+        if (OBCA) for (int k = 0; k < N; k++) psi[k] = pxo[(k + 1) * 7 + IPSI];
         double s1, v1;
         ca_step(pxo[N * 7 + IS], pxo[N * 7 + IV], puo[(N - 1) * 2], dt, &s1, &v1);
         if (v1 > 5.0) ca_step(pxo[N * 7 + IS], pxo[N * 7 + IV], 0.0, dt, &s1, &v1);
         route_xy(rdo, s1, &obs[2 * N], &obs[2 * N + 1]);
+        if (OBCA) psi[N] = route_heading(rdo, s1);
         sN = s1; vN = v1;
     } else {                                                       // constant acceleration from the current state
         double a0 = eb.u_prev[2 * o];
         if (gt && t == 0) a0 = 0.09 * ((o & 1) + 1);               // evaluate.py:207-210
         double s = zo[IS], v = zo[IV];
         obs[0] = zo[IX]; obs[1] = zo[IY];
+        if (OBCA) psi[0] = zo[IPSI];
         for (int k = 0; k < N; k++) {
             ca_step(s, v, a0, dt, &s, &v);
             route_xy(rdo, s, &obs[2 * (k + 1)], &obs[2 * (k + 1) + 1]);
+            if (OBCA) psi[k + 1] = route_heading(rdo, s);
         }
         sN = s; vN = v;
     }
     // filter_preds: the other vehicle is behind the ego (utils.py:365-388)
     const double dx = obs[0] - zb[IX], dy = obs[1] - zb[IY];
-    if (dx * cos(zb[IPSI]) + dy * sin(zb[IPSI]) < 0.0)
+    if (dx * cos(zb[IPSI]) + dy * sin(zb[IPSI]) < 0.0) {
         for (int k = 0; k <= N; k++) { obs[2 * k] = -20.0; obs[2 * k + 1] = -20.0; }
+        if (OBCA) for (int k = 0; k <= N; k++) psi[k] = 0.0;
+    } else if (OBCA && rdo[11] != 0.0) {
+        for (int k = 0; k <= N; k++) psi[k] = fabs(psi[k]);                          // mpc.py:250-253
+    }
     eb.ctx[4 * b] = sN; eb.ctx[4 * b + 1] = vN; eb.ctx[4 * b + 2] = eb.enc[o]; eb.ctx[4 * b + 3] = eb.enc[b];   // mpc.py:326-337
     const int warm = t > 0 && eb.prev_ok[b] && (gt ? t > 1 : 1);   // evaluate.py:232-235 / :478-481
     eb.warm[b] = warm;

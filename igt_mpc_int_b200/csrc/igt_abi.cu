@@ -979,7 +979,7 @@ int igt_debug_round_phases(igt_handle *h, int *ph512x12)
 }
 #endif
 
-int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const double *route_desc, const double *curv,
+int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
                          const double *z0, const double *u_prev0, const double *enc, double *z_cl, double *u_cl,
                          int *solved, float *step_ms)
 {
@@ -987,6 +987,11 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const doub
     if (E < 0 || steps < 1 || !route_desc || !curv || !z0 || !u_prev0 || !enc || !z_cl || !u_cl || !solved) {
         h->err = "igt_episode_run: bad argument"; return IGT_EINVAL;
     }
+    if (mode & ~(IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)) {
+        h->err = "igt_episode_run: unknown mode bits (IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)"; return IGT_EINVAL;
+    }
+    const int gt_mpc = (mode & IGT_EPISODE_GT_MPC) != 0;
+    const bool obca = (mode & IGT_EPISODE_OBCA) != 0;
     if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_episode_run: needs precision f64"; return IGT_EINVAL; }
     if (gt_mpc && !h->has_mlp) { h->err = "igt_episode_run: gt_mpc needs igt_set_mlp"; return IGT_ENOMLP; }
     if (E == 0) return IGT_OK;
@@ -1001,8 +1006,8 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const doub
     // one device block: state, records, solver inputs and two sets of solver outputs (the plans of t and t-1)
     const size_t n_z = nb * 7, n_up = nb * 2, n_cv = nb * 3, n_rd = nb * ROUTE_DESC, n_en = nb, n_obs = nb * (N + 1) * 2,
                  n_ctx = nb * 4, n_ui = nb * N * 2, n_zcl = nb * (T + 1) * 7, n_ucl = nb * T * 2, n_x = nb * (N + 1) * 7,
-                 n_u = nb * N * 2;
-    const size_t n_dbl = n_z + n_up + n_cv + n_rd + n_en + n_obs + n_ctx + n_ui + n_zcl + n_ucl + 2 * (n_x + n_u + 2 * nb);
+                 n_u = nb * N * 2, n_op = obca ? nb * (N + 1) : 0;
+    const size_t n_dbl = n_z + n_up + n_cv + n_rd + n_en + n_obs + n_ctx + n_ui + n_zcl + n_ucl + 2 * (n_x + n_u + 2 * nb) + n_op;
     const size_t n_int = nb /*warm*/ + nb /*prev_ok*/ + nb * T /*solved*/ + 2 * 2 * nb /*status, iters x2*/;
     rc = grow(h, &h->episode, &h->episode_bytes, n_dbl * 8 + n_int * 4, st);
     if (rc) return rc;
@@ -1015,6 +1020,7 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const doub
     eb.z_cl = d; d += n_zcl; eb.u_cl = d; d += n_ucl;
     double *px[2], *pu[2], *pcost[2], *pviol[2];
     for (int i = 0; i < 2; i++) { px[i] = d; d += n_x; pu[i] = d; d += n_u; pcost[i] = d; d += nb; pviol[i] = d; d += nb; }
+    eb.obs_psi = obca ? d : nullptr; d += n_op;
     int *ip = (int *)d;
     eb.warm = ip; ip += nb; eb.prev_ok = ip; ip += nb; eb.solved = ip; ip += nb * T;
     int *pst[2], *pit[2];
@@ -1033,9 +1039,10 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const doub
     int cs = 0;
     for (int t = 0; t < T; t++) {
         const int cur = t & 1, prv = cur ^ 1;
-        episode_pre_kernel<<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
+        if (obca) episode_pre_kernel<true><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
+        else episode_pre_kernel<false><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
         h->launches++;
-        rc = solve_dev_impl(h, B, eb.z, eb.u_prev, eb.curv, eb.obs, nullptr, gt_mpc ? eb.ctx : nullptr, eb.u_init, px[cur], pu[cur],
+        rc = solve_dev_impl(h, B, eb.z, eb.u_prev, eb.curv, eb.obs, eb.obs_psi, gt_mpc ? eb.ctx : nullptr, eb.u_init, px[cur], pu[cur],
                             pcost[cur], pviol[cur], pst[cur], pit[cur], st, eb.warm);
         if (rc) return rc;
         rc = acquire_cslot(h, 1, st, &cs);

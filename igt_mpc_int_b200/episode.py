@@ -12,7 +12,17 @@ Mirrors the per-timestep glue of the reference's `evaluate.py`, 'mpc' branch (ev
   brake fallback     a = a_min if v > 0 else 0, previous steering, one model step; v < 0 -> hold pose, v = 0
                      evaluate.py:511-545
   outcome            deadlock = (#vehicles with final s <= 30) >= 2, evaluate.py:566-569; collision
-                     (min centre distance < d_min) and goal (final s > 30) are derived here.
+                     (min centre distance < d_min; in OBCA mode: the two 4.47 x 2.0 rectangles overlap at a
+                     recorded step) and goal (final s > 30) are derived here.
+
+Collision avoidance (`ca_type`, the reference's mpc.yaml collision_avoidance_type): 'circle' (default) or 'obca'
+(mpc.py:42-43, :170-175, :211-221; the solver must have d_min = 0).  OBCA needs the obstacle's heading forecast
+obs_psi[b, k], k = 0..N, built with the convention of MPC_Planner.update_predictions (mpc.py:250-253):
+  constant acceleration   k = 0 the other vehicle's current psi, k >= 1 the route heading at the forecast s_k
+  V2V                     k < N its previous plan's psi at k + 1, k = N the route heading at the extra step's s
+  flip                    abs() of every point if the other vehicle's route is 32 or 41
+  filter_preds            0.0 for an obstacle moved to (-20, -20)
+(csrc/episode.cuh episode_pre_kernel builds the same numbers on the device.)
 
 The solver is any object with the BatchSolver methods `solve_batch` and `evaluate`; tests drive the
 same loop with the CPU oracle wrapped in that interface to compare outcomes.
@@ -67,14 +77,31 @@ def reference_episode_specs(scenarios=range(1, 9), sample=0, seed=2026):
     return specs
 
 
-def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_latency=False, mode="mpc"):
+def _outcome(z_cl, u_cl, solved, d_min, ca_type, lat):
+    """deadlock (evaluate.py:566-569), collision, goal.  min_distance is the centre distance in both modes."""
+    dist = np.sqrt(np.sum((z_cl[:, 0, :, :2] - z_cl[:, 1, :, :2]) ** 2, axis=-1))
+    if ca_type == "obca":
+        collision = G.rectangles_overlap(z_cl[:, 0][..., [0, 1, 6]], z_cl[:, 1][..., [0, 1, 6]]).any(axis=1)
+    else:
+        collision = dist.min(axis=1) < d_min - 1e-6
+    final_s = z_cl[:, :, -1, 2]
+    return EpisodeResult(z_cl=z_cl, u_cl=u_cl, solved=solved, deadlock=np.sum(final_s <= 30, axis=1) >= 2,
+                         collision=collision, goal=final_s > 30, num_infeasible=(~solved).sum(axis=2),
+                         min_distance=dist.min(axis=1), step_latency_ms=lat)
+
+
+def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_latency=False, mode="mpc",
+                    ca_type="circle"):
     """mode 'gt_mpc' (the solver must have been given the value network): previous input (0, 0) instead of
     (0.1, 0) (evaluate.py:171 / :419); the first forecast assumes a = 0.09 (i + 1) for vehicle i
     (evaluate.py:207-210); warm starts only from t = 2 on (evaluate.py:232-235); every solve gets
     nn_ctx = (s_tv, v_tv, e_tv, e_ego): the other vehicle's forecast at step N (mpc.py:330) and the
-    scenario codes of utils.scenario_encoding (mpc.py:336-337)."""
-    assert mode in ("mpc", "gt_mpc")
+    scenario codes of utils.scenario_encoding (mpc.py:336-337).
+    ca_type 'obca': every solve also gets obs_psi (module docstring); the solver must have been made with d_min = 0.
+    Circle mode calls solve_batch without obs_psi, so solvers that do not know the keyword still work."""
+    assert mode in ("mpc", "gt_mpc") and ca_type in ("circle", "obca")
     gt = mode == "gt_mpc"
+    obca = ca_type == "obca"
     E = len(specs)
     B = 2 * E
     routes = [sp.routes for sp in specs]
@@ -103,6 +130,15 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
             x[idx], y[idx] = G.frenet2global_xy(s[idx], r, exit_coord=G.EXIT_COORD.get(r))
         return x, y
 
+    def route_psi(s):
+        """route heading of every vehicle's arc length(s): s[B] or s[B, K]"""
+        th = np.empty_like(s)
+        for r, idx in groups.items():
+            th[idx] = G.route_heading(s[idx], r)
+        return th
+
+    flip = np.array([r in ('32', '41') for r in route_of])                                  # mpc.py:250-253
+
     def ca_step(s, v, a):
         """one constant-acceleration predictor step, constant_acceleration_model.py:69-71 (vectorised)"""
         return s + v * dt + 0.5 * a * dt * dt, np.minimum(np.maximum(v + a * dt, V_PRED_MIN), V_PRED_MAX)
@@ -121,6 +157,10 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
         fc[:, :, 0], fc[:, :, 1] = route_xy(sk)
         fc[:, 0, 0], fc[:, 0, 1] = z[:, 0], z[:, 1]
         fc[:, :, 2], fc[:, :, 3] = sk, vk
+        if obca:
+            fpsi = np.empty((B, N + 1))
+            fpsi[:, 0] = z[:, 6]
+            fpsi[:, 1:] = route_psi(sk[:, 1:])
         if t > 0 and prev_ok.any():
             # V2V: a vehicle that solved at t-1 is forecast by its previous plan shifted by one + one
             # constant-acceleration step (redone with a = 0 if that exceeds v = 5), utils.py:339-352
@@ -134,6 +174,9 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
             s1, v1 = np.where(over, s1b, s1), np.where(over, v1b, v1)
             x1, y1 = route_xy(s1)
             fc[v2v, N, 0], fc[v2v, N, 1], fc[v2v, N, 2], fc[v2v, N, 3] = x1[v2v], y1[v2v], s1[v2v], v1[v2v]
+            if obca:
+                fpsi[v2v, :N] = prev_x[v2v, 1:, 6]
+                fpsi[v2v, N] = route_psi(s1)[v2v]
         # ---- per-vehicle obstacle = the other vehicle's forecast; all of it moves to (-20, -20) if the other
         #      vehicle is behind the ego (negative dot product with the ego heading), utils.py:365-388 ----
         other = np.arange(B) ^ 1
@@ -141,6 +184,10 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
         dx, dy = obs[:, 0, 0] - fc[:, 0, 0], obs[:, 0, 1] - fc[:, 0, 1]
         behind = dx * np.cos(z[:, 6]) + dy * np.sin(z[:, 6]) < 0
         obs[behind] = -20.0
+        if obca:
+            obs_psi = fpsi[other]
+            obs_psi[flip[other]] = np.abs(obs_psi[flip[other]])
+            obs_psi[behind] = 0.0
         # ---- solve: warm-started vehicles and cold ones in two batched calls ----
         t0 = time.perf_counter()
         u_init = np.concatenate([prev_u[:, 1:], prev_u[:, -1:]], axis=1)                   # utils.py:362
@@ -155,6 +202,8 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
             if len(idx) == 0:
                 continue
             kw = dict(nn_ctx=nn_ctx[idx]) if gt else {}
+            if obca:
+                kw["obs_psi"] = obs_psi[idx]
             r = solver.solve_batch(z[idx], u_prev[idx], curv[idx], obs[idx], u_init=u_init[idx] if warm else None, **kw)
             out["x"][idx], out["u"][idx], out["status"][idx] = r["x"], r["u"], r["status"]
         if record_latency:
@@ -182,21 +231,25 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
         z, u_prev = z_next, u_app
         z_cl[:, :, t + 1] = z.reshape(E, 2, 7); u_cl[:, :, t] = u_app.reshape(E, 2, 2)
         solved[:, :, t] = ok.reshape(E, 2)
-    dist = np.sqrt(np.sum((z_cl[:, 0, :, :2] - z_cl[:, 1, :, :2]) ** 2, axis=-1))
-    final_s = z_cl[:, :, -1, 2]
-    return EpisodeResult(z_cl=z_cl, u_cl=u_cl, solved=solved, deadlock=np.sum(final_s <= 30, axis=1) >= 2,
-                         collision=dist.min(axis=1) < d_min - 1e-6, goal=final_s > 30,
-                         num_infeasible=(~solved).sum(axis=2), min_distance=dist.min(axis=1), step_latency_ms=lat)
+    return _outcome(z_cl, u_cl, solved, d_min, ca_type, lat)
 
 
-def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc", record_latency=False):
+def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc", record_latency=False, ca_type="circle"):
     """The same closed loop with the per-timestep glue on the GPU (csrc/episode.cuh, igt_episode_run_host): all E
     episodes advance `steps` steps without the host in the loop -- per step one glue kernel, one batched solve of all 2E
     vehicles (per-problem warm / cold start), one plant kernel.  `solver` is a planner.BatchSolver (fp64) with horizon N.
-    Returns an EpisodeResult; step_latency_ms = device time per step (all episodes together)."""
+    Returns an EpisodeResult; step_latency_ms = device time per step (all episodes together).
+    ca_type 'obca' builds the obstacle heading forecast on the device as well (module docstring) and needs a solver
+    made with d_min = 0 (mpc.py:42-43): with the circle gap of 5.6 m the rectangles would be kept that far apart."""
     import ctypes as C
     assert mode in ("mpc", "gt_mpc") and solver.N == N
+    if ca_type not in ("circle", "obca"):
+        raise ValueError("ca_type must be 'circle' or 'obca', got %r" % (ca_type,))
+    if ca_type == "obca" and solver.params.d_min != 0:
+        raise ValueError("ca_type='obca' needs a solver with d_min = 0 (mpc.py:42-43), this one has d_min = %g"
+                         % solver.params.d_min)
     gt = mode == "gt_mpc"
+    flags = (_lib.EPISODE_GT_MPC if gt else 0) | (_lib.EPISODE_OBCA if ca_type == "obca" else 0)
     E = len(specs)
     B = 2 * E
     rd = np.array([G.route_descriptor(r, exit_coord=G.EXIT_COORD.get(r)) for sp in specs for r in sp.routes], dtype=np.float64)
@@ -213,13 +266,7 @@ def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc"
     z_cl = np.zeros((E, 2, steps + 1, 7)); u_cl = np.zeros((E, 2, steps, 2)); solved = np.zeros((E, 2, steps), dtype=np.int32)
     ms = np.zeros(steps, dtype=np.float32)
     vp = lambda a: C.c_void_p(a.ctypes.data)
-    rc = solver.lib.igt_episode_run_host(solver._h, E, steps, 1 if gt else 0, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
+    rc = solver.lib.igt_episode_run_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
                                          vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
     solver._check(rc, "igt_episode_run_host")
-    solved = solved.astype(bool)
-    dist = np.sqrt(np.sum((z_cl[:, 0, :, :2] - z_cl[:, 1, :, :2]) ** 2, axis=-1))
-    final_s = z_cl[:, :, -1, 2]
-    return EpisodeResult(z_cl=z_cl, u_cl=u_cl, solved=solved, deadlock=np.sum(final_s <= 30, axis=1) >= 2,
-                         collision=dist.min(axis=1) < d_min - 1e-6, goal=final_s > 30,
-                         num_infeasible=(~solved).sum(axis=2), min_distance=dist.min(axis=1),
-                         step_latency_ms=[float(v) for v in ms] if record_latency else [])
+    return _outcome(z_cl, u_cl, solved.astype(bool), d_min, ca_type, [float(v) for v in ms] if record_latency else [])

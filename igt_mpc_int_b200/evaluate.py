@@ -10,6 +10,10 @@ rotation of the scenario and the order of the two vehicles with an unseeded `ran
 (utils.py:177-179); here they are arguments (--rotation, --order; --all_variants runs the eight of them).
 No video is rendered (evaluate.py:589 needs matplotlib/ffmpeg: out of scope).
 
+`--ca_type obca` runs the reference's other collision-avoidance mode (mpc.yaml collision_avoidance_type, mpc.py:42-43):
+rectangle rows with d_min = 0 instead of the 5.6 m circle gap; an episode's collision flag then means that the two
+4.47 x 2.0 rectangles overlapped at a recorded step (min_distance stays the centre distance).
+
 `--eval_mode gt_mpc` needs the value network: --nn_weights FILE.npz with arrays W0, b0, W1, b1, ...
 (model.py:14-51 layer order) and optionally Wn, mu_f, sigma_t, mu_t (mpc.py:109-118; the reference's
 processed_sc*.pkl statistics are not shipped, identity / zero are used when absent).
@@ -39,7 +43,12 @@ def load_mlp(path):
 
 
 def main(args, solver=None):
+    """`solver`: any object with the BatchSolver methods (default: a BatchSolver made here, d_min = 0 for OBCA)."""
     seed = 2026
+    ca_type = getattr(args, 'ca_type', 'circle')
+    if ca_type not in ('circle', 'obca'):
+        raise ValueError("ca_type must be 'circle' or 'obca', got %r" % (ca_type,))
+    policy_config = dict(POLICY_CONFIG, collision_avoidance_type=ca_type)
     N, dt = POLICY_CONFIG['N'], POLICY_CONFIG['dt']
     T = getattr(args, 'steps', None) or 150                                                # T_sim / dt, evaluate.py:84-85
     timenow = datetime.datetime.now().strftime("%Y%m%d_%H%M%S")
@@ -48,14 +57,14 @@ def main(args, solver=None):
     if own:
         from .planner import BatchSolver
         mlp = load_mlp(args.nn_weights) if args.eval_mode == 'gt_mpc' else None
-        solver = BatchSolver(N=N, dt=dt, mlp=mlp)
+        solver = BatchSolver(N=N, dt=dt, mlp=mlp, **(dict(d_min=0.0) if ca_type == 'obca' else {}))
     variants = [(r, o) for r in range(4) for o in range(2)] if args.all_variants else [(args.rotation, args.order)]
     summary = []
     for it in range(args.num_samples):
         all_specs = episode.reference_episode_specs(scenarios=[args.sc], sample=it, seed=seed)
         specs = [all_specs[r * 2 + o] for r, o in variants]
         loop = episode.run_closed_loop_device if getattr(args, 'device_loop', False) else episode.run_closed_loop
-        res = loop(solver, specs, steps=T, N=N, record_latency=True, mode=args.eval_mode)
+        res = loop(solver, specs, steps=T, N=N, record_latency=True, mode=args.eval_mode, ca_type=ca_type)
         for e, sp in enumerate(specs):
             starts = [G.frenet2global(sp.s0[i], sp.routes[i]) for i in range(2)]
             refs = [RT.reference_dict(sp.routes[i], starts[i][0], starts[i][1], n=T) for i in range(2)]
@@ -65,7 +74,7 @@ def main(args, solver=None):
             times = [[1e-3 * ms for ms in res.step_latency_ms]] * 2          # both vehicles are solved in one batched call
             sub = results.write_episode(run_dir, args.eval_mode, res.z_cl[e], res.u_cl[e], res.solved[e], res.deadlock[e],
                                         times, N=N, refs=refs, initial_agents=agents, initial_default=default,
-                                        routes=sp.routes, goals=goals, policy_config=POLICY_CONFIG)
+                                        routes=sp.routes, goals=goals, policy_config=policy_config)
             summary.append(dict(sample=it, routes=sp.routes, deadlock=bool(res.deadlock[e]), collision=bool(res.collision[e]),
                                 goal=[bool(g) for g in res.goal[e]], infeasible=[int(n) for n in res.num_infeasible[e]],
                                 min_distance=float(res.min_distance[e])))
@@ -88,6 +97,8 @@ def build_parser():
     p.add_argument('--nn_weights', type=str, default=None)
     p.add_argument('--steps', type=int, default=150, help='closed-loop steps (the reference simulates 15 s = 150)')
     p.add_argument('--device_loop', action='store_true', help='run the per-timestep glue on the GPU as well (igt_episode_run_host)')
+    p.add_argument('--ca_type', type=str, default='circle', choices=['circle', 'obca'],
+                   help="collision avoidance (mpc.yaml collision_avoidance_type): 5.6 m circles or OBCA rectangles with d_min = 0")
     return p
 
 

@@ -137,18 +137,21 @@ def frenet2global(s, route, ey=0.0, W=ROAD_WIDTH, L=ROAD_LENGTH, ca=CA_RADIUS, e
 
 
 def route_descriptor(route, W=ROAD_WIDTH, L=ROAD_LENGTH, ca=CA_RADIUS, exit_coord=None):
-    """The 12 numbers the device-side closed loop needs to evaluate `frenet2global_xy` for this route
-    (csrc/episode.cuh route_xy): x0, y0, t0x, t0y, turn sign, b0, b1, r, exit axis (0: x, 1: y, -1: none), exit
-    coordinate, 0, 0."""
+    """The 12 numbers the device-side closed loop needs to evaluate `frenet2global_xy` and `route_heading` for this
+    route (csrc/episode.cuh route_xy / route_heading): x0, y0, t0x, t0y, turn sign, b0, b1, r, exit axis (0: x, 1: y,
+    -1: none), exit coordinate, start heading th0 (stored, not recovered with atan2, so that the device heading is
+    bit-identical), flip (1.0 on routes 32 and 41, whose headings the planner takes abs() of, mpc.py:250-253)."""
     x0, y0, th0 = start_pose(route[0], W, L, ca)
     t0 = (math.cos(th0), math.sin(th0))
     sgn = turn_sign(route)
+    flip = 1.0 if route in ('32', '41') else 0.0
     if sgn == 0:
-        return [x0, y0, t0[0], t0[1], 0.0, 1e30, 1e30, 1.0, -1.0, 0.0, 0.0, 0.0]
+        return [x0, y0, t0[0], t0[1], 0.0, 1e30, 1e30, 1.0, -1.0, 0.0, th0, flip]
     b0, b1, K = curvature_params(route, W, L, ca)
     t1x = sgn * (-t0[1])
     axis = -1.0 if exit_coord is None else (0.0 if abs(t1x) < 0.5 else 1.0)
-    return [x0, y0, t0[0], t0[1], float(sgn), b0, b1, 1.0 / abs(K), axis, 0.0 if exit_coord is None else float(exit_coord), 0.0, 0.0]
+    return [x0, y0, t0[0], t0[1], float(sgn), b0, b1, 1.0 / abs(K), axis, 0.0 if exit_coord is None else float(exit_coord),
+            th0, flip]
 
 
 def frenet2global_xy(s, route, W=ROAD_WIDTH, L=ROAD_LENGTH, ca=CA_RADIUS, exit_coord=None):
@@ -177,6 +180,38 @@ def frenet2global_xy(s, route, W=ROAD_WIDTH, L=ROAD_LENGTH, ca=CA_RADIUS, exit_c
     x = np.where(s < b0, x0 + s * t0[0], np.where(s <= b1, xa, xe))
     y = np.where(s < b0, y0 + s * t0[1], np.where(s <= b1, ya, ye))
     return x, y
+
+
+def route_heading(s, route, W=ROAD_WIDTH, L=ROAD_LENGTH, ca=CA_RADIUS):
+    """The path heading of `frenet2global` (its third output) for an array of arc lengths: th0 before the arc,
+    th0 + sgn * phi on it, th0 + sgn * pi / 2 after it.  No abs() flip (that is the planner's, mpc.py:250-253)."""
+    s = np.asarray(s, dtype=np.float64)
+    th0 = start_pose(route[0], W, L, ca)[2]
+    sgn = turn_sign(route)
+    if sgn == 0:
+        return np.full_like(s, th0)
+    b0, b1, K = curvature_params(route, W, L, ca)
+    r = 1.0 / abs(K)
+    phi = (s - b0) / r
+    return np.where(s < b0, th0, np.where(s <= b1, th0 + sgn * phi, th0 + sgn * math.pi / 2))
+
+
+def rectangles_overlap(p, q, h=4.47, w=2.0):
+    """Do the h x w rectangles centred at (x, y) with heading psi (length along the heading, csrc/obca.cuh) overlap?
+    p, q[..., 3] = (x, y, psi) -> bool[...].  Separating-axis test over the four face normals; rectangles that only
+    touch do not overlap."""
+    p = np.asarray(p, dtype=np.float64); q = np.asarray(q, dtype=np.float64)
+    cp, sp, cq, sq = np.cos(p[..., 2]), np.sin(p[..., 2]), np.cos(q[..., 2]), np.sin(q[..., 2])
+    dx, dy = q[..., 0] - p[..., 0], q[..., 1] - p[..., 1]
+    hl, hw = h / 2, w / 2
+    sep = np.zeros(np.broadcast(p[..., 0], q[..., 0]).shape, dtype=bool)
+    for ax, ay, he in ((cp, sp, hl), (-sp, cp, hw)):              # p's face normals: p's half-extent he along them
+        ho = hl * np.abs(ax * cq + ay * sq) + hw * np.abs(-ax * sq + ay * cq)
+        sep |= np.abs(ax * dx + ay * dy) >= he + ho
+    for ax, ay, ho in ((cq, sq, hl), (-sq, cq, hw)):              # q's face normals
+        he = hl * np.abs(ax * cp + ay * sp) + hw * np.abs(-ax * sp + ay * cp)
+        sep |= np.abs(ax * dx + ay * dy) >= he + ho
+    return ~sep
 
 
 def scenario_routes(sc, rotation, order):

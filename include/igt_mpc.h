@@ -167,13 +167,25 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
  * (constant-acceleration forecast constant_acceleration_model.py:18-82, shared plans utils.py:339-352, filter_preds
  * utils.py:365-388, warm start utils.py:354-363, value-network context mpc.py:326-337), one batched solve of all 2E
  * vehicles (per-problem warm / cold start), one kernel after it (plant evaluate.py:491-510, brake fallback :511-545).
- * Vehicle b = 2 e + i is agent i of episode e.  Host fp64 arrays:
- *   route_desc[2E,12] = (x0, y0, t0x, t0y, turn sign, b0, b1, r, exit axis (0 x, 1 y, -1 none), exit coordinate, 0, 0):
- *                       the closed-form lane centre of the vehicle's route (igt_mpc_int_b200/geometry.py);
+ * Vehicle b = 2 e + i is agent i of episode e.
+ * mode: a bit set.  0 = the 'mpc' branch with circle rows;
+ *   IGT_EPISODE_GT_MPC -- the 'gt_mpc' branch (value-network terminal cost; the handle needs igt_set_mlp);
+ *   IGT_EPISODE_OBCA   -- collision_avoidance_type 'obca' (mpc.py:42-43): the glue also forecasts the other vehicle's
+ *                         heading (k = 0 its current psi; k >= 1 the route heading at the forecast arc length, or its
+ *                         previous plan's psi in the shared-plan case; abs() on routes 32 / 41, mpc.py:250-253; 0 for
+ *                         a filtered obstacle) and every solve gets it as obs_psi (see igt_solve_*).  The handle's
+ *                         d_min should be 0, as the reference sets it for this mode.
+ *   Any other bit: IGT_EINVAL.
+ * Host fp64 arrays:
+ *   route_desc[2E,12] = (x0, y0, t0x, t0y, turn sign, b0, b1, r, exit axis (0 x, 1 y, -1 none), exit coordinate,
+ *                       th0, flip): the closed-form lane centre of the vehicle's route (igt_mpc_int_b200/geometry.py);
+ *                       th0 = start heading, flip = 1.0 on routes 32 and 41, else 0.0 -- read in OBCA mode only;
  *   curv[2E,3]; z0[2E,7] initial states; u_prev0[2E,2]; enc[2E] scenario codes (utils.py:141-169, gt_mpc only);
  *   out: z_cl[E,2,steps+1,7], u_cl[E,2,steps,2], solved[E,2,steps] (int32), step_ms[steps] (device time per step; may
- *   be NULL).  The handle's horizon N, limits and (gt_mpc != 0) value network apply; precision must be f64. */
-int igt_episode_run_host(igt_handle *h, int E, int steps, int gt_mpc, const double *route_desc, const double *curv,
+ *   be NULL).  The handle's horizon N, limits and (gt_mpc) value network apply; precision must be f64. */
+#define IGT_EPISODE_GT_MPC 1
+#define IGT_EPISODE_OBCA 2
+int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
                          const double *z0, const double *u_prev0, const double *enc, double *z_cl, double *u_cl,
                          int *solved, float *step_ms);
 
