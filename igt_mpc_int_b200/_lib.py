@@ -13,9 +13,11 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("IGT_LIB", os.path.join(_HERE, "lib", "libigtmpc.so"))   # IGT_LIB: developer override
 
 MAX_CINF, MAX_LAYERS = 128, 5
+MAX_MLP_NETS = 8        # value networks per handle (igt_set_mlp_at)
 PREC_F32, PREC_F64 = 0, 1
+STATUS_BAD_NET = 7      # a bank solve whose net_idx names no loaded network (igt_solve_ex_dev)
 STATUS_NAMES = {0: "converged", 1: "max_iter", 2: "x0_infeasible", 3: "reg_limit", 4: "line_search",
-                5: "stalled_infeasible", 6: "acceptable"}
+                5: "stalled_infeasible", 6: "acceptable", 7: "bad_net"}
 EPISODE_GT_MPC, EPISODE_OBCA = 1, 2   # mode bits of igt_episode_run_host
 STATUS_OK = (0, 6)      # converged, or stopped within the reference's own IPOPT tolerances (igt_mpc.h: IGT_STATUS_ACCEPTABLE)
 
@@ -67,7 +69,8 @@ _lib = None
 EXPORTS = ("igt_version", "igt_default_params", "igt_create", "igt_destroy", "igt_last_error",
            "igt_set_mlp", "igt_rollout_dev", "igt_rollout_host", "igt_eval_host", "igt_solve_dev",
            "igt_solve_host", "igt_launch_count", "igt_measure_fma_peak", "igt_mlp_value_host", "igt_set_option",
-           "igt_episode_run_host")
+           "igt_episode_run_host", "igt_set_mlp_at", "igt_solve_ex_dev", "igt_solve_ex_host", "igt_eval_ex_host",
+           "igt_mlp_value_ex_host", "igt_episode_run_ex_host")
 
 
 def load():
@@ -103,6 +106,15 @@ def load():
     lib.igt_launch_count.restype = C.c_longlong
     lib.igt_episode_run_host.argtypes = [vp, C.c_int, C.c_int, C.c_int] + [vp] * 9
     lib.igt_episode_run_host.restype = C.c_int
+    lib.igt_set_mlp_at.argtypes = [vp, C.c_int, C.c_int, _ip, C.POINTER(_dp), C.POINTER(_dp), _dp, _dp, C.c_double, C.c_double]
+    lib.igt_solve_ex_dev.argtypes = [vp, C.c_int] + [vp] * 14 + [vp]
+    lib.igt_solve_ex_host.argtypes = [vp, C.c_int] + [vp] * 14
+    lib.igt_eval_ex_host.argtypes = [vp, C.c_int] + [vp] * 11
+    lib.igt_mlp_value_ex_host.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp, C.c_int]
+    lib.igt_episode_run_ex_host.argtypes = [vp, C.c_int, C.c_int, C.c_int] + [vp] * 10
+    for f in ("igt_set_mlp_at", "igt_solve_ex_dev", "igt_solve_ex_host", "igt_eval_ex_host", "igt_mlp_value_ex_host",
+              "igt_episode_run_ex_host"):
+        getattr(lib, f).restype = C.c_int
     for f in ("igt_default_params", "igt_create", "igt_set_mlp", "igt_rollout_dev", "igt_rollout_host",
               "igt_eval_host", "igt_solve_dev", "igt_solve_host"):
         getattr(lib, f).restype = C.c_int

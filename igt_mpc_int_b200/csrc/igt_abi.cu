@@ -59,8 +59,9 @@ __global__ void __launch_bounds__(128) guess_kernel(ProbIO io, long B, double *g
 #ifndef IGT_RSTG
 #define IGT_RSTG 1     // row staging in the node phases of the plain throughput kernels (solver_core.cuh, Ws RSTG)
 #endif
-template <typename T, bool TC, bool OBCA, bool COOP = false>
-__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(ProbIO io, T *ws, long n_slots, long B, Sched sc,
+// BANK: gt_mpc with the handle's network bank, network io.net_idx[p] per problem (not with TC)
+template <typename T, bool TC, bool OBCA, bool COOP = false, bool BANK = false>
+__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type io, T *ws, long n_slots, long B, Sched sc,
                                                                const double *guess, T *mlp_scratch, int mlp_width,
                                                                MlpTcWeights wt, int quota, int cs)
 {
@@ -72,7 +73,7 @@ __global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(ProbIO io, T *ws,
     constexpr bool RSTG = IGT_RSTG && !TC && !COOP;                 // (TC fills shared memory itself; with COOP the value term's
                                                                     //  weight reads need the L1 more: measured 120 -> 146 ms per batch)
     // dynamic shared memory: [cooperative value-term buffers (COOP)] [row staging (RSTG)]
-    solve_persistent<T, TC, 32, OBCA, COOP, RSTG>(P, io, ws, slot, B, sc, guess,
+    solve_persistent<T, TC, 32, OBCA, COOP, RSTG, BANK>(P, io, ws, slot, B, sc, guess,
                             mlp_scratch ? mlp_scratch + slot * 12 * (long)mlp_width : nullptr, mlp_width, &tc, quota, cs, dyn_smem,
                             RSTG ? dyn_smem + (COOP ? mlp_coop_smem_bytes<T>(SOLVE_BLOCK) : 0) : nullptr);
     if (TC) mlp_tc_teardown(tc);
@@ -178,13 +179,16 @@ __global__ void __launch_bounds__(128) rollout_euler_kernel(int B, const float *
     }
 }
 
-// fp64 re-roll + cost + max inequality row (reference units) of given controls
+// fp64 re-roll + cost + max inequality row (reference units) of given controls; BANK: value term of network
+// net_idx[p] of the bank (indices checked by the host)
+template <bool BANK>
 __global__ void __launch_bounds__(128) eval_kernel(long B, const double *__restrict__ x0_, const double *__restrict__ uprev_,
                                                    const double *__restrict__ curv_, const double *__restrict__ obs_,
                                                    const double *__restrict__ ctx_, const double *__restrict__ U,
                                                    double *__restrict__ cost, double *__restrict__ viol,
                                                    double *__restrict__ Zout, double *mlp_scratch, int mlp_width, int cs,
-                                                   const double *__restrict__ obs_psi_)
+                                                   const double *__restrict__ obs_psi_, const int *__restrict__ net_idx,
+                                                   const MlpNet<double> *nets)
 {
     long p = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= B) return;
@@ -228,7 +232,8 @@ __global__ void __launch_bounds__(128) eval_kernel(long B, const double *__restr
         TermVal<double> t;
         double ctx[4] = { ctx_[4 * p], ctx_[4 * p + 1], ctx_[4 * p + 2], ctx_[4 * p + 3] };
         double *sc = mlp_scratch + p * 12 * (long)mlp_width;
-        mlp_eval_thread(P, z[IS], z[IV], ctx, sc, sc + 6 * mlp_width, mlp_width, t, false);
+        if (BANK) mlp_eval_thread_net(nets[net_idx[p]], z[IS], z[IV], ctx, sc, sc + 6 * mlp_width, mlp_width, t, false);
+        else mlp_eval_thread(P, z[IS], z[IV], ctx, sc, sc + 6 * mlp_width, mlp_width, t, false);
         J -= t.V;
     } else {
         J -= z[IS] - s0;
@@ -257,8 +262,10 @@ __global__ void __launch_bounds__(256, 1) mlp_tc_kernel(MlpTcWeights wt, long B,
     mlp_tc_teardown(c);
 }
 
+template <bool BANK>
 __global__ void __launch_bounds__(128) mlp_ref_kernel(long B, const double *sN, const double *vN, const double *ctx,
-                                                      double *out, double *scratch, int width, int cs)
+                                                      double *out, double *scratch, int width, int cs, const int *net_idx,
+                                                      const MlpNet<double> *nets)
 {
     long p = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= B) return;
@@ -266,13 +273,15 @@ __global__ void __launch_bounds__(128) mlp_ref_kernel(long B, const double *sN, 
     TermVal<double> t;
     double cx[4] = { ctx[4 * p], ctx[4 * p + 1], ctx[4 * p + 2], ctx[4 * p + 3] };
     double *sc = scratch + p * 12 * (long)width;
-    mlp_eval_thread(P, sN[p], vN[p], cx, sc, sc + 6 * width, width, t, true);
+    if (BANK) mlp_eval_thread_net(nets[net_idx[p]], sN[p], vN[p], cx, sc, sc + 6 * width, width, t, true);
+    else mlp_eval_thread(P, sN[p], vN[p], cx, sc, sc + 6 * width, width, t, true);
     out[6 * p] = t.V; out[6 * p + 1] = t.gs; out[6 * p + 2] = t.gv; out[6 * p + 3] = t.Hss; out[6 * p + 4] = t.Hsv; out[6 * p + 5] = t.Hvv;
 }
 
-// the exact cooperative evaluation (mlp_coop.cuh) standalone: one CTA pass per 256 problems
+// the exact cooperative evaluation (mlp_coop.cuh) standalone: one CTA pass per 256 problems; BANK: network net_idx[p]
+template <bool BANK>
 __global__ void __launch_bounds__(256, 1) mlp_coop_kernel(long B, const double *sN, const double *vN, const double *ctx,
-                                                          double *out, int cs)
+                                                          double *out, int cs, const int *net_idx, const MlpNet<double> *nets)
 {
     extern __shared__ __align__(16) uint8_t dyn_smem[];
     const DevParams<double> &P = c_Pd[cs];
@@ -280,8 +289,10 @@ __global__ void __launch_bounds__(256, 1) mlp_coop_kernel(long B, const double *
         const long p = base + threadIdx.x;
         const bool valid = p < B;
         double cx[4] = { 0, 0, 0, 0 }, o[6], s = 0, v = 0;
-        if (valid) { s = sN[p]; v = vN[p]; for (int i = 0; i < 4; i++) cx[i] = ctx[4 * p + i]; }
-        mlp_coop_eval(P, dyn_smem, valid, s, v, cx, o);
+        int net = 0;
+        if (valid) { s = sN[p]; v = vN[p]; for (int i = 0; i < 4; i++) cx[i] = ctx[4 * p + i]; if (BANK) net = net_idx[p]; }
+        if (BANK) mlp_coop_eval_bank(nets, dyn_smem, valid, net, s, v, cx, o);
+        else mlp_coop_eval(P, dyn_smem, valid, s, v, cx, o);
         if (valid) for (int i = 0; i < 6; i++) out[6 * p + i] = o[i];
     }
 }
@@ -311,7 +322,13 @@ struct igt_handle {
     bool coop_ok = false;              // every layer <= MLP_COOP_W wide: the exact CTA-cooperative evaluation applies
     int use_small = 1;                 // igt_set_option("latency_path", 0) keeps small batches on the throughput kernel
     int mlp_width = 0;
-    std::vector<void *> mlp_bufs;      // device weight buffers (both precisions)
+    // network bank (igt_set_mlp_at): slot 0 is also the network above (Pf / Pd, tc); a solve with net_idx reads the
+    // device table `bank` = [MAX_MLP_NETS] MlpNet<double>, then [MAX_MLP_NETS] MlpNet<float>
+    std::vector<void *> mlp_bufs[MAX_MLP_NETS];   // device weight buffers of each slot (both precisions)
+    MlpNet<double> netd[MAX_MLP_NETS] = {};
+    MlpNet<float> netf[MAX_MLP_NETS] = {};
+    int net_width[MAX_MLP_NETS] = {};  // widest layer of each slot, 0 = empty
+    void *bank = nullptr;
     void *ws = nullptr; size_t ws_bytes = 0;
     void *mlp_scratch = nullptr; size_t mlp_scratch_bytes = 0;
     void *stage = nullptr; size_t stage_bytes = 0;     // device staging for *_host calls
@@ -341,6 +358,7 @@ static CSlot g_slots[MAX_DEV][2][N_CSLOTS];
 static unsigned g_slot_rr[MAX_DEV][2];
 
 static std::string g_create_err;
+static_assert(IGT_MAX_MLP_NETS == MAX_MLP_NETS, "bank size");
 
 #define CK(call)                                                                                   \
     do {                                                                                           \
@@ -457,7 +475,8 @@ void igt_destroy(igt_handle *h)
             for (int i = 0; i < N_CSLOTS; i++)
                 if (g_slots[dev][prec][i].owner == h) { g_slots[dev][prec][i].owner = nullptr; g_slots[dev][prec][i].version = 0; }
     }
-    for (void *b : h->mlp_bufs) cudaFree(b);
+    for (auto &v : h->mlp_bufs) for (void *b : v) cudaFree(b);
+    if (h->bank) cudaFree(h->bank);
     if (h->hstream) cudaStreamDestroy(h->hstream);
     if (h->pin) cudaFreeHost(h->pin);
     if (h->ws) cudaFree(h->ws);
@@ -472,52 +491,74 @@ const char *igt_last_error(const igt_handle *h) { return h ? h->err.c_str() : g_
 
 long long igt_launch_count(const igt_handle *h) { return h ? h->launches : 0; }
 
-int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *const *W, const double *const *b,
-                const double *Wn, const double *mu_f, double sigma_t, double mu_t)
+int igt_set_mlp_at(igt_handle *h, int net, int n_layers, const int *dims, const double *const *W, const double *const *b,
+                   const double *Wn, const double *mu_f, double sigma_t, double mu_t)
 {
     if (!h) return IGT_EINVAL;
+    if (net < 0 || net >= IGT_MAX_MLP_NETS) { h->err = "igt_set_mlp: net must be in 0..IGT_MAX_MLP_NETS-1"; return IGT_EINVAL; }
     if (n_layers < 1 || n_layers > IGT_MAX_MLP_LAYERS || !dims || !W || !b || !Wn || !mu_f || dims[0] != 6 ||
         dims[n_layers] != 1) { h->err = "igt_set_mlp: bad layer description"; return IGT_EINVAL; }
+    int width = 6;
+    for (int l = 0; l <= n_layers; l++) { if (dims[l] < 1 || dims[l] > 1024) { h->err = "igt_set_mlp: bad width"; return IGT_EINVAL; } if (dims[l] > width) width = dims[l]; }
+    for (int l = 0; l < n_layers; l++) if (!W[l] || !b[l]) { h->err = "igt_set_mlp: null layer"; return IGT_EINVAL; }
     std::lock_guard<std::mutex> lk(h->mu);
     CK(cudaSetDevice(h->device));
     if (h->last_use && h->used) CK(cudaEventSynchronize(h->last_use));   // no kernel of this handle reads the old network
+    if (!h->bank) CK(cudaMalloc(&h->bank, MAX_MLP_NETS * (sizeof(MlpNet<double>) + sizeof(MlpNet<float>))));
     h->version[0]++; h->version[1]++;
-    for (void *q : h->mlp_bufs) cudaFree(q);
-    h->mlp_bufs.clear();
-    int width = 6;
-    for (int l = 0; l <= n_layers; l++) { if (dims[l] < 1 || dims[l] > 1024) { h->err = "igt_set_mlp: bad width"; return IGT_EINVAL; } if (dims[l] > width) width = dims[l]; }
-    h->mlp_width = width;
-    h->Pf.n_layers = h->Pd.n_layers = n_layers;
-    for (int l = 0; l <= n_layers; l++) h->Pf.dims[l] = h->Pd.dims[l] = dims[l];
+    for (void *q : h->mlp_bufs[net]) cudaFree(q);
+    h->mlp_bufs[net].clear();
+    h->net_width[net] = 0;
+    MlpNet<double> &nd = h->netd[net];
+    MlpNet<float> &nf = h->netf[net];
+    nd = MlpNet<double>(); nf = MlpNet<float>();
+    std::vector<void *> &bufs = h->mlp_bufs[net];
+    nf.n_layers = nd.n_layers = n_layers;
+    for (int l = 0; l <= n_layers; l++) nf.dims[l] = nd.dims[l] = dims[l];
     for (int l = 0; l < n_layers; l++) {
         size_t nw = (size_t)dims[l] * dims[l + 1], nb = dims[l + 1];
         std::vector<float> wf(nw), bf(nb);
         for (size_t i = 0; i < nw; i++) wf[i] = (float)W[l][i];
         for (size_t i = 0; i < nb; i++) bf[i] = (float)b[l][i];
         void *dWd, *dbd, *dWf, *dbf;
-        CK(cudaMalloc(&dWd, nw * 8)); h->mlp_bufs.push_back(dWd);
-        CK(cudaMalloc(&dbd, nb * 8)); h->mlp_bufs.push_back(dbd);
-        CK(cudaMalloc(&dWf, nw * 4)); h->mlp_bufs.push_back(dWf);
-        CK(cudaMalloc(&dbf, nb * 4)); h->mlp_bufs.push_back(dbf);
+        CK(cudaMalloc(&dWd, nw * 8)); bufs.push_back(dWd);
+        CK(cudaMalloc(&dbd, nb * 8)); bufs.push_back(dbd);
+        CK(cudaMalloc(&dWf, nw * 4)); bufs.push_back(dWf);
+        CK(cudaMalloc(&dbf, nb * 4)); bufs.push_back(dbf);
         CK(cudaMemcpy(dWd, W[l], nw * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dbd, b[l], nb * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dWf, wf.data(), nw * 4, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dbf, bf.data(), nb * 4, cudaMemcpyHostToDevice));
-        h->Pd.W[l] = (const double *)dWd; h->Pd.b[l] = (const double *)dbd;
-        h->Pf.W[l] = (const float *)dWf; h->Pf.b[l] = (const float *)dbf;
+        nd.W[l] = (const double *)dWd; nd.b[l] = (const double *)dbd;
+        nf.W[l] = (const float *)dWf; nf.b[l] = (const float *)dbf;
         // transposed copies [in][out] for the cooperative evaluation (mlp_coop.cuh)
         std::vector<double> wtd(nw); std::vector<float> wtf(nw);
         for (int o = 0; o < dims[l + 1]; o++)
             for (int i = 0; i < dims[l]; i++) { wtd[(size_t)i * dims[l + 1] + o] = W[l][(size_t)o * dims[l] + i]; wtf[(size_t)i * dims[l + 1] + o] = (float)W[l][(size_t)o * dims[l] + i]; }
         void *dTd, *dTf;
-        CK(cudaMalloc(&dTd, nw * 8)); h->mlp_bufs.push_back(dTd);
-        CK(cudaMalloc(&dTf, nw * 4)); h->mlp_bufs.push_back(dTf);
+        CK(cudaMalloc(&dTd, nw * 8)); bufs.push_back(dTd);
+        CK(cudaMalloc(&dTf, nw * 4)); bufs.push_back(dTf);
         CK(cudaMemcpy(dTd, wtd.data(), nw * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dTf, wtf.data(), nw * 4, cudaMemcpyHostToDevice));
-        h->Pd.Wt[l] = (const double *)dTd; h->Pf.Wt[l] = (const float *)dTf;
+        nd.Wt[l] = (const double *)dTd; nf.Wt[l] = (const float *)dTf;
     }
-    h->coop_ok = true;
-    for (int l = 0; l <= n_layers; l++) if (dims[l] > MLP_COOP_W) h->coop_ok = false;
+    for (int i = 0; i < 36; i++) { nd.Wn[i] = Wn[i]; nf.Wn[i] = (float)Wn[i]; }
+    for (int i = 0; i < 6; i++) { nd.mu_f[i] = mu_f[i]; nf.mu_f[i] = (float)mu_f[i]; }
+    nd.sigma_t = sigma_t; nd.mu_t = mu_t; nf.sigma_t = (float)sigma_t; nf.mu_t = (float)mu_t;
+    h->net_width[net] = width;
+    // the whole descriptor table (empty slots: n_layers = 0); bank launches pass it to the kernels (ProbIONet::nets)
+    CK(cudaMemcpy(h->bank, h->netd, sizeof(h->netd), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy((char *)h->bank + sizeof(h->netd), h->netf, sizeof(h->netf), cudaMemcpyHostToDevice));
+    if (net != 0) return IGT_OK;
+    // slot 0 is the handle's network of the single-network calls: in DevParams (constant memory) and the tcgen05 copy
+    h->mlp_width = width;
+    h->Pf.n_layers = h->Pd.n_layers = n_layers;
+    for (int l = 0; l <= n_layers; l++) h->Pf.dims[l] = h->Pd.dims[l] = dims[l];
+    for (int l = 0; l < n_layers; l++) {
+        h->Pd.W[l] = nd.W[l]; h->Pd.b[l] = nd.b[l]; h->Pd.Wt[l] = nd.Wt[l];
+        h->Pf.W[l] = nf.W[l]; h->Pf.b[l] = nf.b[l]; h->Pf.Wt[l] = nf.Wt[l];
+    }
+    h->coop_ok = width <= MLP_COOP_W;
     for (int i = 0; i < 36; i++) { h->Pd.Wn[i] = Wn[i]; h->Pf.Wn[i] = (float)Wn[i]; }
     for (int i = 0; i < 6; i++) { h->Pd.mu_f[i] = mu_f[i]; h->Pf.mu_f[i] = (float)mu_f[i]; }
     h->Pd.sigma_t = sigma_t; h->Pd.mu_t = mu_t; h->Pf.sigma_t = (float)sigma_t; h->Pf.mu_t = (float)mu_t;
@@ -548,11 +589,11 @@ int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *cons
                 memcpy(&blob[off], &hi, 2); memcpy(&blob[TC_TILE_BYTES + off], &mid, 2); memcpy(&blob[2 * TC_TILE_BYTES + off], &lo, 2);
             }
         void *dblob, *dw1, *db1, *db2, *dw3;
-        CK(cudaMalloc(&dblob, blob.size())); h->mlp_bufs.push_back(dblob);
-        CK(cudaMalloc(&dw1, w1eff.size() * 4)); h->mlp_bufs.push_back(dw1);
-        CK(cudaMalloc(&db1, MLP_H * 4)); h->mlp_bufs.push_back(db1);
-        CK(cudaMalloc(&db2, MLP_H * 4)); h->mlp_bufs.push_back(db2);
-        CK(cudaMalloc(&dw3, MLP_H * 4)); h->mlp_bufs.push_back(dw3);
+        CK(cudaMalloc(&dblob, blob.size())); bufs.push_back(dblob);
+        CK(cudaMalloc(&dw1, w1eff.size() * 4)); bufs.push_back(dw1);
+        CK(cudaMalloc(&db1, MLP_H * 4)); bufs.push_back(db1);
+        CK(cudaMalloc(&db2, MLP_H * 4)); bufs.push_back(db2);
+        CK(cudaMalloc(&dw3, MLP_H * 4)); bufs.push_back(dw3);
         CK(cudaMemcpy(dblob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dw1, w1eff.data(), w1eff.size() * 4, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(db1, b1eff.data(), MLP_H * 4, cudaMemcpyHostToDevice));
@@ -565,6 +606,41 @@ int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *cons
         CK(cudaFuncSetAttribute(mlp_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
     }
     return IGT_OK;
+}
+
+int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *const *W, const double *const *b,
+                const double *Wn, const double *mu_f, double sigma_t, double mu_t)
+{
+    return igt_set_mlp_at(h, 0, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t);
+}
+
+// Bank calls: every index names a loaded slot (checked on the host before anything is launched, under h->mu, so that
+// a concurrent igt_set_mlp_at cannot empty a slot between the check and the launch); the widest network
+// of the bank sizes the per-thread scratch, and the cooperative evaluation applies when every slot is <= 128 wide.
+static int check_net_idx(igt_handle *h, int n, const int *net_idx, const char *who)
+{
+    for (int i = 0; i < n; i++) {
+        const int k = net_idx[i];
+        if (k < 0 || k >= IGT_MAX_MLP_NETS || h->net_width[k] == 0) {
+            h->err = std::string(who) + ": net_idx[" + std::to_string(i) + "] = " + std::to_string(k) + " names no loaded network";
+            return IGT_EINVAL;
+        }
+    }
+    return IGT_OK;
+}
+static ProbIONet<float> iob_f32(const ProbIONet<double> &io, const igt_handle *h)
+{
+    ProbIONet<float> r;
+    static_cast<ProbIO &>(r) = io;
+    r.net_idx = io.net_idx;
+    r.nets = (const MlpNet<float> *)((const char *)h->bank + sizeof(h->netd));
+    return r;
+}
+static int bank_width(const igt_handle *h)
+{
+    int w = 0;
+    for (int k = 0; k < MAX_MLP_NETS; k++) if (h->net_width[k] > w) w = h->net_width[k];
+    return w;
 }
 
 static int rollout_dev_impl(igt_handle *h, int B, const float *z0, const float *u, const float *curv, float *z,
@@ -622,12 +698,15 @@ int igt_rollout_host(igt_handle *h, int B, const float *z0, const float *u, cons
 static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                           const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init,
                           double *x, double *u, double *cost, double *viol, int *status, int *iters, cudaStream_t st,
-                          const int *warm = nullptr)
+                          const int *warm = nullptr, const int *net_idx = nullptr)
 {
     if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !x || !u || !cost || !viol || !status || !iters) {
         h->err = "igt_solve: null argument"; return IGT_EINVAL;
     }
-    if (nn_ctx && !h->has_mlp) { h->err = "igt_solve: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
+    const bool bank = net_idx != nullptr;
+    if (bank && !nn_ctx) { h->err = "igt_solve: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
+    if (bank && bank_width(h) == 0) { h->err = "igt_solve: net_idx given but no network was loaded"; return IGT_ENOMLP; }
+    if (nn_ctx && !bank && !h->has_mlp) { h->err = "igt_solve: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
     const bool f64 = h->prm.precision == IGT_PREC_F64, obca = obs_psi != nullptr;
     if (obca && !f64) { h->err = "igt_solve: the OBCA collision rows (obs_psi) need precision f64"; return IGT_EINVAL; }
     if (B == 0) return IGT_OK;
@@ -650,10 +729,12 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
     long n_slots = n_cta * bs;
     rc = small ? IGT_OK : grow(h, &h->ws, &h->ws_bytes, (size_t)L.total * n_slots * esz, st);
     if (rc) return rc;
-    const bool use_tc = nn_ctx && h->tc.enabled && h->use_tc && !obca;   // (OBCA + gt_mpc: per-thread value term)
-    const bool use_coop = nn_ctx && !use_tc && f64 && h->coop_ok && !obca;
+    // (OBCA + gt_mpc: per-thread value term; a bank: exact evaluation whatever tensor_core_mlp says)
+    const bool use_tc = nn_ctx && !bank && h->tc.enabled && h->use_tc && !obca;
+    const int width = bank ? bank_width(h) : h->mlp_width;
+    const bool use_coop = nn_ctx && !use_tc && f64 && (bank ? width <= MLP_COOP_W : h->coop_ok) && !obca;
     if (nn_ctx && !use_tc && !use_coop) {                                 // per-thread evaluation: activations in HBM
-        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * h->mlp_width * n_slots * esz, st);
+        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * n_slots * esz, st);
         if (rc) return rc;
     }
     // scheduler block (the work counter), then the cold-start guesses
@@ -670,6 +751,10 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
     ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters };
     io.obs_psi = obs_psi;
     io.warm = warm;
+    ProbIONet<double> iob;   // (the bank kernels' inputs: the f32 one reinterprets nets, same layout)
+    static_cast<ProbIO &>(iob) = io;
+    iob.net_idx = net_idx;
+    iob.nets = (const MlpNet<double> *)h->bank;
     if (!u_init || warm) {
         int gbs = 128, ggs = (B + gbs - 1) / gbs;
         if (obca) guess_kernel<double, true><<<ggs, gbs, 0, st>>>(io, B, guess, cs);
@@ -688,6 +773,25 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
         } else {
             CK(cudaFuncSetAttribute(solve_small_kernel<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
             solve_small_kernel<float, false><<<B, bs, small_smem, st>>>(io, B, sc, guess, cs);
+        }
+    } else if (bank) {
+        // gt_mpc with the network bank: the same kernels' BANK instantiations (problems with a bad index get
+        // IGT_STATUS_BAD_NET); cooperative value term where every network fits it, else per thread
+        double *scr = (double *)h->mlp_scratch;
+        const int rsm = IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * (int)esz : 0;
+        if (use_coop) {
+            const int sm = mlp_coop_bank_smem_bytes<double>(SOLVE_BLOCK);
+            CK(cudaFuncSetAttribute(solve_kernel<double, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+            solve_kernel<double, false, false, true, true><<<gs, bs, sm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, nullptr, width, h->tc, quota, cs);
+        } else if (obca) {
+            CK(cudaFuncSetAttribute(solve_kernel<double, false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
+            solve_kernel<double, false, true, false, true><<<gs, bs, rsm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, scr, width, h->tc, quota, cs);
+        } else if (f64) {
+            CK(cudaFuncSetAttribute(solve_kernel<double, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
+            solve_kernel<double, false, false, false, true><<<gs, bs, rsm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, scr, width, h->tc, quota, cs);
+        } else {
+            CK(cudaFuncSetAttribute(solve_kernel<float, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
+            solve_kernel<float, false, false, false, true><<<gs, bs, rsm, st>>>(iob_f32(iob, h), (float *)h->ws, n_slots, B, sc, guess, (float *)h->mlp_scratch, width, h->tc, quota, cs);
         }
     } else if (use_tc) {
         if (f64) {
@@ -723,29 +827,39 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
     return end_call(h, st, f64 ? 2 : 1);
 }
 
+int igt_solve_ex_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                     const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx, const double *u_init,
+                     double *x, double *u, double *cost, double *viol, int *status, int *iters, void *stream)
+{
+    if (!h) return IGT_EINVAL;
+    std::lock_guard<std::mutex> lk(h->mu);
+    return solve_dev_impl(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, u_init, x, u, cost, viol, status, iters,
+                          (cudaStream_t)stream, nullptr, net_idx);
+}
+
 int igt_solve_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                   const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init, double *x,
                   double *u, double *cost, double *viol, int *status, int *iters, void *stream)
 {
-    if (!h) return IGT_EINVAL;
-    std::lock_guard<std::mutex> lk(h->mu);
-    return solve_dev_impl(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, u_init, x, u, cost, viol, status, iters, (cudaStream_t)stream);
+    return igt_solve_ex_dev(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, nullptr, u_init, x, u, cost, viol, status, iters, stream);
 }
 
 // Host-pointer solve.  All inputs travel in ONE host-to-device copy and all outputs in ONE device-to-host copy on
 // the handle's own non-blocking stream: small batches (a closed-loop step solves B = 2) are packed into pinned
 // staging blocks first; large batches are copied array by array straight from the caller's (ideally pinned)
 // memory -- packing 100 MB on the host would cost more than the copies.
-int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
-                   const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init, double *x,
-                   double *u, double *cost, double *viol, int *status, int *iters)
+int igt_solve_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                      const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx, const double *u_init,
+                      double *x, double *u, double *cost, double *viol, int *status, int *iters)
 {
     if (!h) return IGT_EINVAL;
     if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !x || !u || !cost || !viol || !status || !iters) {
         h->err = "igt_solve: null argument"; return IGT_EINVAL;
     }
+    if (net_idx && !nn_ctx) { h->err = "igt_solve: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
     if (B == 0) return IGT_OK;
     std::lock_guard<std::mutex> lk(h->mu);
+    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_solve"); if (rc0) return rc0; }
     CK(cudaSetDevice(h->device));
     if (!h->hstream) CK(cudaStreamCreateWithFlags(&h->hstream, cudaStreamNonBlocking));
     cudaStream_t st = h->hstream;
@@ -757,8 +871,10 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
     size_t n_ui = u_init ? nb * N * 2 : 0, n_x = nb * (N + 1) * 7, n_u = nb * N * 2, n_op = obs_psi ? nb * (N + 1) : 0;
     size_t n_in = n_x0 + n_up + n_c + n_o + n_ctx + n_ui + n_op, n_out = n_x + n_u + 2 * nb;
     size_t in_bytes = n_in * 8, out_bytes = n_out * 8 + 2 * nb * 4, total = in_bytes + out_bytes;
-    rc = grow(h, &h->stage, &h->stage_bytes, total, st);
+    rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), st);
     if (rc) return rc;
+    int *dnet = (int *)((char *)h->stage + total);                     // net_idx: after the outputs, copied on its own
+    if (net_idx) CK(cudaMemcpyAsync(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice, st));
     double *d = (double *)h->stage;
     double *dx0 = d, *dup = dx0 + n_x0, *dc = dup + n_up, *dob = dc + n_c, *dctx = dob + n_o, *dui = dctx + n_ctx;
     double *dop = dui + n_ui;
@@ -790,7 +906,7 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
         if (obs_psi) CK(cudaMemcpyAsync(dop, obs_psi, n_op * 8, cudaMemcpyHostToDevice, st));
     }
     rc = solve_dev_impl(h, B, dx0, dup, dc, dob, obs_psi ? dop : nullptr, nn_ctx ? dctx : nullptr, u_init ? dui : nullptr,
-                        dx, du, dcost, dviol, dst, dit, st);
+                        dx, du, dcost, dviol, dst, dit, st, nullptr, net_idx ? dnet : nullptr);
     if (rc) return rc;
     if (packed) {
         char *q = (char *)h->pin + in_bytes;
@@ -814,15 +930,24 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
     return IGT_OK;
 }
 
-int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
-                  const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u, double *cost,
-                  double *viol, double *z)
+int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                   const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init, double *x,
+                   double *u, double *cost, double *viol, int *status, int *iters)
+{
+    return igt_solve_ex_host(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, nullptr, u_init, x, u, cost, viol, status, iters);
+}
+
+int igt_eval_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                     const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx, const double *u,
+                     double *cost, double *viol, double *z)
 {
     if (!h) return IGT_EINVAL;
     if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !u || !cost || !viol) { h->err = "igt_eval: null argument"; return IGT_EINVAL; }
-    if (nn_ctx && !h->has_mlp) { h->err = "igt_eval: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
+    if (net_idx && !nn_ctx) { h->err = "igt_eval: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
+    if (nn_ctx && !net_idx && !h->has_mlp) { h->err = "igt_eval: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
     if (B == 0) return IGT_OK;
     std::lock_guard<std::mutex> lk(h->mu);
+    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_eval"); if (rc0) return rc0; }
     int cs = 0;
     { int rc0 = begin_call(h, nullptr); if (rc0) return rc0; }
     const int N = h->prm.N;
@@ -830,9 +955,12 @@ int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, 
     size_t n_x0 = nb * 7, n_up = nb * 2, n_c = nb * 3, n_o = nb * (N + 1) * 2, n_ctx = nn_ctx ? nb * 4 : 0;
     size_t n_u = nb * N * 2, n_z = nb * (N + 1) * 7, n_op = obs_psi ? nb * (N + 1) : 0;
     size_t total = (n_x0 + n_up + n_c + n_o + n_ctx + n_u + n_z + 2 * nb + n_op) * 8;
-    int rc = grow(h, &h->stage, &h->stage_bytes, total, nullptr);
+    int rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), nullptr);
     if (rc) return rc;
-    if (nn_ctx) { rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * h->mlp_width * B * 8, nullptr); if (rc) return rc; }
+    const int width = net_idx ? bank_width(h) : h->mlp_width;
+    if (nn_ctx) { rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * B * 8, nullptr); if (rc) return rc; }
+    int *dnet = (int *)((char *)h->stage + total);
+    if (net_idx) CK(cudaMemcpy(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice));
     double *d = (double *)h->stage;
     double *dx0 = d, *dup = dx0 + n_x0, *dc = dup + n_up, *dob = dc + n_c, *dctx = dob + n_o, *du = dctx + n_ctx;
     double *dz = du + n_u, *dcost = dz + n_z, *dviol = dcost + nb, *dop = dviol + nb;
@@ -846,8 +974,12 @@ int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, 
     rc = acquire_cslot(h, 1, nullptr, &cs);
     if (rc) return rc;
     int bs = 128, gs = (B + bs - 1) / bs;
-    eval_kernel<<<gs, bs>>>(B, dx0, dup, dc, dob, nn_ctx ? dctx : nullptr, du, dcost, dviol, dz,
-                            nn_ctx ? (double *)h->mlp_scratch : nullptr, h->mlp_width, cs, obs_psi ? dop : nullptr);
+    if (net_idx)
+        eval_kernel<true><<<gs, bs>>>(B, dx0, dup, dc, dob, dctx, du, dcost, dviol, dz, (double *)h->mlp_scratch, width, cs,
+                                      obs_psi ? dop : nullptr, dnet, (const MlpNet<double> *)h->bank);
+    else
+        eval_kernel<false><<<gs, bs>>>(B, dx0, dup, dc, dob, nn_ctx ? dctx : nullptr, du, dcost, dviol, dz,
+                                       nn_ctx ? (double *)h->mlp_scratch : nullptr, h->mlp_width, cs, obs_psi ? dop : nullptr, nullptr, nullptr);
     h->launches++;
     CK(cudaGetLastError());
     rc = end_call(h, nullptr, 2);
@@ -856,6 +988,13 @@ int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, 
     CK(cudaMemcpy(viol, dviol, nb * 8, cudaMemcpyDeviceToHost));
     if (z) CK(cudaMemcpy(z, dz, n_z * 8, cudaMemcpyDeviceToHost));
     return IGT_OK;
+}
+
+int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                  const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u, double *cost,
+                  double *viol, double *z)
+{
+    return igt_eval_ex_host(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, nullptr, u, cost, viol, z);
 }
 
 int igt_measure_fma_peak(igt_handle *h, int precision, double *tflops)
@@ -888,23 +1027,32 @@ int igt_measure_fma_peak(igt_handle *h, int precision, double *tflops)
     return IGT_OK;
 }
 
-int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx, double *out,
-                       int use_tensor_cores)
+int igt_mlp_value_ex_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx, const int *net_idx,
+                          double *out, int use_tensor_cores)
 {
     if (!h) return IGT_EINVAL;
     if (B < 0 || !sN || !vN || !nn_ctx || !out) { h->err = "igt_mlp_value: null argument"; return IGT_EINVAL; }
-    if (!h->has_mlp) { h->err = "igt_mlp_value: igt_set_mlp was never called"; return IGT_ENOMLP; }
+    if (net_idx && use_tensor_cores != 0 && use_tensor_cores != 2) {
+        h->err = "igt_mlp_value: with net_idx the mode must be 0 (per thread) or 2 (cooperative)"; return IGT_EINVAL;
+    }
+    std::lock_guard<std::mutex> lk(h->mu);   // (the bank state below is read under the lock: igt_set_mlp_at takes it)
+    const int width = net_idx ? bank_width(h) : h->mlp_width;
+    if (net_idx ? width == 0 : !h->has_mlp) { h->err = "igt_mlp_value: igt_set_mlp was never called"; return IGT_ENOMLP; }
     if (use_tensor_cores == 1 && !h->tc.enabled) { h->err = "igt_mlp_value: tensor-core path needs a 6-128-128-1 network"; return IGT_EINVAL; }
-    if (use_tensor_cores == 2 && !h->coop_ok) { h->err = "igt_mlp_value: the cooperative evaluation needs layers <= 128 wide"; return IGT_EINVAL; }
+    if (use_tensor_cores == 2 && (net_idx ? width > MLP_COOP_W : !h->coop_ok)) {
+        h->err = "igt_mlp_value: the cooperative evaluation needs layers <= 128 wide"; return IGT_EINVAL;
+    }
     if (B == 0) return IGT_OK;
-    std::lock_guard<std::mutex> lk(h->mu);
+    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_mlp_value"); if (rc0) return rc0; }
     int cs = 0;
     int rc = begin_call(h, nullptr);
     if (rc) return rc;
     size_t nb = (size_t)B, total = (nb * 2 + nb * 4 + nb * 6) * 8;
-    rc = grow(h, &h->stage, &h->stage_bytes, total, nullptr);
+    rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), nullptr);
     if (rc) return rc;
     double *ds = (double *)h->stage, *dv = ds + nb, *dc = dv + nb, *dout = dc + nb * 4;
+    int *dnet = (int *)((char *)h->stage + total);
+    if (net_idx) CK(cudaMemcpy(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(ds, sN, nb * 8, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dv, vN, nb * 8, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dc, nn_ctx, nb * 32, cudaMemcpyHostToDevice));
@@ -913,19 +1061,26 @@ int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN,
         if (rc) return rc;
         int grid = (int)((nb + 255) / 256);
         if (grid > h->n_sm) grid = h->n_sm;
-        const int sm = mlp_coop_smem_bytes<double>(256);
-        CK(cudaFuncSetAttribute(mlp_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-        mlp_coop_kernel<<<grid, 256, sm>>>(B, ds, dv, dc, dout, cs);
+        if (net_idx) {
+            const int sm = mlp_coop_bank_smem_bytes<double>(256);
+            CK(cudaFuncSetAttribute(mlp_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+            mlp_coop_kernel<true><<<grid, 256, sm>>>(B, ds, dv, dc, dout, cs, dnet, (const MlpNet<double> *)h->bank);
+        } else {
+            const int sm = mlp_coop_smem_bytes<double>(256);
+            CK(cudaFuncSetAttribute(mlp_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+            mlp_coop_kernel<false><<<grid, 256, sm>>>(B, ds, dv, dc, dout, cs, nullptr, nullptr);
+        }
     } else if (use_tensor_cores) {
         int grid = (int)((nb + 255) / 256);
         if (grid > h->n_sm) grid = h->n_sm;
         mlp_tc_kernel<<<grid, 256, TC_SMEM_BYTES>>>(h->tc, B, ds, dv, dc, dout);
     } else {
-        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * h->mlp_width * nb * 8, nullptr);
+        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * nb * 8, nullptr);
         if (rc) return rc;
         rc = acquire_cslot(h, 1, nullptr, &cs);
         if (rc) return rc;
-        mlp_ref_kernel<<<(int)((nb + 127) / 128), 128>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, h->mlp_width, cs);
+        if (net_idx) mlp_ref_kernel<true><<<(int)((nb + 127) / 128), 128>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, width, cs, dnet, (const MlpNet<double> *)h->bank);
+        else mlp_ref_kernel<false><<<(int)((nb + 127) / 128), 128>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, width, cs, nullptr, nullptr);
     }
     h->launches++;
     CK(cudaGetLastError());
@@ -933,6 +1088,12 @@ int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN,
     if (rc) return rc;
     CK(cudaMemcpy(out, dout, nb * 48, cudaMemcpyDeviceToHost));
     return IGT_OK;
+}
+
+int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx, double *out,
+                       int use_tensor_cores)
+{
+    return igt_mlp_value_ex_host(h, B, sN, vN, nn_ctx, nullptr, out, use_tensor_cores);
 }
 
 
@@ -979,9 +1140,9 @@ int igt_debug_round_phases(igt_handle *h, int *ph512x12)
 }
 #endif
 
-int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
-                         const double *z0, const double *u_prev0, const double *enc, double *z_cl, double *u_cl,
-                         int *solved, float *step_ms)
+int igt_episode_run_ex_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
+                            const double *z0, const double *u_prev0, const double *enc, const int *net_idx, double *z_cl,
+                            double *u_cl, int *solved, float *step_ms)
 {
     if (!h) return IGT_EINVAL;
     if (E < 0 || steps < 1 || !route_desc || !curv || !z0 || !u_prev0 || !enc || !z_cl || !u_cl || !solved) {
@@ -993,9 +1154,11 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double
     const int gt_mpc = (mode & IGT_EPISODE_GT_MPC) != 0;
     const bool obca = (mode & IGT_EPISODE_OBCA) != 0;
     if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_episode_run: needs precision f64"; return IGT_EINVAL; }
-    if (gt_mpc && !h->has_mlp) { h->err = "igt_episode_run: gt_mpc needs igt_set_mlp"; return IGT_ENOMLP; }
+    if (net_idx && !gt_mpc) { h->err = "igt_episode_run: net_idx needs the IGT_EPISODE_GT_MPC mode bit"; return IGT_EINVAL; }
+    if (gt_mpc && !net_idx && !h->has_mlp) { h->err = "igt_episode_run: gt_mpc needs igt_set_mlp"; return IGT_ENOMLP; }
     if (E == 0) return IGT_OK;
     std::lock_guard<std::mutex> lk(h->mu);
+    if (net_idx) { const int rc0 = check_net_idx(h, E, net_idx, "igt_episode_run"); if (rc0) return rc0; }
     CK(cudaSetDevice(h->device));
     if (!h->hstream) CK(cudaStreamCreateWithFlags(&h->hstream, cudaStreamNonBlocking));
     cudaStream_t st = h->hstream;
@@ -1008,7 +1171,7 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double
                  n_ctx = nb * 4, n_ui = nb * N * 2, n_zcl = nb * (T + 1) * 7, n_ucl = nb * T * 2, n_x = nb * (N + 1) * 7,
                  n_u = nb * N * 2, n_op = obca ? nb * (N + 1) : 0;
     const size_t n_dbl = n_z + n_up + n_cv + n_rd + n_en + n_obs + n_ctx + n_ui + n_zcl + n_ucl + 2 * (n_x + n_u + 2 * nb) + n_op;
-    const size_t n_int = nb /*warm*/ + nb /*prev_ok*/ + nb * T /*solved*/ + 2 * 2 * nb /*status, iters x2*/;
+    const size_t n_int = nb /*warm*/ + nb /*prev_ok*/ + nb * T /*solved*/ + 2 * 2 * nb /*status, iters x2*/ + (net_idx ? nb : 0);
     rc = grow(h, &h->episode, &h->episode_bytes, n_dbl * 8 + n_int * 4, st);
     if (rc) return rc;
     double *d = (double *)h->episode;
@@ -1025,6 +1188,13 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double
     eb.warm = ip; ip += nb; eb.prev_ok = ip; ip += nb; eb.solved = ip; ip += nb * T;
     int *pst[2], *pit[2];
     for (int i = 0; i < 2; i++) { pst[i] = ip; ip += nb; pit[i] = ip; ip += nb; }
+    int *dnet = net_idx ? ip : nullptr;
+    std::vector<int> veh_net;
+    if (net_idx) {   // both vehicles of episode e plan with network net_idx[e]: expanded once, the glue kernels never see it
+        veh_net.resize(nb);
+        for (int b = 0; b < B; b++) veh_net[b] = net_idx[b / 2];
+        CK(cudaMemcpyAsync(dnet, veh_net.data(), nb * 4, cudaMemcpyHostToDevice, st));
+    }
     CK(cudaMemcpyAsync(eb.z, z0, n_z * 8, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(eb.u_prev, u_prev0, n_up * 8, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(dcv, curv, n_cv * 8, cudaMemcpyHostToDevice, st));
@@ -1043,7 +1213,7 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double
         else episode_pre_kernel<false><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
         h->launches++;
         rc = solve_dev_impl(h, B, eb.z, eb.u_prev, eb.curv, eb.obs, eb.obs_psi, gt_mpc ? eb.ctx : nullptr, eb.u_init, px[cur], pu[cur],
-                            pcost[cur], pviol[cur], pst[cur], pit[cur], st, eb.warm);
+                            pcost[cur], pviol[cur], pst[cur], pit[cur], st, eb.warm, dnet);
         if (rc) return rc;
         rc = acquire_cslot(h, 1, st, &cs);
         if (rc) return rc;
@@ -1063,6 +1233,13 @@ int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double
         for (auto &e : ev) cudaEventDestroy(e);
     }
     return IGT_OK;
+}
+
+int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
+                         const double *z0, const double *u_prev0, const double *enc, double *z_cl, double *u_cl,
+                         int *solved, float *step_ms)
+{
+    return igt_episode_run_ex_host(h, E, steps, mode, route_desc, curv, z0, u_prev0, enc, nullptr, z_cl, u_cl, solved, step_ms);
 }
 
 int igt_set_option(igt_handle *h, const char *name, double value)

@@ -11,6 +11,12 @@
 // first version read 131 KB of weights from L1 / L2 per evaluation and layer and ran at a sixth of the FP64 rate).
 // Same operation order per output as mlp_eval_thread: bit-identical results (tests/hostsim runs that one on the
 // CPU).  Any network with layer widths <= MLP_COOP_W.
+//
+// Network bank (mlp_coop_eval_bank): every request names one of up to MAX_MLP_NETS networks.  The requests are
+// compacted by network instead (a counting sort, thread order kept inside a group), and each non-empty group runs the
+// same waves with its own descriptor, biases and output layer staged in shared memory.  The operation order per output
+// is unchanged, so a request's result is bit-identical to the single-network evaluation of its network, whatever
+// shares its wave.
 #pragma once
 #include <cstdint>
 
@@ -27,6 +33,14 @@ constexpr int mlp_coop_smem_bytes(int block)
 {
     return (int)sizeof(T) * (block * (COOP_ITEM + COOP_ROWS) + (block / 32) * COOP_E * COOP_ROWS * MLP_COOP_W + 2 * COOP_TI * MLP_COOP_W +
                              (MAX_MLP_LAYERS + 1) * MLP_COOP_W) + 4 * (block + 32);
+}
+// the bank variant appends the current group's descriptor and the per-warp group counts [MAX_MLP_NETS][32]
+template <typename T>
+constexpr int mlp_coop_desc_bytes() { return (int)((sizeof(MlpNet<T>) + 15) / 16 * 16); }
+template <typename T>
+constexpr int mlp_coop_bank_smem_bytes(int block)
+{
+    return mlp_coop_smem_bytes<T>(block) + mlp_coop_desc_bytes<T>() + 4 * MAX_MLP_NETS * 32;
 }
 
 #ifdef __CUDACC__
@@ -77,36 +91,26 @@ __device__ __forceinline__ void coop_tile_fma(T (&acc)[COOP_E][4][6], const T *t
     }
 }
 
-// CTA-uniform call (like mlp_tc_eval): every thread passes its own request (valid = false: none) and gets
-// out[6] = (V, dV/ds, dV/dv, d2V/dss, d2V/dsv, d2V/dvv), already scaled by sigma_t (+ mu_t on V).
-template <typename T>
-__device__ __noinline__ void mlp_coop_eval(const DevParams<T> &P, uint8_t *smem, bool valid, T sN, T vN, const T *ctx, T *out)
+// biases of every layer and the output layer's weights of network P -> shared memory (NP: DevParams<T> or MlpNet<T>)
+template <typename T, typename NP>
+__device__ __forceinline__ void coop_stage(const NP &P, T *bias, T *wlast)
 {
-    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nthr = blockDim.x, nw = nthr >> 5;
-    T *items = reinterpret_cast<T *>(smem);                       // [nthr][8]: sN, vN, ctx[4]
-    T *res = items + nthr * COOP_ITEM;                            // [nthr][6]
-    T *act = res + nthr * COOP_ROWS + warp * (E * COOP_ROWS * W); // this warp's [E][6][W] activation rows (updated in place)
-    T *tiles = res + nthr * COOP_ROWS + nw * (E * COOP_ROWS * W); // [2][TI][W]
-    T *bias = tiles + 2 * TI * W, *wlast = bias + MAX_MLP_LAYERS * W;   // [layers][W], [W]: staged once per call
-    int *list = reinterpret_cast<int *>(wlast + W), *wcnt = list + nthr;
+    constexpr int W = MLP_COOP_W;
+    const int tid = threadIdx.x, nthr = blockDim.x;
     for (int idx = tid; idx < (P.n_layers + 1) * W; idx += nthr) {
         const int l = idx / W, o = idx - l * W;
         if (l < P.n_layers) { if (o < P.dims[l + 1]) bias[idx] = P.b[l][o]; }
         else if (o < P.dims[P.n_layers - 1]) wlast[o] = P.Wt[P.n_layers - 1][o];
     }
-    for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
-    items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
-#pragma unroll
-    for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
-    // the valid requests in thread order
-    const unsigned vm = __ballot_sync(0xffffffffu, valid);
-    if (lane == 0) wcnt[warp] = __popc(vm);
-    __syncthreads();
-    int base = 0, nv = 0;
-    for (int i = 0; i < nw; i++) { const int c = wcnt[i]; if (i < warp) base += c; nv += c; }
-    if (valid) list[base + __popc(vm & ((1u << lane) - 1u))] = tid;
-    __syncthreads();
+}
+
+// the waves of the nv requests list[0 .. nv) through network P (staged by coop_stage); CTA-uniform
+template <typename T, typename NP>
+__device__ __forceinline__ void coop_waves(const NP &P, const T *items, T *res, T *act, T *tiles, const T *bias, const T *wlast,
+                                           const int *list, int nv)
+{
+    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
     for (int wave0 = 0; wave0 < nv; wave0 += nw * E) {             // CTA-uniform
         int ev[E];
 #pragma unroll
@@ -206,7 +210,94 @@ __device__ __noinline__ void mlp_coop_eval(const DevParams<T> &P, uint8_t *smem,
             }
         }
     }
+}
+
+// CTA-uniform call (like mlp_tc_eval): every thread passes its own request (valid = false: none) and gets
+// out[6] = (V, dV/ds, dV/dv, d2V/dss, d2V/dsv, d2V/dvv), already scaled by sigma_t (+ mu_t on V).
+template <typename T>
+__device__ __noinline__ void mlp_coop_eval(const DevParams<T> &P, uint8_t *smem, bool valid, T sN, T vN, const T *ctx, T *out)
+{
+    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nthr = blockDim.x, nw = nthr >> 5;
+    T *items = reinterpret_cast<T *>(smem);                       // [nthr][8]: sN, vN, ctx[4]
+    T *res = items + nthr * COOP_ITEM;                            // [nthr][6]
+    T *act = res + nthr * COOP_ROWS + warp * (E * COOP_ROWS * W); // this warp's [E][6][W] activation rows (updated in place)
+    T *tiles = res + nthr * COOP_ROWS + nw * (E * COOP_ROWS * W); // [2][TI][W]
+    T *bias = tiles + 2 * TI * W, *wlast = bias + MAX_MLP_LAYERS * W;   // [layers][W], [W]: staged once per call
+    int *list = reinterpret_cast<int *>(wlast + W), *wcnt = list + nthr;
+    coop_stage(P, bias, wlast);
+    for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
+    items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
+#pragma unroll
+    for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+    // the valid requests in thread order
+    const unsigned vm = __ballot_sync(0xffffffffu, valid);
+    if (lane == 0) wcnt[warp] = __popc(vm);
     __syncthreads();
+    int base = 0, nv = 0;
+    for (int i = 0; i < nw; i++) { const int c = wcnt[i]; if (i < warp) base += c; nv += c; }
+    if (valid) list[base + __popc(vm & ((1u << lane) - 1u))] = tid;
+    __syncthreads();
+    coop_waves(P, items, res, act, tiles, bias, wlast, list, nv);
+    __syncthreads();
+    if (valid) {
+#pragma unroll
+        for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];
+    }
+    __syncthreads();
+}
+
+// The same over a network bank: request t uses nets[net] (0 <= net < MAX_MLP_NETS, a loaded slot: the callers check).
+// Shared memory: mlp_coop_bank_smem_bytes.
+template <typename T>
+__device__ __noinline__ void mlp_coop_eval_bank(const MlpNet<T> *nets, uint8_t *smem, bool valid, int net, T sN, T vN, const T *ctx, T *out)
+{
+    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nthr = blockDim.x, nw = nthr >> 5;
+    T *items = reinterpret_cast<T *>(smem);
+    T *res = items + nthr * COOP_ITEM;
+    T *act = res + nthr * COOP_ROWS + warp * (E * COOP_ROWS * W);
+    T *tiles = res + nthr * COOP_ROWS + nw * (E * COOP_ROWS * W);
+    T *bias = tiles + 2 * TI * W, *wlast = bias + MAX_MLP_LAYERS * W;   // staged once per group
+    int *list = reinterpret_cast<int *>(wlast + W);
+    MlpNet<T> *desc = reinterpret_cast<MlpNet<T> *>(smem + mlp_coop_smem_bytes<T>(nthr));   // the current group's network
+    int *gcnt = reinterpret_cast<int *>(reinterpret_cast<uint8_t *>(desc) + mlp_coop_desc_bytes<T>());   // [net][warp]
+    for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
+    items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
+#pragma unroll
+    for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+    // counting sort of the valid requests by network: group g holds its requests in thread order
+    int rank = 0;
+    for (int g = 0; g < MAX_MLP_NETS; g++) {
+        const bool mine = valid && net == g;
+        const unsigned m = __ballot_sync(0xffffffffu, mine);
+        if (lane == 0) gcnt[g * nw + warp] = __popc(m);
+        if (mine) rank = __popc(m & ((1u << lane) - 1u));
+    }
+    __syncthreads();
+    if (valid && (unsigned)net < (unsigned)MAX_MLP_NETS) {
+        int base = rank;
+        for (int g = 0; g <= net; g++)
+            for (int i = 0; i < nw; i++) if (g < net || i < warp) base += gcnt[g * nw + i];
+        list[base] = tid;
+    }
+    __syncthreads();
+    for (int g = 0, start = 0; g < MAX_MLP_NETS; g++) {           // CTA-uniform
+        int n = 0;
+        for (int i = 0; i < nw; i++) n += gcnt[g * nw + i];
+        if (n == 0) continue;
+        {   // descriptor -> shared memory (the previous group's waves are done with it: barrier at their end)
+            const int *src = reinterpret_cast<const int *>(nets + g);
+            int *dst = reinterpret_cast<int *>(desc);
+            for (int i = tid; i < (int)(sizeof(MlpNet<T>) / 4); i += nthr) dst[i] = src[i];
+        }
+        __syncthreads();
+        coop_stage(*desc, bias, wlast);
+        __syncthreads();
+        coop_waves(*desc, items, res, act, tiles, bias, wlast, list + start, n);
+        __syncthreads();
+        start += n;
+    }
     if (valid) {
 #pragma unroll
         for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];

@@ -62,7 +62,19 @@ constexpr int MAX_ALPHA = 6, NBUF = MAX_ALPHA + 1;
 constexpr int NTC = 8;     // per-candidate scalars: finite flag, cost, terminal value term and its 5 derivatives
 IGT_HD constexpr int cand_buf(int cur, int j) { return j < cur ? j : j + 1; }
 constexpr int MAX_MLP_LAYERS = 5;
+constexpr int MAX_MLP_NETS = 8;   // value networks of one handle's bank (IGT_MAX_MLP_NETS)
 constexpr int N_GUESS = 5;
+
+// One value network: the network fields of DevParams, same names (the value-term code is written against either).
+// A handle's bank is a table of MAX_MLP_NETS of these in global memory; n_layers == 0 marks an empty slot.
+template <typename T>
+struct MlpNet {
+    int n_layers;
+    int dims[MAX_MLP_LAYERS + 1];
+    T Wn[36], mu_f[6], sigma_t, mu_t;
+    const T *W[MAX_MLP_LAYERS], *b[MAX_MLP_LAYERS];
+    const T *Wt[MAX_MLP_LAYERS];
+};
 
 template <typename T>
 struct DevParams {
@@ -229,6 +241,17 @@ struct ProbIO {
     const double *obs_psi = nullptr;                         // [B,N+1] obstacle heading forecast: OBCA collision rows
     const int *warm = nullptr;                               // [B] per-problem warm-start flags (with u_init); null: all warm
 };
+// inputs of a bank solve (the BANK kernels): a type of its own, so that the other kernels' parameters stay as they are
+template <typename T>
+struct ProbIONet : ProbIO {
+    const int *net_idx = nullptr;                            // [B] value network of each problem in nets
+    const MlpNet<T> *nets = nullptr;                         // the handle's bank: [MAX_MLP_NETS] descriptors
+    // a bank index that may be dereferenced: 0..MAX_MLP_NETS-1 and a loaded slot
+    IGT_HD bool net_ok(int k) const { return (unsigned)k < (unsigned)MAX_MLP_NETS && nets[k].n_layers > 0; }
+};
+// (only for an io that is a ProbIONet<T>: the BANK code paths)
+template <typename T>
+IGT_HD const ProbIONet<T> &bank_io(const ProbIO &io) { return static_cast<const ProbIONet<T> &>(io); }
 
 // ------------------------------------------------------------------ dynamics -----------
 IGT_HD void sincos_t(float x, float *s, float *c) { sincosf(x, s, c); }
@@ -534,10 +557,10 @@ struct TermVal { T V, gs, gv, Hss, Hsv, Hvv; };
 
 // gt_mpc terminal value (mpc.py:326-354, :367-369; model.py:14-67) on CUDA cores, one
 // problem per thread: value + first and second forward tangents in (s_N, v_N).
-// Scratch: two [6][width] slabs of the caller's workspace.
-template <typename T>
-IGT_HDN void mlp_eval_thread(const DevParams<T> &P, T sN, T vN, const T *ctx, T *ha, T *hb, int width,
-                             TermVal<T> &out, bool want_deriv)
+// Scratch: two [6][width] slabs of the caller's workspace.  NP: DevParams<T> (the handle's network, mlp_eval_thread) or
+// MlpNet<T> (a bank entry, mlp_eval_thread_net).
+template <typename T, typename NP>
+IGT_HD void mlp_eval_body(const NP &P, T sN, T vN, const T *ctx, T *ha, T *hb, int width, TermVal<T> &out, bool want_deriv)
 {
     T xN[6] = { ctx[0], ctx[1], ctx[2], sN - ctx[0], vN - ctx[1], ctx[3] - ctx[2] };
     const int R = want_deriv ? 6 : 1;
@@ -584,6 +607,18 @@ IGT_HDN void mlp_eval_thread(const DevParams<T> &P, T sN, T vN, const T *ctx, T 
     } else {
         out.gs = out.gv = out.Hss = out.Hsv = out.Hvv = T(0);
     }
+}
+template <typename T>
+IGT_HDN void mlp_eval_thread(const DevParams<T> &P, T sN, T vN, const T *ctx, T *ha, T *hb, int width,
+                             TermVal<T> &out, bool want_deriv)
+{
+    mlp_eval_body(P, sN, vN, ctx, ha, hb, width, out, want_deriv);
+}
+template <typename T>
+IGT_HDN void mlp_eval_thread_net(const MlpNet<T> &P, T sN, T vN, const T *ctx, T *ha, T *hb, int width,
+                                 TermVal<T> &out, bool want_deriv)
+{
+    mlp_eval_body(P, sN, vN, ctx, ha, hb, width, out, want_deriv);
 }
 
 // sum of log(y_i) with one log per LOGCHUNK factors (slacks lie in [1e-11, 1e3], so a product of
@@ -1052,9 +1087,14 @@ IGT_HD void node_phase3(const DevParams<T> &P, const W &w, const NodeCtx<T> &c, 
 }
 
 // ------------------------------------------------------------------ the solver ---------
-template <typename T, typename W = Ws<T>>
-struct Solver {
+// BANK: gt_mpc problems take their value network from the bank, nets[net_idx[p]] of ProbIONet.  The pointer lives in a base
+// that is empty without BANK, so the other solvers keep their layout (and their local-memory footprint).
+template <typename T, bool BANK> struct SolverNet { const MlpNet<T> *net; };   // this problem's network
+template <typename T> struct SolverNet<T, false> {};
+template <typename T, typename W = Ws<T>, bool BANK = false>
+struct Solver : SolverNet<T, BANK> {
     static constexpr bool obca = W::obca;
+    static constexpr bool bank = BANK;
     const DevParams<T> &P;
     W w;
     T x0[NZ], uprev[2], curv[3], ctx[4];
@@ -1095,6 +1135,8 @@ struct Solver {
     {
         if (!gt) {
             t.V = sN - x0[IS]; t.gs = T(1); t.gv = T(0); t.Hss = t.Hsv = t.Hvv = T(0);
+        } else if constexpr (BANK) {
+            mlp_eval_thread_net(*this->net, sN, vN, ctx, mlp_scratch, mlp_scratch + 6 * mlp_width, mlp_width, t, want_deriv);
         } else {
             mlp_eval_thread(P, sN, vN, ctx, mlp_scratch, mlp_scratch + 6 * mlp_width, mlp_width, t, want_deriv);
         }
@@ -1218,6 +1260,14 @@ struct Solver {
         const int N = P.N;
         load_inputs(io, p, has_ctx);
         cur = 0; status = 1; iters = 0; ls = 0; need_back = 2; done = false; trials = 0;
+        if constexpr (BANK) {   // an index outside the bank or naming an empty slot: no solve, never dereferenced
+            if (gt) {
+                const ProbIONet<T> &bio = bank_io<T>(io);
+                const int k = bio.net_idx[p];
+                if (!bio.net_ok(k)) { status = 7; done = true; return false; }
+                this->net = bio.nets + k;
+            }
+        }
         mu = warm ? P.mu0_warm : P.mu0; reg = T(0); alpha = T(1); reg_hint = T(0);
         const T y_min = warm ? P.y_init_min_warm : P.y_init_min;
         {   // rows on x0 alone: mpc.py:316-317 and :298-299 at k = 0
@@ -1671,10 +1721,10 @@ struct Solver {
     IGT_HD void write_out(const ProbIO &io, long p)
     {
         const int N = P.N, b = cur;
-        if (status == 2) {
+        if (status == 2 || (BANK && status == 7)) {
             for (int i = 0; i < (N + 1) * NZ; i++) io.x[p * (N + 1) * NZ + i] = NAN;
             for (int i = 0; i < N * 2; i++) io.u[p * N * 2 + i] = NAN;
-            io.cost[p] = NAN; io.viol[p] = INFINITY; io.status[p] = 2; io.iters[p] = 0;
+            io.cost[p] = NAN; io.viol[p] = INFINITY; io.status[p] = BANK ? status : 2; io.iters[p] = 0;
             return;
         }
         T m = T(0);
@@ -1795,10 +1845,13 @@ __device__ __forceinline__ int cta_list_build(bool need, long bound, const S &sv
 // The item loops of the CTA-wide phases live in functions of their own (not inlined): each gets its own
 // register allocation, so that the spills of one phase do not leak into the others or into the
 // per-problem sweeps of the main loop.  The parameters come from constant memory through ConstP<T>,
-// which the translation unit defines.
+// which the translation unit defines.  BANK does not change what they compute: it only gives the bank kernels
+// instantiations of their own, so that each instantiation keeps a single calling kernel (NVVM then binds the work list
+// argument to that kernel's __shared__ NodeList instead of passing a generic pointer) and the other kernels compile as
+// they would without the bank.
 template <typename T> struct ConstP;
 
-template <typename T, int PHASE, int STRIDE, bool OBCA, bool RSTG>
+template <typename T, int PHASE, int STRIDE, bool OBCA, bool RSTG, bool BANK>
 __device__ __noinline__ void phase_items(T *ws_base, const NodeList<T> *nl, int n, int n_spec)
 {
     const DevParams<T> &P = ConstP<T>::get(nl->cslot);
@@ -1831,7 +1884,7 @@ __device__ __forceinline__ void node_phase_cta(const DevParams<T> &P, T *ws_base
                                                long bound, const S &sv, NodeList<T> &nl)
 {
     const int n = cta_list_build(need, bound, sv, nl);
-    if (n > 0) phase_items<T, PHASE, STRIDE, S::obca, RSTG>(ws_base, &nl, n, 1);
+    if (n > 0) phase_items<T, PHASE, STRIDE, S::obca, RSTG, S::bank>(ws_base, &nl, n, 1);
     __syncthreads();
 }
 
@@ -1862,10 +1915,10 @@ __device__ __forceinline__ int trial_phase_cta(const DevParams<T> &P, T *ws_base
     // IGT_SPEC_BUDGET: most candidates (problems x halvings) evaluated at once; the default fills the CTA's threads
     int n_spec = 1;
     if (speculate) { n_spec = IGT_SPEC_BUDGET / n; n_spec = n_spec < 1 ? 1 : (n_spec > P.n_alpha ? P.n_alpha : n_spec); }
-    phase_items<T, 3, STRIDE, S::obca, false>(ws_base, &nl, n, n_spec);
+    phase_items<T, 3, STRIDE, S::obca, false, S::bank>(ws_base, &nl, n, n_spec);
     __syncthreads();
     IGT_MID_TICK();
-    phase_items<T, 4, STRIDE, S::obca, RSTG>(ws_base, &nl, n, n_spec);
+    phase_items<T, 4, STRIDE, S::obca, RSTG, S::bank>(ws_base, &nl, n, n_spec);
     __syncthreads();
     return n_spec;
 }
@@ -1873,8 +1926,9 @@ __device__ __forceinline__ int trial_phase_cta(const DevParams<T> &P, T *ws_base
 // gt_mpc with the tensor-core value term: the terminal values (and derivatives) of all n * n_spec
 // line-search candidates of the CTA in one CTA-wide evaluation -- thread t takes candidate t / n of the
 // t % n-th listed problem -- left in Tc(candidate buffer, 2..7) for the owner's accept_trials.
-// COOP: the same with the exact cooperative evaluation (mlp_coop.cuh) instead of the tensor cores.
-template <typename T, bool COOP, typename WS>
+// COOP: the same with the exact cooperative evaluation (mlp_coop.cuh) instead of the tensor cores; COOP + BANK: each
+// candidate with its problem's network, the index read here from io (not held by the solver loop).
+template <typename T, bool COOP, bool BANK, typename WS>
 __device__ __forceinline__ void tc_candidates(const DevParams<T> &P, const ProbIO &io, T *ws_base, const WS &wproto,
                                               const NodeList<T> &nl, int n, int n_spec, MlpTcCtx *tc, uint8_t *coop_smem,
                                               int jlo = 0, bool filter = false)
@@ -1886,6 +1940,7 @@ __device__ __forceinline__ void tc_candidates(const DevParams<T> &P, const ProbI
     int nb = 0;
     using V = typename std::conditional<COOP, T, float>::type;
     V cx[4] = { V(0), V(0), V(0), V(0) }, o[6], sN = V(0), vN = V(0);
+    int net = 0;
     if (valid) {
         w.bind(ws_base, nl.slot[q]);
         nb = cand_buf(nl.ctx[q].cur, j);
@@ -1896,9 +1951,11 @@ __device__ __forceinline__ void tc_candidates(const DevParams<T> &P, const ProbI
 #pragma unroll
         for (int i = 0; i < 4; i++) cx[i] = V(io.ctx[p * 4 + i]);
         sN = V(w.Z(nb, P.N, IS)); vN = V(w.Z(nb, P.N, IV));
+        if (BANK) net = bank_io<T>(io).net_idx[p];
     }
     if (__syncthreads_or(valid)) {
-        if constexpr (COOP) mlp_coop_eval(P, coop_smem, valid, sN, vN, cx, o);
+        if constexpr (COOP && BANK) mlp_coop_eval_bank(bank_io<T>(io).nets, coop_smem, valid, net, sN, vN, cx, o);
+        else if constexpr (COOP) mlp_coop_eval(P, coop_smem, valid, sN, vN, cx, o);
         else mlp_tc_eval(*tc, valid, sN, vN, cx, o);
         if (valid) {
 #pragma unroll
@@ -1923,7 +1980,9 @@ __device__ int g_round_mx[512][4];       // per loop pass, max over CTA 0's thre
 #define IGT_TICK(i) do { } while (0)
 #endif
 
-template <typename T, bool TC, int STRIDE = 32, bool OBCA = false, bool COOP = false, bool RSTG = false>
+// BANK: gt_mpc with the handle's network bank, each problem with network io.net_idx[p] (per-thread or, with COOP,
+// cooperative value term; not with TC)
+template <typename T, bool TC, int STRIDE = 32, bool OBCA = false, bool COOP = false, bool RSTG = false, bool BANK = false>
 __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const ProbIO &io, T *ws_base,
                                                  long slot, long B, const Sched &sc,
                                                  const double *guess, T *mlp_scratch, int mlp_width, MlpTcCtx *tc,
@@ -1931,7 +1990,8 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
 {
     __shared__ NodeList<T> nl;
     if (threadIdx.x == 0) { nl.cslot = cslot; nl.rstg = rstg_smem; }   // (the first CTA barrier of the loop publishes them)
-    Solver<T, Ws<T, STRIDE, OBCA>> sv(P);
+    static_assert(!(TC && BANK), "the tensor-core value term holds one network");
+    Solver<T, Ws<T, STRIDE, OBCA>, BANK> sv(P);
     sv.w.init_layout(P.N, P.n_cinf);
     sv.w.bind(ws_base, slot);
     sv.mlp_scratch = mlp_scratch; sv.mlp_width = mlp_width;
@@ -1984,7 +2044,8 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
             if (__syncthreads_or(want)) {
                 T o[6];
                 const T sN = want ? sv.w.Z(sv.cur, P.N, IS) : T(0), vN = want ? sv.w.Z(sv.cur, P.N, IV) : T(0);
-                mlp_coop_eval(P, coop_smem, want, sN, vN, sv.ctx, o);
+                if constexpr (BANK) mlp_coop_eval_bank(bank_io<T>(io).nets, coop_smem, want, want ? bank_io<T>(io).net_idx[p] : 0, sN, vN, sv.ctx, o);
+                else mlp_coop_eval(P, coop_smem, want, sN, vN, sv.ctx, o);
                 if (want) { sv.tcur.V = o[0]; sv.tcur.gs = o[1]; sv.tcur.gv = o[2]; sv.tcur.Hss = o[3]; sv.tcur.Hsv = o[4]; sv.tcur.Hvv = o[5]; }
             }
         }
@@ -2061,14 +2122,14 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
             // first, accepted nine times out of ten); the speculative candidates only of the problems whose first
             // was rejected.  Same candidates judged in the same order: same iterates.
             const int left = P.n_alpha - sv.ls, nj = n_spec < left ? n_spec : left;
-            tc_candidates<T, COOP>(P, io, ws_base, sv.w, nl, n_try, 1, tc, coop_smem);
+            tc_candidates<T, COOP, BANK>(P, io, ws_base, sv.w, nl, n_try, 1, tc, coop_smem);
             int tried = 0, jacc = -1;
             if (trying) jacc = sv.judge_trials(0, 1, true, tried);
             const bool more = trying && jacc < 0 && nj > 1;
             if (trying) nl.more[my_idx] = more ? 1 : 0;
             if (__syncthreads_or(more)) {
                 // candidates 1 .. n_spec-1: (n_spec - 1) n <= blockDim.x requests, one pass
-                tc_candidates<T, COOP>(P, io, ws_base, sv.w, nl, n_try, n_spec, tc, coop_smem, 1, true);
+                tc_candidates<T, COOP, BANK>(P, io, ws_base, sv.w, nl, n_try, n_spec, tc, coop_smem, 1, true);
                 if (more) jacc = sv.judge_trials(1, nj, true, tried);
             }
             if (trying) sv.finish_trials(jacc, tried);

@@ -44,6 +44,7 @@ V_PRED_MIN, V_PRED_MAX = -2.0, 20.0   # fourwayint.yaml:23-24 (predictor clip)
 class EpisodeSpec:
     routes: list                 # [route_0, route_1], e.g. ['13', '23']
     s0: tuple                    # start offsets along the routes (evaluate.py:91-94, :404-418)
+    scenario: int = 0            # reference scenario 1..8 (0: not from reference_episode_specs)
 
 
 @dataclass
@@ -73,7 +74,7 @@ def reference_episode_specs(scenarios=range(1, 9), sample=0, seed=2026):
         for rot in range(4):
             for order in range(2):
                 routes = G.scenario_routes(sc, rot, order)
-                specs.append(EpisodeSpec(routes=routes, s0=tuple(offs[r[0]] for r in routes)))
+                specs.append(EpisodeSpec(routes=routes, s0=tuple(offs[r[0]] for r in routes), scenario=sc))
     return specs
 
 
@@ -90,20 +91,33 @@ def _outcome(z_cl, u_cl, solved, d_min, ca_type, lat):
                          min_distance=dist.min(axis=1), step_latency_ms=lat)
 
 
+def _vehicle_nets(net_idx, E):
+    """per-episode bank slots [E] -> per-vehicle [2E] (both vehicles of an episode plan with its network)"""
+    a = np.asarray(net_idx, dtype=np.int32)
+    if a.shape != (E,):
+        raise ValueError("net_idx: one bank slot per episode, expected shape (%d,), got %s" % (E, a.shape))
+    return np.repeat(a, 2)
+
+
 def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_latency=False, mode="mpc",
-                    ca_type="circle"):
+                    ca_type="circle", net_idx=None):
     """mode 'gt_mpc' (the solver must have been given the value network): previous input (0, 0) instead of
     (0.1, 0) (evaluate.py:171 / :419); the first forecast assumes a = 0.09 (i + 1) for vehicle i
     (evaluate.py:207-210); warm starts only from t = 2 on (evaluate.py:232-235); every solve gets
     nn_ctx = (s_tv, v_tv, e_tv, e_ego): the other vehicle's forecast at step N (mpc.py:330) and the
     scenario codes of utils.scenario_encoding (mpc.py:336-337).
     ca_type 'obca': every solve also gets obs_psi (module docstring); the solver must have been made with d_min = 0.
-    Circle mode calls solve_batch without obs_psi, so solvers that do not know the keyword still work."""
+    Circle mode calls solve_batch without obs_psi, so solvers that do not know the keyword still work.
+    net_idx[E] (gt_mpc): the solver's network-bank slot of each episode (evaluate.py:123, network k for scenario k), so
+    that episodes of several scenarios run in one loop; passed to solve_batch only when given."""
     assert mode in ("mpc", "gt_mpc") and ca_type in ("circle", "obca")
+    if net_idx is not None and mode != "gt_mpc":
+        raise ValueError("net_idx selects value networks: mode 'gt_mpc' only")
     gt = mode == "gt_mpc"
     obca = ca_type == "obca"
     E = len(specs)
     B = 2 * E
+    veh_net = None if net_idx is None else _vehicle_nets(net_idx, E)
     routes = [sp.routes for sp in specs]
     curv = np.array([G.curvature_params(r) for sp in specs for r in sp.routes])           # [B, 3]
     z = np.zeros((B, 7))
@@ -204,6 +218,8 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
             kw = dict(nn_ctx=nn_ctx[idx]) if gt else {}
             if obca:
                 kw["obs_psi"] = obs_psi[idx]
+            if veh_net is not None:
+                kw["net_idx"] = veh_net[idx]
             r = solver.solve_batch(z[idx], u_prev[idx], curv[idx], obs[idx], u_init=u_init[idx] if warm else None, **kw)
             out["x"][idx], out["u"][idx], out["status"][idx] = r["x"], r["u"], r["status"]
         if record_latency:
@@ -234,15 +250,19 @@ def run_closed_loop(solver, specs, steps=150, N=40, dt=0.1, d_min=5.6, record_la
     return _outcome(z_cl, u_cl, solved, d_min, ca_type, lat)
 
 
-def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc", record_latency=False, ca_type="circle"):
+def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc", record_latency=False, ca_type="circle",
+                           net_idx=None):
     """The same closed loop with the per-timestep glue on the GPU (csrc/episode.cuh, igt_episode_run_host): all E
     episodes advance `steps` steps without the host in the loop -- per step one glue kernel, one batched solve of all 2E
     vehicles (per-problem warm / cold start), one plant kernel.  `solver` is a planner.BatchSolver (fp64) with horizon N.
     Returns an EpisodeResult; step_latency_ms = device time per step (all episodes together).
     ca_type 'obca' builds the obstacle heading forecast on the device as well (module docstring) and needs a solver
-    made with d_min = 0 (mpc.py:42-43): with the circle gap of 5.6 m the rectangles would be kept that far apart."""
+    made with d_min = 0 (mpc.py:42-43): with the circle gap of 5.6 m the rectangles would be kept that far apart.
+    net_idx[E] (gt_mpc): bank slot of each episode, as in run_closed_loop (igt_episode_run_ex_host)."""
     import ctypes as C
     assert mode in ("mpc", "gt_mpc") and solver.N == N
+    if net_idx is not None and mode != "gt_mpc":
+        raise ValueError("net_idx selects value networks: mode 'gt_mpc' only")
     if ca_type not in ("circle", "obca"):
         raise ValueError("ca_type must be 'circle' or 'obca', got %r" % (ca_type,))
     if ca_type == "obca" and solver.params.d_min != 0:
@@ -266,7 +286,15 @@ def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc"
     z_cl = np.zeros((E, 2, steps + 1, 7)); u_cl = np.zeros((E, 2, steps, 2)); solved = np.zeros((E, 2, steps), dtype=np.int32)
     ms = np.zeros(steps, dtype=np.float32)
     vp = lambda a: C.c_void_p(a.ctypes.data)
-    rc = solver.lib.igt_episode_run_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
-                                         vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
-    solver._check(rc, "igt_episode_run_host")
+    if net_idx is None:
+        rc = solver.lib.igt_episode_run_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
+                                             vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
+        solver._check(rc, "igt_episode_run_host")
+    else:
+        nets = np.ascontiguousarray(net_idx, dtype=np.int32)
+        if nets.shape != (E,):
+            raise ValueError("net_idx: one bank slot per episode, expected shape (%d,), got %s" % (E, nets.shape))
+        rc = solver.lib.igt_episode_run_ex_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
+                                                vp(nets), vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
+        solver._check(rc, "igt_episode_run_ex_host")
     return _outcome(z_cl, u_cl, solved.astype(bool), d_min, ca_type, [float(v) for v in ms] if record_latency else [])

@@ -17,6 +17,12 @@ rectangle rows with d_min = 0 instead of the 5.6 m circle gap; an episode's coll
 `--eval_mode gt_mpc` needs the value network: --nn_weights FILE.npz with arrays W0, b0, W1, b1, ...
 (model.py:14-51 layer order) and optionally Wn, mu_f, sigma_t, mu_t (mpc.py:109-118; the reference's
 processed_sc*.pkl statistics are not shipped, identity / zero are used when absent).
+
+`--sc all` runs the episodes of all eight scenarios through ONE closed loop (one batched solve per step for every
+vehicle of every scenario) and writes one run directory per scenario, laid out as for `--sc k`.  In gt_mpc mode the
+reference plans scenario k with its own network V_GT_sc{k} (evaluate.py:123): a --nn_weights path containing `{sc}`
+is filled in per scenario, and with `--sc all` the eight networks form the solver's network bank (episode of
+scenario k -> slot k - 1).  A plain path is one network for every scenario.
 """
 import argparse
 import datetime
@@ -42,8 +48,30 @@ def load_mlp(path):
                 mu_t=float(d['mu_t']) if 'mu_t' in d.files else 0.0)
 
 
+def networks(path, scenarios):
+    """--nn_weights for the given scenarios: a plain path or one scenario -> one network dict; a path with `{sc}` and
+    several scenarios -> the network bank, a list with entry k - 1 = scenario k's network (None for the others)."""
+    if '{sc}' not in path:
+        return load_mlp(path)
+    if len(scenarios) == 1:
+        return load_mlp(path.format(sc=scenarios[0]))
+    return [load_mlp(path.format(sc=k)) if k in scenarios else None for k in range(1, max(scenarios) + 1)]
+
+
+def scenario_arg(v):
+    """--sc: a scenario number 1..8 or 'all'"""
+    if v == 'all':
+        return v
+    k = int(v)
+    if not 1 <= k <= 8:
+        raise argparse.ArgumentTypeError("--sc must be 1..8 or 'all', got %r" % (v,))
+    return k
+
+
 def main(args, solver=None):
-    """`solver`: any object with the BatchSolver methods (default: a BatchSolver made here, d_min = 0 for OBCA)."""
+    """`solver`: any object with the BatchSolver methods (default: a BatchSolver made here, d_min = 0 for OBCA); with
+    `--sc all` and a `{sc}` weights path it gets a per-problem `net_idx` keyword (its network bank).
+    Returns (run directory, summary) -- with `--sc all`, a list of run directories, one per scenario."""
     seed = 2026
     ca_type = getattr(args, 'ca_type', 'circle')
     if ca_type not in ('circle', 'obca'):
@@ -52,20 +80,25 @@ def main(args, solver=None):
     N, dt = POLICY_CONFIG['N'], POLICY_CONFIG['dt']
     T = getattr(args, 'steps', None) or 150                                                # T_sim / dt, evaluate.py:84-85
     timenow = datetime.datetime.now().strftime("%Y%m%d_%H%M%S")
-    run_dir = os.path.join(args.save_dir, '%s_sc%d_seed%d_%s' % (args.eval_mode, args.sc, seed, timenow))
+    scenarios = list(range(1, 9)) if args.sc == 'all' else [args.sc]
+    run_dirs = {k: os.path.join(args.save_dir, '%s_sc%d_seed%d_%s' % (args.eval_mode, k, seed, timenow)) for k in scenarios}
+    gt = args.eval_mode == 'gt_mpc'
+    bank = gt and len(scenarios) > 1 and '{sc}' in (args.nn_weights or '')    # network k - 1 for scenario k
     own = solver is None
     if own:
         from .planner import BatchSolver
-        mlp = load_mlp(args.nn_weights) if args.eval_mode == 'gt_mpc' else None
+        mlp = networks(args.nn_weights, scenarios) if gt else None
         solver = BatchSolver(N=N, dt=dt, mlp=mlp, **(dict(d_min=0.0) if ca_type == 'obca' else {}))
     variants = [(r, o) for r in range(4) for o in range(2)] if args.all_variants else [(args.rotation, args.order)]
     summary = []
     for it in range(args.num_samples):
-        all_specs = episode.reference_episode_specs(scenarios=[args.sc], sample=it, seed=seed)
-        specs = [all_specs[r * 2 + o] for r, o in variants]
+        all_specs = episode.reference_episode_specs(scenarios=scenarios, sample=it, seed=seed)
+        specs = [all_specs[8 * j + r * 2 + o] for j in range(len(scenarios)) for r, o in variants]
         loop = episode.run_closed_loop_device if getattr(args, 'device_loop', False) else episode.run_closed_loop
-        res = loop(solver, specs, steps=T, N=N, record_latency=True, mode=args.eval_mode, ca_type=ca_type)
+        kw = dict(net_idx=np.array([sp.scenario - 1 for sp in specs])) if bank else {}
+        res = loop(solver, specs, steps=T, N=N, record_latency=True, mode=args.eval_mode, ca_type=ca_type, **kw)
         for e, sp in enumerate(specs):
+            run_dir = run_dirs[scenarios[e // len(variants)]]
             starts = [G.frenet2global(sp.s0[i], sp.routes[i]) for i in range(2)]
             refs = [RT.reference_dict(sp.routes[i], starts[i][0], starts[i][1], n=T) for i in range(2)]
             goals = np.array([[G.goal_pose(r[1])[0] for r in sp.routes], [G.goal_pose(r[1])[1] for r in sp.routes]])
@@ -75,14 +108,14 @@ def main(args, solver=None):
             sub = results.write_episode(run_dir, args.eval_mode, res.z_cl[e], res.u_cl[e], res.solved[e], res.deadlock[e],
                                         times, N=N, refs=refs, initial_agents=agents, initial_default=default,
                                         routes=sp.routes, goals=goals, policy_config=policy_config)
-            summary.append(dict(sample=it, routes=sp.routes, deadlock=bool(res.deadlock[e]), collision=bool(res.collision[e]),
+            summary.append(dict(sample=it, **(dict(scenario=sp.scenario) if args.sc == 'all' else {}), routes=sp.routes, deadlock=bool(res.deadlock[e]), collision=bool(res.collision[e]),
                                 goal=[bool(g) for g in res.goal[e]], infeasible=[int(n) for n in res.num_infeasible[e]],
                                 min_distance=float(res.min_distance[e])))
             print("sample %d routes %s: deadlock %s, goals %s, failed solves %s, min distance %.2f m -> %s"
                   % (it, sp.routes, res.deadlock[e], list(res.goal[e]), list(res.num_infeasible[e]), res.min_distance[e], sub))
     if own:
         solver.close()
-    return run_dir, summary
+    return (list(run_dirs.values()) if args.sc == 'all' else run_dirs[args.sc]), summary
 
 
 def build_parser():
@@ -90,11 +123,12 @@ def build_parser():
     p.add_argument('--save_dir', type=str, required=True)
     p.add_argument('--num_samples', type=int, default=1)
     p.add_argument('--eval_mode', type=str, required=True, choices=['mpc', 'gt_mpc'])
-    p.add_argument('--sc', type=int, default=1)
+    p.add_argument('--sc', type=scenario_arg, default=1, help="scenario 1..8, or 'all': every scenario in one loop")
     p.add_argument('--rotation', type=int, default=0, choices=range(4))
     p.add_argument('--order', type=int, default=0, choices=range(2))
     p.add_argument('--all_variants', action='store_true')
-    p.add_argument('--nn_weights', type=str, default=None)
+    p.add_argument('--nn_weights', type=str, default=None,
+                   help="gt_mpc value network(s), .npz; '{sc}' in the path is replaced by the scenario number")
     p.add_argument('--steps', type=int, default=150, help='closed-loop steps (the reference simulates 15 s = 150)')
     p.add_argument('--device_loop', action='store_true', help='run the per-timestep glue on the GPU as well (igt_episode_run_host)')
     p.add_argument('--ca_type', type=str, default='circle', choices=['circle', 'obca'],

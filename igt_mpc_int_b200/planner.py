@@ -34,6 +34,16 @@ def _hp(a):
     return None if a is None else _vp(a.ctypes.data)
 
 
+def _net_idx(net_idx, B):
+    """per-problem bank slots as a contiguous int32 [B] array (None stays None)"""
+    if net_idx is None:
+        return None
+    a = np.ascontiguousarray(net_idx, dtype=np.int32)
+    if a.shape != (B,):
+        raise ValueError("net_idx: expected shape (%d,), got %s" % (B, a.shape))
+    return a
+
+
 _CINF_CACHE = {}
 
 
@@ -50,7 +60,9 @@ class BatchSolver:
     precision: 'f64' (default; parity path) or 'f32'.  `options` override fields of
     `igt_params` (include/igt_mpc.h), e.g. tol=..., max_iter=..., mu0=...
     mlp: optional dict(weights=[(W, b), ...], Wn=6x6, mu_f=[6], sigma_t=float, mu_t=float)
-    enabling the gt_mpc terminal cost (mpc.py:105-127, :367-369).
+    enabling the gt_mpc terminal cost (mpc.py:105-127, :367-369), or a list of at most 8 such dicts (None: an empty
+    slot): a network bank, entry k in slot k.  Calls with `net_idx` pick a slot per problem (the reference's
+    network k for scenario k, evaluate.py:123); calls without it use slot 0.
     """
 
     def __init__(self, N=40, dt=0.1, n_rk=4, precision="f64", mlp=None, jerk_limit=0.9,
@@ -75,7 +87,13 @@ class BatchSolver:
             raise _lib.IgtError("igt_create failed (%d): %s" % (rc, self.lib.igt_last_error(None).decode()))
         self._h = h
         self.has_mlp = False
-        if mlp is not None:
+        if isinstance(mlp, (list, tuple)):
+            if len(mlp) > _lib.MAX_MLP_NETS:
+                raise ValueError("a network bank holds at most %d networks, got %d" % (_lib.MAX_MLP_NETS, len(mlp)))
+            for k, net in enumerate(mlp):
+                if net is not None:
+                    self.set_mlp(**net, net=k)
+        elif mlp is not None:
             self.set_mlp(**mlp)
 
     # -- lifetime --------------------------------------------------------------------------
@@ -106,7 +124,8 @@ class BatchSolver:
         return out.value
 
     # -- value network ---------------------------------------------------------------------
-    def set_mlp(self, weights, Wn, mu_f, sigma_t, mu_t):
+    def set_mlp(self, weights, Wn, mu_f, sigma_t, mu_t, net=0):
+        """load a value network into bank slot `net` (0 = the network of calls without net_idx)"""
         n = len(weights)
         Ws = [_f64(W) for W, _ in weights]
         bs = [_f64(b).ravel() for _, b in weights]
@@ -115,28 +134,36 @@ class BatchSolver:
         Wp = (dp * n)(*[w.ctypes.data_as(dp) for w in Ws])
         bp = (dp * n)(*[b.ctypes.data_as(dp) for b in bs])
         Wn, mu_f = _f64(Wn, (6, 6)), _f64(mu_f, (6,))
-        rc = self.lib.igt_set_mlp(self._h, n, (C.c_int * len(dims))(*dims), Wp, bp, Wn.ctypes.data_as(dp),
-                                  mu_f.ctypes.data_as(dp), float(sigma_t), float(mu_t))
-        self._check(rc, "igt_set_mlp")
+        rc = self.lib.igt_set_mlp_at(self._h, int(net), n, (C.c_int * len(dims))(*dims), Wp, bp, Wn.ctypes.data_as(dp),
+                                     mu_f.ctypes.data_as(dp), float(sigma_t), float(mu_t))
+        self._check(rc, "igt_set_mlp_at")
         self.has_mlp = True
 
     def set_option(self, name, value):
         self._check(self.lib.igt_set_option(self._h, name.encode(), float(value)), "igt_set_option")
 
-    def mlp_value(self, sN, vN, nn_ctx, tensor_cores=True):
+    def mlp_value(self, sN, vN, nn_ctx, tensor_cores=True, net_idx=None):
         """Value term and its (s_N, v_N) derivatives: out[B,6] = (V, Vs, Vv, Vss, Vsv, Vvv).
-        tensor_cores: True / 1 tcgen05 kernel, False / 0 per-thread fp64, 2 the solver's cooperative fp64 evaluation."""
+        tensor_cores: True / 1 tcgen05 kernel, False / 0 per-thread fp64, 2 the solver's cooperative fp64 evaluation.
+        net_idx[B]: bank slot of each row (modes 0 and 2 only)."""
         sN = _f64(sN).ravel(); B = sN.shape[0]
         vN = _f64(vN, (B,)); nn_ctx = _f64(nn_ctx, (B, 4))
         out = np.empty((B, 6))
-        rc = self.lib.igt_mlp_value_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(out), int(tensor_cores))
-        self._check(rc, "igt_mlp_value_host")
+        if net_idx is None:
+            rc = self.lib.igt_mlp_value_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(out), int(tensor_cores))
+            self._check(rc, "igt_mlp_value_host")
+        else:
+            rc = self.lib.igt_mlp_value_ex_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(_net_idx(net_idx, B)), _hp(out),
+                                                int(tensor_cores))
+            self._check(rc, "igt_mlp_value_ex_host")
         return out
 
     # -- host-pointer calls (copies inside) ---------------------------------------------------
-    def solve_batch(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, obs_psi=None):
+    def solve_batch(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, obs_psi=None, net_idx=None):
         """numpy in / numpy out.  Returns dict(x[B,N+1,7], u[B,N,2], cost, viol, status, iters).
-        obs_psi[B,N+1] (obstacle heading forecast) selects the OBCA collision rows (mpc.py:211-221)."""
+        obs_psi[B,N+1] (obstacle heading forecast) selects the OBCA collision rows (mpc.py:211-221).
+        net_idx[B] (with nn_ctx): the bank slot of each problem's value network; an index that names no loaded
+        network raises IgtError before anything runs."""
         N = self.N
         x0 = _f64(x0)
         B = x0.shape[0]
@@ -148,14 +175,20 @@ class BatchSolver:
         if out is None:
             out = dict(x=np.empty((B, N + 1, 7)), u=np.empty((B, N, 2)), cost=np.empty(B), viol=np.empty(B),
                        status=np.empty(B, dtype=np.int32), iters=np.empty(B, dtype=np.int32))
-        rc = self.lib.igt_solve_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                     _hp(u_init), _hp(out["x"]), _hp(out["u"]), _hp(out["cost"]),
-                                     _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
-        self._check(rc, "igt_solve_host")
+        if net_idx is None:
+            rc = self.lib.igt_solve_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                         _hp(u_init), _hp(out["x"]), _hp(out["u"]), _hp(out["cost"]),
+                                         _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
+            self._check(rc, "igt_solve_host")
+        else:
+            rc = self.lib.igt_solve_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                            _hp(_net_idx(net_idx, B)), _hp(u_init), _hp(out["x"]), _hp(out["u"]),
+                                            _hp(out["cost"]), _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
+            self._check(rc, "igt_solve_ex_host")
         return out
 
-    def evaluate(self, x0, u_prev, curv, obs_xy, u, nn_ctx=None, obs_psi=None):
-        """Cost (mpc.py:356-373) and max inequality-row value of given controls."""
+    def evaluate(self, x0, u_prev, curv, obs_xy, u, nn_ctx=None, obs_psi=None, net_idx=None):
+        """Cost (mpc.py:356-373) and max inequality-row value of given controls (net_idx: as in solve_batch)."""
         N = self.N
         x0 = _f64(x0)
         B = x0.shape[0]
@@ -164,9 +197,14 @@ class BatchSolver:
         nn_ctx = None if nn_ctx is None else _f64(nn_ctx, (B, 4))
         obs_psi = None if obs_psi is None else _f64(obs_psi, (B, N + 1))
         cost, viol, z = np.empty(B), np.empty(B), np.empty((B, N + 1, 7))
-        rc = self.lib.igt_eval_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                    _hp(u), _hp(cost), _hp(viol), _hp(z))
-        self._check(rc, "igt_eval_host")
+        if net_idx is None:
+            rc = self.lib.igt_eval_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                        _hp(u), _hp(cost), _hp(viol), _hp(z))
+            self._check(rc, "igt_eval_host")
+        else:
+            rc = self.lib.igt_eval_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                           _hp(_net_idx(net_idx, B)), _hp(u), _hp(cost), _hp(viol), _hp(z))
+            self._check(rc, "igt_eval_ex_host")
         return dict(cost=cost, viol=viol, x=z)
 
     def rollout(self, z0, u, curv=None, jac=False, model=0):
@@ -188,8 +226,11 @@ class BatchSolver:
         return (z, A, Bm) if jac else z
 
     # -- device-pointer call (torch tensors already in HBM; no copies, no sync) ---------------
-    def solve_batch_device(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, stream=None, obs_psi=None):
-        """torch CUDA float64 tensors in / out; enqueues on the current torch stream."""
+    def solve_batch_device(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, stream=None, obs_psi=None,
+                           net_idx=None):
+        """torch CUDA float64 tensors in / out; enqueues on the current torch stream.
+        net_idx: int32 device tensor [B] of bank slots (with nn_ctx); checked in the kernel: a problem whose index
+        names no loaded network gets status 7 (STATUS_BAD_NET) and NaN outputs."""
         import torch
         N = self.N
         B = x0.shape[0]
@@ -204,6 +245,8 @@ class BatchSolver:
                              (obs_psi, (B, N + 1), "obs_psi")):
             if t is not None:
                 check(t, shp, torch.float64, name)
+        if net_idx is not None:
+            check(net_idx, (B,), torch.int32, "net_idx")
         if out is None:
             out = dict(x=torch.empty((B, N + 1, 7), dtype=torch.float64, device=dev),
                        u=torch.empty((B, N, 2), dtype=torch.float64, device=dev),
@@ -217,10 +260,16 @@ class BatchSolver:
                 check(out[k], shp, dt, "out[%r]" % k)
         st = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
         p = lambda t: None if t is None else _vp(t.data_ptr())
-        rc = self.lib.igt_solve_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(u_init),
-                                    p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]), p(out["status"]),
-                                    p(out["iters"]), _vp(st))
-        self._check(rc, "igt_solve_dev")
+        if net_idx is None:
+            rc = self.lib.igt_solve_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(u_init),
+                                        p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]), p(out["status"]),
+                                        p(out["iters"]), _vp(st))
+            self._check(rc, "igt_solve_dev")
+        else:
+            rc = self.lib.igt_solve_ex_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(net_idx),
+                                           p(u_init), p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]),
+                                           p(out["status"]), p(out["iters"]), _vp(st))
+            self._check(rc, "igt_solve_ex_dev")
         return out
 
 

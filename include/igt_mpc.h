@@ -31,6 +31,7 @@ extern "C" {
 
 #define IGT_MAX_CINF 128
 #define IGT_MAX_MLP_LAYERS 5
+#define IGT_MAX_MLP_NETS 8   /* value networks per handle (igt_set_mlp_at) */
 
 #define IGT_OK 0
 #define IGT_EINVAL (-1)   /* bad argument (NULL, size, unsupported horizon ...) */
@@ -47,6 +48,8 @@ extern "C" {
 #define IGT_STATUS_STALLED 5         /* still infeasible (|c + slack| > stall_rp) after stall_iter iterations */
 #define IGT_STATUS_ACCEPTABLE 6      /* failed to converge tightly, but the final point is within the reference's IPOPT tolerances (see acc_tol):
                                         a success for the host (IPOPT returns Solve_Succeeded there), reported apart */
+#define IGT_STATUS_BAD_NET 7         /* *_ex_dev with net_idx: the index is outside 0..IGT_MAX_MLP_NETS-1 or names an empty
+                                        slot; no solve, NaN outputs, the other problems are unaffected */
 
 #define IGT_PREC_F32 0
 #define IGT_PREC_F64 1
@@ -123,6 +126,15 @@ int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *cons
                 const double *const *b, const double *Wn, const double *mu_f, double sigma_t,
                 double mu_t);
 
+/* Network bank, mpc.py:105-127 once per network: the reference ships one value network per scenario (V_GT_sc{1..8}.pt)
+ * and evaluate.py:123 loads network k for scenario k.  Loads a network as igt_set_mlp does into slot `net`
+ * (0..IGT_MAX_MLP_NETS-1) of the handle's bank; the *_ex entry points below pick a slot per problem (net_idx).
+ * net = 0 is exactly igt_set_mlp: slot 0 is also the network of every call without net_idx.  All arguments are
+ * checked before anything is replaced; only slot `net`'s buffers are freed.  A bank solve always evaluates the value
+ * term exactly (fp64 / the solver's precision): the "tensor_core_mlp" option applies to single-network calls only. */
+int igt_set_mlp_at(igt_handle *h, int net, int n_layers, const int *dims, const double *const *W,
+                   const double *const *b, const double *Wn, const double *mu_f, double sigma_t, double mu_t);
+
 /* Replaces KinematicBicycleModelFrenet.__call__ (common/kinematic_bicycle_model_frenet.py:
  * 69-185; model 0) and KinematicBicycleModel.__call__ (common/kinematic_bicycle_model.py:
  * 15-50; model 1) rolled over the horizon, plus the Jacobians CasADi derives by AD.
@@ -143,6 +155,11 @@ int igt_rollout_host(igt_handle *h, int B, const float *z0, const float *u, cons
 int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                   const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u,
                   double *cost, double *viol, double *z);
+/* The same with net_idx[B] (int32, needs nn_ctx) or NULL: problem b's value term uses bank slot net_idx[b]
+ * (evaluate.py:198-312 per scenario).  Every index must name a loaded slot, else IGT_EINVAL before any launch. */
+int igt_eval_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                     const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                     const double *u, double *cost, double *viol, double *z);
 
 /* Replaces MPC_Planner.update_initial_condition / update_predictions / solve
  * (mpc.py:280-294, :241-278, :383-406) for a batch of independent problems.
@@ -161,6 +178,19 @@ int igt_solve_dev(igt_handle *h, int B, const double *x0, const double *u_prev, 
 int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                    const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init,
                    double *x, double *u, double *cost, double *viol, int *status, int *iters);
+/* The gt_mpc branch of evaluate.py:198-312 for many scenarios in one batch (evaluate.py:123: scenario k plans with
+ * network k): igt_solve_* plus net_idx[B] (int32) or NULL.  Problem b's value term uses bank slot net_idx[b]
+ * (igt_set_mlp_at); net_idx needs nn_ctx, else IGT_EINVAL.  NULL is exactly igt_solve_*.
+ * _host checks the indices and returns IGT_EINVAL before any launch if one names no loaded slot; _dev checks them in
+ * the kernel: such a problem gets IGT_STATUS_BAD_NET.  Bank solves use the exact value term (cooperative if every
+ * loaded network is <= 128 wide and the solve is fp64 circle mode; per thread otherwise). */
+int igt_solve_ex_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                     const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                     const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters,
+                     void *stream);
+int igt_solve_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                      const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                      const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters);
 
 /* Replaces the per-timestep loop of evaluate.py:451-564 ('mpc') / :198-312 ('gt_mpc') for E independent two-vehicle
  * episodes: `steps` closed-loop steps entirely on the device -- per step one kernel for the glue before the solve
@@ -188,6 +218,12 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
 int igt_episode_run_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
                          const double *z0, const double *u_prev0, const double *enc, double *z_cl, double *u_cl,
                          int *solved, float *step_ms);
+/* The same with net_idx[E] (int32) or NULL: both vehicles of episode e plan with bank slot net_idx[e], so episodes
+ * of all scenarios run in one loop, each with its own network (evaluate.py:123, :198-312).  Needs the
+ * IGT_EPISODE_GT_MPC bit (with or without IGT_EPISODE_OBCA); indices are checked as in igt_solve_ex_host. */
+int igt_episode_run_ex_host(igt_handle *h, int E, int steps, int mode, const double *route_desc, const double *curv,
+                            const double *z0, const double *u_prev0, const double *enc, const int *net_idx, double *z_cl,
+                            double *u_cl, int *solved, float *step_ms);
 
 /* Number of kernels this library has launched on `h` so far (bench.py's gpu_launches). */
 long long igt_launch_count(const igt_handle *h);
@@ -198,6 +234,10 @@ long long igt_launch_count(const igt_handle *h);
  * CTA-cooperative evaluation the solver uses (csrc/mlp_coop.cuh; any network with layers <= 128 wide).  Host fp64 arrays. */
 int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx,
                        double *out, int use_tensor_cores);
+/* The same with net_idx[B] (int32) or NULL: row b uses bank slot net_idx[b] (mpc.py:367-369 with network k of
+ * evaluate.py:123).  Modes 0 and 2 only (1 with net_idx: IGT_EINVAL); indices checked as in igt_solve_ex_host. */
+int igt_mlp_value_ex_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx,
+                          const int *net_idx, double *out, int use_tensor_cores);
 
 /* Run-time switches.
  * "tensor_core_mlp" (default 0).  The gt_mpc value term is evaluated exactly (fp64) by default, CTA-cooperatively
