@@ -179,6 +179,10 @@ __global__ void __launch_bounds__(128) rollout_euler_kernel(int B, const float *
     }
 }
 
+// largest row so far.  Unlike fmax, which drops a NaN operand, a NaN row wins and then stays: controls that drive the
+// state non-finite must not come back with the violation of the rows before the NaN
+__device__ __forceinline__ double row_max(double m, double r) { return (r > m || r != r) ? r : m; }
+
 // fp64 re-roll + cost + max inequality row (reference units) of given controls; BANK: value term of network
 // net_idx[p] of the bank (indices checked by the host)
 template <bool BANK>
@@ -202,26 +206,26 @@ __global__ void __launch_bounds__(128) eval_kernel(long B, const double *__restr
     for (int k = 0; k <= N; k++) {
         if (Zout) for (int i = 0; i < NZ; i++) Zout[(p * (N + 1) + k) * NZ + i] = z[i];
         J += z[IEPSI] * z[IEPSI] + z[IEY] * z[IEY];
-        m = fmax(m, fabs(z[IEY]) - P.ey_lim);
+        m = row_max(m, fabs(z[IEY]) - P.ey_lim);
         if (k >= 1) {
             if (obs_psi_) {                                      // OBCA rows in dual-eliminated form (obca.cuh)
                 double gd[3];
-                m = fmax(m, P.d_min + OBCA_MARGIN - obca_rect_sdist(z[IX], z[IY], z[IPSI], obs[2 * k], obs[2 * k + 1], obs_psi_[p * (N + 1) + k], gd));
+                m = row_max(m, P.d_min + OBCA_MARGIN - obca_rect_sdist(z[IX], z[IY], z[IPSI], obs[2 * k], obs[2 * k + 1], obs_psi_[p * (N + 1) + k], gd));
             } else {
                 double dx = z[IX] - obs[2 * k], dy = z[IY] - obs[2 * k + 1];
-                m = fmax(m, P.d_min * P.d_min - dx * dx - dy * dy);
+                m = row_max(m, P.d_min * P.d_min - dx * dx - dy * dy);
             }
         }
         if (k == N) break;
         double u[2] = { U[(p * N + k) * 2], U[(p * N + k) * 2 + 1] };
         su += u[0] * u[0] + u[1] * u[1];
-        m = fmax(m, fmax(P.v_min - z[IV], z[IV] - P.v_max));
-        m = fmax(m, fmax(P.a_min - u[0], u[0] - P.a_max));
-        m = fmax(m, fabs(u[1]) - P.df_max);
-        m = fmax(m, fabs(u[0] - up[0]) - P.da_max);
-        m = fmax(m, fabs(u[1] - up[1]) - P.ddf_max);
+        m = row_max(m, row_max(P.v_min - z[IV], z[IV] - P.v_max));
+        m = row_max(m, row_max(P.a_min - u[0], u[0] - P.a_max));
+        m = row_max(m, fabs(u[1]) - P.df_max);
+        m = row_max(m, fabs(u[0] - up[0]) - P.da_max);
+        m = row_max(m, fabs(u[1] - up[1]) - P.ddf_max);
         if (k == N - 1)
-            for (int q = 0; q < P.n_cinf; q++) m = fmax(m, P.cinf_A[q][0] * z[IV] + P.cinf_A[q][1] * u[0] - P.cinf_b[q]);
+            for (int q = 0; q < P.n_cinf; q++) m = row_max(m, P.cinf_A[q][0] * z[IV] + P.cinf_A[q][1] * u[0] - P.cinf_b[q]);
         double zn[NZ];
         rk4_step(P, z, u, curv, zn);
         for (int i = 0; i < NZ; i++) z[i] = zn[i];

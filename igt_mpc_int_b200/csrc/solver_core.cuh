@@ -1754,16 +1754,13 @@ struct Solver : SolverNet<T, BANK> {
     }
 };
 
-// Whole solve of problem p in workspace slot `slot`, one thread, start to finish.
+// Whole solve of problem p by a solver already bound to its workspace slot, one thread, start to finish.  The solver
+// may have solved other problems before: init() must leave nothing of them that the next solve reads.
 // (tests/hostsim calls this on the CPU; the kernels use the persistent-lane driver below.)
-template <typename T, bool OBCA = false>
-IGT_HD void solve_problem(const DevParams<T> &P, const ProbIO &io, T *ws_base, long slot, long p,
-                          double *guess_buf, T *mlp_scratch, int mlp_width)
+template <typename S>
+IGT_HD void solve_bound(S &sv, const ProbIO &io, long p, double *guess_buf)
 {
-    Solver<T, Ws<T, 32, OBCA>> sv(P);
-    sv.w.init_layout(P.N, P.n_cinf);
-    sv.w.bind(ws_base, slot);
-    sv.mlp_scratch = mlp_scratch; sv.mlp_width = mlp_width;
+    const auto &P = sv.P;
     const double *u_src = io.u_init ? io.u_init + p * P.N * 2 : guess_buf;
     if (!io.u_init) sv.compute_guess(io, p, guess_buf);
     if (sv.init(io, p, io.ctx != nullptr, u_src, io.u_init != nullptr)) {
@@ -1775,6 +1772,18 @@ IGT_HD void solve_problem(const DevParams<T> &P, const ProbIO &io, T *ws_base, l
         }
     }
     sv.write_out(io, p);
+}
+
+// Whole solve of problem p in workspace slot `slot` with a fresh solver object.
+template <typename T, bool OBCA = false>
+IGT_HD void solve_problem(const DevParams<T> &P, const ProbIO &io, T *ws_base, long slot, long p,
+                          double *guess_buf, T *mlp_scratch, int mlp_width)
+{
+    Solver<T, Ws<T, 32, OBCA>> sv(P);
+    sv.w.init_layout(P.N, P.n_cinf);
+    sv.w.bind(ws_base, slot);
+    sv.mlp_scratch = mlp_scratch; sv.mlp_width = mlp_width;
+    solve_bound(sv, io, p, guess_buf);
 }
 
 #ifdef __CUDACC__

@@ -151,7 +151,9 @@ int igt_rollout_host(igt_handle *h, int B, const float *z0, const float *u, cons
  * mpc.py:177-180,:223-226,:296-321 (collision in squared-distance units), of given controls.
  * The state trajectory is re-rolled on the device.  fp64 arrays: x0[B,7], u_prev[B,2],
  * curv[B,3], obs_xy[B,N+1,2], obs_psi[B,N+1] or NULL (see igt_solve_*), nn_ctx[B,4] = (s_tv, v_tv, e_tv, e_ego) or
- * NULL ('mpc' cost), u[B,N,2] -> cost[B], viol[B], z[B,N+1,7] (z may be NULL). */
+ * NULL ('mpc' cost), u[B,N,2] -> cost[B], viol[B], z[B,N+1,7] (z may be NULL).
+ * viol[b] = max(0, largest row); a NaN row makes it NaN, so controls with a NaN, or controls that drive the state
+ * non-finite, never report a violation that looks feasible (their cost is non-finite as well). */
 int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                   const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u,
                   double *cost, double *viol, double *z);

@@ -46,7 +46,9 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(_dp)
 
 
-def solve(p, x0, u_prev, curv, obs, nn_ctx=None, u_init=None, mlp=None):
+def solve(p, x0, u_prev, curv, obs, nn_ctx=None, u_init=None, mlp=None, lanes=False):
+    """lanes: one solver object per slot reused for problems q, q + 32, ... (persistent lanes) instead of a fresh one
+    per problem"""
     x0, u_prev, curv, obs, nn_ctx, u_init = map(_c, (x0, u_prev, curv, obs, nn_ctx, u_init))
     B, N = x0.shape[0], p.N
     Z = np.empty((B, N + 1, 7)); U = np.empty((B, N, 2)); cost = np.empty(B); viol = np.empty(B)
@@ -64,7 +66,7 @@ def solve(p, x0, u_prev, curv, obs, nn_ctx=None, u_init=None, mlp=None):
     rc = lib().hostsim_solve(C.byref(p), B, _ptr(x0), _ptr(u_prev), _ptr(curv), _ptr(obs), _ptr(nn_ctx), _ptr(u_init),
                              _ptr(Z), _ptr(U), _ptr(cost), _ptr(viol), status.ctypes.data_as(C.POINTER(C.c_int)),
                              iters.ctypes.data_as(C.POINTER(C.c_int)), n_layers, dims, Wp, bp, _ptr(Wn), _ptr(mu_f),
-                             C.c_double(st), C.c_double(mt))
+                             C.c_double(st), C.c_double(mt), int(bool(lanes)))
     assert rc == 0
     return dict(Z=Z, U=U, cost=cost, viol=viol, status=status, iters=iters)
 
@@ -80,15 +82,15 @@ def rollout(p, prec, z0, U, curv, jac=False):
     return (Z, A, Bm) if jac else Z
 
 
-def solve_obca(p, x0, u_prev, curv, obs, obs_psi, u_init=None):
-    """product solver code (OBCA collision rows, fp64) on the CPU"""
+def solve_obca(p, x0, u_prev, curv, obs, obs_psi, u_init=None, lanes=False):
+    """product solver code (OBCA collision rows, fp64) on the CPU; lanes: as in solve"""
     x0, u_prev, curv, obs, obs_psi, u_init = map(_c, (x0, u_prev, curv, obs, obs_psi, u_init))
     B, N = x0.shape[0], p.N
     Z = np.empty((B, N + 1, 7)); U = np.empty((B, N, 2)); cost = np.empty(B); viol = np.empty(B)
     status = np.empty(B, dtype=np.int32); iters = np.empty(B, dtype=np.int32)
     rc = lib().hostsim_solve_obca(C.byref(p), B, _ptr(x0), _ptr(u_prev), _ptr(curv), _ptr(obs), _ptr(obs_psi), _ptr(u_init),
                                   _ptr(Z), _ptr(U), _ptr(cost), _ptr(viol), status.ctypes.data_as(C.POINTER(C.c_int)),
-                                  iters.ctypes.data_as(C.POINTER(C.c_int)))
+                                  iters.ctypes.data_as(C.POINTER(C.c_int)), int(bool(lanes)))
     assert rc == 0
     return dict(Z=Z, U=U, cost=cost, viol=viol, status=status, iters=iters)
 

@@ -12,7 +12,7 @@ template <typename T, bool OBCA = false>
 static int run(const igt_params *p, int B, const double *x0, const double *u_prev, const double *curv,
                const double *obs, const double *obs_psi, const double *ctx, const double *u_init, double *x, double *u, double *cost,
                double *viol, int *status, int *iters, int n_layers, const int *dims, const double *const *W,
-               const double *const *b, const double *Wn, const double *mu_f, double sigma_t, double mu_t)
+               const double *const *b, const double *Wn, const double *mu_f, double sigma_t, double mu_t, bool lanes = false)
 {
     DevParams<T> P;
     fill_dev_params(*p, P);
@@ -37,30 +37,46 @@ static int run(const igt_params *p, int B, const double *x0, const double *u_pre
     std::vector<double> guess((size_t)2 * p->N);
     ProbIO io = { x0, u_prev, curv, obs, ctx, u_init, x, u, cost, viol, status, iters };
     io.obs_psi = obs_psi;
-    for (long q = 0; q < B; q++) solve_problem<T, OBCA>(P, io, ws.data(), q % 32, q, guess.data(), scratch.data(), width);
+    if (!lanes) {
+        for (long q = 0; q < B; q++) solve_problem<T, OBCA>(P, io, ws.data(), q % 32, q, guess.data(), scratch.data(), width);
+        return 0;
+    }
+    // persistent lanes, as in the kernels: one solver object per slot, bound once; slot q % 32 solves problems
+    // q, q + 32, ... one after the other without the object being rebuilt in between
+    std::vector<Solver<T, Ws<T, 32, OBCA>>> sv;
+    sv.reserve(32);
+    for (int s = 0; s < 32; s++) {
+        sv.emplace_back(P);
+        sv[s].w.init_layout(P.N, P.n_cinf);
+        sv[s].w.bind(ws.data(), s);
+        sv[s].mlp_scratch = scratch.data(); sv[s].mlp_width = width;
+    }
+    for (long q = 0; q < B; q++) solve_bound(sv[q % 32], io, q, guess.data());
     return 0;
 }
 
 extern "C" {
 int hostsim_default_params(igt_params *p, int precision) { return default_params(p, precision); }
 
+// lanes = 0: a fresh solver object per problem; lanes != 0: one object per slot, reused for every 32nd problem (the
+// kernels' persistent lanes).  Both write problem q's results to row q.
 int hostsim_solve(const igt_params *p, int B, const double *x0, const double *u_prev, const double *curv,
                   const double *obs, const double *ctx, const double *u_init, double *x, double *u, double *cost,
                   double *viol, int *status, int *iters, int n_layers, const int *dims, const double *const *W,
-                  const double *const *b, const double *Wn, const double *mu_f, double sigma_t, double mu_t)
+                  const double *const *b, const double *Wn, const double *mu_f, double sigma_t, double mu_t, int lanes)
 {
     if (p->precision == IGT_PREC_F64)
-        return run<double>(p, B, x0, u_prev, curv, obs, nullptr, ctx, u_init, x, u, cost, viol, status, iters, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t);
-    return run<float>(p, B, x0, u_prev, curv, obs, nullptr, ctx, u_init, x, u, cost, viol, status, iters, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t);
+        return run<double>(p, B, x0, u_prev, curv, obs, nullptr, ctx, u_init, x, u, cost, viol, status, iters, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t, lanes != 0);
+    return run<float>(p, B, x0, u_prev, curv, obs, nullptr, ctx, u_init, x, u, cost, viol, status, iters, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t, lanes != 0);
 }
 
-// OBCA collision mode (obs_psi[B][N+1] obstacle headings), fp64, 'mpc' cost
+// OBCA collision mode (obs_psi[B][N+1] obstacle headings), fp64, 'mpc' cost.  lanes: as in hostsim_solve
 int hostsim_solve_obca(const igt_params *p, int B, const double *x0, const double *u_prev, const double *curv,
                        const double *obs, const double *obs_psi, const double *u_init, double *x, double *u, double *cost,
-                       double *viol, int *status, int *iters)
+                       double *viol, int *status, int *iters, int lanes)
 {
     return run<double, true>(p, B, x0, u_prev, curv, obs, obs_psi, nullptr, u_init, x, u, cost, viol, status, iters, 0,
-                             nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0);
+                             nullptr, nullptr, nullptr, nullptr, nullptr, 0.0, 0.0, lanes != 0);
 }
 
 // rectangle signed distance + gradient (csrc/obca.cuh) for n pose pairs: ego[n][3], obs[n][3] -> d[n], g[n][3]

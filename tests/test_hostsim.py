@@ -114,3 +114,43 @@ def test_product_solver_code_obca_mode_matches_oracle(oracle_params):
     dmin = [min(obca.rect_distance(o["Z"][i][k, [0, 1, 6]], np.array([pb.obs[i, k, 0], pb.obs[i, k, 1], pb.obs_psi[i, k]]))[0]
                 for k in range(1, N + 1)) for i in np.where(ok)[0]]
     assert min(dmin) < 1e-5 and min(dmin) > -1e-9
+
+
+def _lane_batch(B, seed):
+    """B mid_episode problems with problems that init rejects (v and ey outside their limits, NaN v) and problems
+    with a non-finite state that init accepts and the solve then fails on, spread over the batch"""
+    pb = S.mid_episode(B, N=40, seed=seed)
+    x0 = pb.x0.copy()
+    bad = np.random.default_rng(seed).choice(B, 12, replace=False)
+    for i, q in enumerate(bad):
+        col, val = ((5, 5.5), (5, -0.4), (3, 0.3), (5, np.nan), (0, np.nan), (2, np.inf))[i % 6]
+        x0[q, col] = val
+    return pb, x0, bad
+
+
+@pytest.mark.parametrize("case", ["f64", "f32", "obca", "gt_mpc"])
+def test_core_lane_reuse_equals_fresh_solver_objects(cinf, case):
+    """The kernels keep one Solver object per lane and hand it problem after problem; Solver::init must leave nothing
+    of the previous problem that the next solve reads.  Slot q % 32 of the harness solves problems q, q + 32, ... with
+    one object (10 problems per slot here), bit-identical to a fresh object per problem -- with rejected problems, failed
+    solves and an iteration cap low enough for capped ones (status 1 / 6) in the mix."""
+    from tests.test_value_nets import shipped_net
+    from oracle import nlp
+    B = 320
+    pb, x0, bad = _lane_batch(B, seed=31)
+    p = H.default_params(0 if case == "f32" else 1)
+    p.set_cinf(*cinf)
+    p.max_iter = 25
+    if case == "obca":
+        p.d_min = 0.0
+        run = lambda lanes: H.solve_obca(p, x0, pb.u_prev, pb.curv, pb.obs, pb.obs_psi, lanes=lanes)
+    else:
+        mlp = nlp.MLPTerm(**shipped_net(3)[0]) if case == "gt_mpc" else None
+        ctx = pb.nn_ctx if case == "gt_mpc" else None
+        run = lambda lanes: H.solve(p, x0, pb.u_prev, pb.curv, pb.obs, nn_ctx=ctx, mlp=mlp, lanes=lanes)
+    fresh, reused = run(False), run(True)
+    for k in ("status", "iters", "cost", "viol", "U", "Z"):
+        assert np.array_equal(reused[k], fresh[k], equal_nan=True), k
+    st = fresh["status"]
+    assert np.all(st[bad] != 0) and (st[bad] == 2).sum() >= 8
+    assert (st == 0).mean() > 0.5 and len(set(st[st != 0]) - {2}) >= 2     # more than one failure status besides 2
