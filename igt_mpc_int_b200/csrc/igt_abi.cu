@@ -83,12 +83,36 @@ __global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(typename std::con
 // its whole workspace in shared memory (stride-1 layout), so the sweeps of the problem's one owner thread run at
 // shared-memory latency instead of an L2 round trip per stage; the node phases and the line-search candidates
 // are dealt out over the CTA's 256 threads as in the throughput kernel.  Same code, same arithmetic, same results.
-template <typename T, bool OBCA>
-__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_small_kernel(ProbIO io, long B, Sched sc, const double *guess, int cs)
+// GT: gt_mpc, with the value term evaluated by the CTA (COOP: exact cooperative evaluation, its buffers sized for one
+// problem's requests and placed before the workspace) or by the owner thread (its [2][6][width] scratch slab in global
+// memory, one per CTA); BANK: the network bank, as in solve_kernel.  The tensor-core value term is not offered here.
+template <typename IO, typename T>
+struct SmallIO : IO {                                     // inputs of a gt_mpc latency solve: IO and the per-thread scratch
+    T *mlp_scratch = nullptr;                             // [grid][2][6][mlp_width], null with COOP
+    int mlp_width = 0;
+};
+// (rounded up to 16 bytes: the workspace that follows keeps the alignment of the start of dynamic shared memory, which
+// the shared solver functions are compiled for)
+template <typename T, bool COOP, bool BANK>
+constexpr int small_coop_bytes()
+{
+    return COOP ? ((BANK ? mlp_coop_bank_smem_bytes<T, COOP_CAP>(SOLVE_BLOCK) : mlp_coop_smem_bytes<T, COOP_CAP>(SOLVE_BLOCK)) + 15) & ~15 : 0;
+}
+template <typename T, bool OBCA, bool COOP = false, bool BANK = false, bool GT = COOP || BANK>
+__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_small_kernel(
+    typename std::conditional<GT, SmallIO<typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type, T>, ProbIO>::type io,
+    long B, Sched sc, const double *guess, int cs)
 {
     extern __shared__ __align__(16) uint8_t dyn_smem[];
     const DevParams<T> &P = ConstP<T>::get(cs);
-    solve_persistent<T, false, 1, OBCA>(P, io, reinterpret_cast<T *>(dyn_smem), 0, B, sc, guess, (T *)nullptr, 0, nullptr, 1, cs);
+    if constexpr (GT) {
+        constexpr int off = small_coop_bytes<T, COOP, BANK>();   // dynamic shared memory: [value term (COOP)] [workspace]
+        T *scr = io.mlp_scratch ? io.mlp_scratch + (long)blockIdx.x * 12 * io.mlp_width : nullptr;
+        solve_persistent<T, false, 1, OBCA, COOP, false, BANK>(P, io, reinterpret_cast<T *>(dyn_smem + off), 0, B, sc, guess, scr,
+                                                               io.mlp_width, nullptr, 1, cs, dyn_smem);
+    } else {
+        solve_persistent<T, false, 1, OBCA>(P, io, reinterpret_cast<T *>(dyn_smem), 0, B, sc, guess, (T *)nullptr, 0, nullptr, 1, cs);
+    }
 }
 
 // fp32 rollout with Kahan-compensated accumulation of the RK4 increments (x, y, s reach ~50 m
@@ -339,6 +363,8 @@ struct igt_handle {
     void *guess = nullptr; size_t guess_bytes = 0;     // cold-start controls [B][N][2] + the work counter
     void *episode = nullptr; size_t episode_bytes = 0; // igt_episode_run_host: state, records, solver inputs / outputs
     int n_sm = 0;
+    int smem_optin = 0;                // shared memory a block may opt in to (the gt_mpc latency path's limit)
+    int small_static[8] = { -1, -1, -1, -1, -1, -1, -1, -1 };   // static shared memory of each k_small_gt kernel, -1: not read yet
     long long launches = 0;
     std::string err;
     int device = 0;
@@ -435,6 +461,43 @@ static int end_call(igt_handle *h, cudaStream_t st, int prec_used_mask)
     return IGT_OK;
 }
 
+// The gt_mpc instantiations of the latency kernel, by small_gt_variant: cooperative value term (circle mode, f64, every
+// layer <= MLP_COOP_W), then per-thread in f64 circle mode, OBCA and f32; each with one network and with the bank.
+static const void *const k_small_gt[8] = {
+    (const void *)solve_small_kernel<double, false, true, false>, (const void *)solve_small_kernel<double, false, true, true>,
+    (const void *)solve_small_kernel<double, false, false, false, true>, (const void *)solve_small_kernel<double, false, false, true>,
+    (const void *)solve_small_kernel<double, true, false, false, true>, (const void *)solve_small_kernel<double, true, false, true>,
+    (const void *)solve_small_kernel<float, false, false, false, true>, (const void *)solve_small_kernel<float, false, false, true>,
+};
+static int small_gt_variant(bool coop, bool bank, bool obca, bool f64) { return (coop ? 0 : obca ? 4 : f64 ? 2 : 6) + (bank ? 1 : 0); }
+
+// whether gt_mpc variant v fits one block's shared memory with `dyn` bytes of workspace and value-term buffers: the
+// kernel's static shared memory is read once per handle
+static int small_gt_fits(igt_handle *h, int v, size_t dyn, bool *fits)
+{
+    if (h->small_static[v] < 0) {
+        cudaFuncAttributes a;
+        CK(cudaFuncGetAttributes(&a, k_small_gt[v]));
+        h->small_static[v] = (int)a.sharedSizeBytes;
+    }
+    *fits = dyn + (size_t)h->small_static[v] <= (size_t)h->smem_optin;
+    return IGT_OK;
+}
+
+template <typename T, bool OBCA, bool COOP, bool BANK>
+static int launch_small_gt(igt_handle *h, const ProbIONet<T> &iob, int B, Sched sc, const double *guess, T *scratch, int width,
+                           size_t smem, int cs, cudaStream_t st)
+{
+    using IO = typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type;
+    SmallIO<IO, T> io;
+    static_cast<IO &>(io) = iob;
+    io.mlp_scratch = COOP ? nullptr : scratch;
+    io.mlp_width = width;
+    CK(cudaFuncSetAttribute(solve_small_kernel<T, OBCA, COOP, BANK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    solve_small_kernel<T, OBCA, COOP, BANK, true><<<B, SOLVE_BLOCK, smem, st>>>(io, B, sc, guess, cs);
+    return IGT_OK;
+}
+
 extern "C" {
 
 const char *igt_version(void) { return "igtmpc 0.1 sm_100a"; }
@@ -463,6 +526,7 @@ int igt_create(const igt_params *p, igt_handle **out)
     }
     cudaDeviceGetAttribute(&h->n_sm, cudaDevAttrMultiProcessorCount, h->device);
     if (h->n_sm <= 0) h->n_sm = 148;
+    cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device);
     *out = h;
     return IGT_OK;
 }
@@ -718,9 +782,21 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
     if (rc) return rc;
     WsLayout L; L.init(h->prm.N, h->prm.n_cinf, obca ? NGE_OBCA : NGE, obca ? NHE_OBCA : NHE);
     size_t esz = f64 ? 8 : 4;
-    // latency path: at most one problem per SM and a workspace that fits shared memory next to the work lists
-    const size_t small_smem = (size_t)L.total * esz;
-    const bool small = h->use_small && !nn_ctx && B <= h->n_sm && small_smem <= 200 * 1024;
+    // value term (OBCA + gt_mpc: per-thread value term; a bank: exact evaluation whatever tensor_core_mlp says)
+    const bool use_tc = nn_ctx && !bank && h->tc.enabled && h->use_tc && !obca;
+    const int width = bank ? bank_width(h) : h->mlp_width;
+    const bool use_coop = nn_ctx && !use_tc && f64 && (bank ? width <= MLP_COOP_W : h->coop_ok) && !obca;
+    // latency path: at most one problem per SM and a workspace that fits shared memory next to the work lists; in
+    // gt_mpc (not with the tensor-core value term) the kernel's whole shared memory -- static, value-term buffers,
+    // workspace -- within the device's opt-in limit per block
+    const int small_v = small_gt_variant(use_coop, bank, obca, f64);
+    size_t small_smem = (size_t)L.total * esz;
+    bool small = h->use_small && !nn_ctx && B <= h->n_sm && small_smem <= 200 * 1024;
+    if (h->use_small && nn_ctx && !use_tc && B <= h->n_sm) {
+        if (use_coop) small_smem += bank ? small_coop_bytes<double, true, true>() : small_coop_bytes<double, true, false>();
+        rc = small_gt_fits(h, small_v, small_smem, &small);
+        if (rc) return rc;
+    }
     // persistent lanes: one CTA of SOLVE_BLOCK threads per SM.  A batch smaller than the machine is spread
     // over all SMs, a whole number of warps each: `quota` threads per CTA fetch problems, the rest of
     // the CTA only helps in the CTA-wide phases (and adopts stragglers in the tail).
@@ -733,12 +809,9 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
     long n_slots = n_cta * bs;
     rc = small ? IGT_OK : grow(h, &h->ws, &h->ws_bytes, (size_t)L.total * n_slots * esz, st);
     if (rc) return rc;
-    // (OBCA + gt_mpc: per-thread value term; a bank: exact evaluation whatever tensor_core_mlp says)
-    const bool use_tc = nn_ctx && !bank && h->tc.enabled && h->use_tc && !obca;
-    const int width = bank ? bank_width(h) : h->mlp_width;
-    const bool use_coop = nn_ctx && !use_tc && f64 && (bank ? width <= MLP_COOP_W : h->coop_ok) && !obca;
     if (nn_ctx && !use_tc && !use_coop) {                                 // per-thread evaluation: activations in HBM
-        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * n_slots * esz, st);
+        // (one slab per persistent lane, or per CTA on the latency path)
+        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * (small ? B : n_slots) * esz, st);
         if (rc) return rc;
     }
     // scheduler block (the work counter), then the cold-start guesses
@@ -767,7 +840,22 @@ static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *
         h->launches++;
     }
     int gs = (int)(n_slots / bs);
-    if (small) {
+    if (small && nn_ctx) {
+        // gt_mpc: the latency kernel's value-term instantiations (a bank problem with a bad index gets IGT_STATUS_BAD_NET)
+        double *scr = (double *)h->mlp_scratch;
+        float *scr_f = (float *)h->mlp_scratch;
+        switch (small_v) {
+        case 0: rc = launch_small_gt<double, false, true, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 1: rc = launch_small_gt<double, false, true, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 2: rc = launch_small_gt<double, false, false, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 3: rc = launch_small_gt<double, false, false, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 4: rc = launch_small_gt<double, true, false, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 5: rc = launch_small_gt<double, true, false, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
+        case 6: rc = launch_small_gt<float, false, false, false>(h, iob_f32(iob, h), B, sc, guess, scr_f, width, small_smem, cs, st); break;
+        default: rc = launch_small_gt<float, false, false, true>(h, iob_f32(iob, h), B, sc, guess, scr_f, width, small_smem, cs, st); break;
+        }
+        if (rc) return rc;
+    } else if (small) {
         if (obca) {
             CK(cudaFuncSetAttribute(solve_small_kernel<double, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
             solve_small_kernel<double, true><<<B, bs, small_smem, st>>>(io, B, sc, guess, cs);

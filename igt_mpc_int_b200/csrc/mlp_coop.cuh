@@ -17,6 +17,14 @@
 // same waves with its own descriptor, biases and output layer staged in shared memory.  The operation order per output
 // is unchanged, so a request's result is bit-identical to the single-network evaluation of its network, whatever
 // shares its wave.
+//
+// Request capacity (template argument CAP of both entry points and their size functions).  CAP = 0: one request slot
+// per thread and COOP_E evaluations per warp and wave (the throughput kernels).  CAP > 0: slots for CAP requests only,
+// one evaluation per warp and wave, and weight tiles of COOP_TI_CAP inputs -- the latency kernel, whose CTA holds one
+// problem and so asks for at most n_alpha <= MAX_ALPHA = COOP_CAP values at a time (the first candidate of its line
+// search, its speculative halvings, or the value at a fresh problem), next to its workspace in shared memory; a request
+// takes the slot of its position in the compacted list.  The operation order per output does not depend on the tile
+// size (inputs in ascending order, the one zero pad row of an odd layer last), so both capacities give the same bits.
 #pragma once
 #include <cstdint>
 
@@ -26,21 +34,31 @@ constexpr int MLP_COOP_W = 128;                       // widest layer handled
 constexpr int COOP_ITEM = 8, COOP_ROWS = 6;
 constexpr int COOP_E = 2;                             // evaluations per warp and wave
 constexpr int COOP_TI = 16;                           // inputs per weight tile
-// [requests block x 8] [results block x 6] [activations warps x E x 6 x W] [weight tiles 2 x TI x W]
-// [biases of every layer + the output layer's weights: (MAX_MLP_LAYERS + 1) x W] [list: block + warps ints]
-template <typename T>
+constexpr int COOP_CAP = MAX_ALPHA;                   // request capacity of the latency kernel's buffers
+constexpr int COOP_TI_CAP = 8;                        // inputs per weight tile with a request capacity
+template <int CAP>
+struct CoopShape {
+    static constexpr int E = CAP ? 1 : COOP_E;        // evaluations per warp and wave
+    static constexpr int TI = CAP ? COOP_TI_CAP : COOP_TI;
+    static constexpr int slots(int block) { return CAP ? CAP : block; }        // request / result slots
+    static constexpr int act_warps(int block) { return CAP ? CAP : block / 32; }   // warps with activation rows
+};
+// [requests slots x 8] [results slots x 6] [activations act_warps x E x 6 x W] [weight tiles 2 x TI x W]
+// [biases of every layer + the output layer's weights: (MAX_MLP_LAYERS + 1) x W] [list: slots + warps ints]
+template <typename T, int CAP = 0>
 constexpr int mlp_coop_smem_bytes(int block)
 {
-    return (int)sizeof(T) * (block * (COOP_ITEM + COOP_ROWS) + (block / 32) * COOP_E * COOP_ROWS * MLP_COOP_W + 2 * COOP_TI * MLP_COOP_W +
-                             (MAX_MLP_LAYERS + 1) * MLP_COOP_W) + 4 * (block + 32);
+    using S = CoopShape<CAP>;
+    return (int)sizeof(T) * (S::slots(block) * (COOP_ITEM + COOP_ROWS) + S::act_warps(block) * S::E * COOP_ROWS * MLP_COOP_W +
+                             2 * S::TI * MLP_COOP_W + (MAX_MLP_LAYERS + 1) * MLP_COOP_W) + 4 * (S::slots(block) + 32);
 }
 // the bank variant appends the current group's descriptor and the per-warp group counts [MAX_MLP_NETS][32]
 template <typename T>
 constexpr int mlp_coop_desc_bytes() { return (int)((sizeof(MlpNet<T>) + 15) / 16 * 16); }
-template <typename T>
+template <typename T, int CAP = 0>
 constexpr int mlp_coop_bank_smem_bytes(int block)
 {
-    return mlp_coop_smem_bytes<T>(block) + mlp_coop_desc_bytes<T>() + 4 * MAX_MLP_NETS * 32;
+    return mlp_coop_smem_bytes<T, CAP>(block) + mlp_coop_desc_bytes<T>() + 4 * MAX_MLP_NETS * 32;
 }
 
 #ifdef __CUDACC__
@@ -63,8 +81,8 @@ __device__ __forceinline__ void coop_load_tile(T *tile, const T *Wt, int i0, int
 
 // acc[e][j][r] += sum over the tile's inputs of weight(input, output lane + 32 j) * activation row r of evaluation e,
 // inputs in ascending order per accumulator (as mlp_eval_thread); two inputs per pass, all loads unguarded
-template <int NE, typename T>
-__device__ __forceinline__ void coop_tile_fma(T (&acc)[COOP_E][4][6], const T *tile_lane, const T *act_i0, int rows2)
+template <int NE, int E, typename T>
+__device__ __forceinline__ void coop_tile_fma(T (&acc)[E][4][6], const T *tile_lane, const T *act_i0, int rows2)
 {
     constexpr int W = MLP_COOP_W;
 #pragma unroll 2
@@ -105,11 +123,11 @@ __device__ __forceinline__ void coop_stage(const NP &P, T *bias, T *wlast)
 }
 
 // the waves of the nv requests list[0 .. nv) through network P (staged by coop_stage); CTA-uniform
-template <typename T, typename NP>
+template <int CAP, typename T, typename NP>
 __device__ __forceinline__ void coop_waves(const NP &P, const T *items, T *res, T *act, T *tiles, const T *bias, const T *wlast,
                                            const int *list, int nv)
 {
-    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    constexpr int W = MLP_COOP_W, E = CoopShape<CAP>::E, TI = CoopShape<CAP>::TI;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
     for (int wave0 = 0; wave0 < nv; wave0 += nw * E) {             // CTA-uniform
         int ev[E];
@@ -158,7 +176,7 @@ __device__ __forceinline__ void coop_waves(const NP &P, const T *items, T *res, 
                     if (!any) continue;
                     const T *tile_lane = tiles + (t & 1) * TI * W + lane;
                     const int i0 = t * TI, rows = nin - i0 < TI ? nin - i0 : TI, rows2 = (rows + 1) & ~1;
-                    if (two) coop_tile_fma<E>(acc, tile_lane, act + i0, rows2);
+                    if (E > 1 && two) coop_tile_fma<E>(acc, tile_lane, act + i0, rows2);
                     else coop_tile_fma<1>(acc, tile_lane, act + i0, rows2);
                 }
                 __syncthreads();                                   // the last tile's buffer is free for the next layer's first
@@ -214,58 +232,102 @@ __device__ __forceinline__ void coop_waves(const NP &P, const T *items, T *res, 
 
 // CTA-uniform call (like mlp_tc_eval): every thread passes its own request (valid = false: none) and gets
 // out[6] = (V, dV/ds, dV/dv, d2V/dss, d2V/dsv, d2V/dvv), already scaled by sigma_t (+ mu_t on V).
-template <typename T>
+// Shared memory: mlp_coop_smem_bytes<T, CAP>.
+template <typename T, int CAP = 0>
 __device__ __noinline__ void mlp_coop_eval(const DevParams<T> &P, uint8_t *smem, bool valid, T sN, T vN, const T *ctx, T *out)
 {
-    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    constexpr int W = MLP_COOP_W, E = CoopShape<CAP>::E, TI = CoopShape<CAP>::TI;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nthr = blockDim.x, nw = nthr >> 5;
-    T *items = reinterpret_cast<T *>(smem);                       // [nthr][8]: sN, vN, ctx[4]
-    T *res = items + nthr * COOP_ITEM;                            // [nthr][6]
-    T *act = res + nthr * COOP_ROWS + warp * (E * COOP_ROWS * W); // this warp's [E][6][W] activation rows (updated in place)
-    T *tiles = res + nthr * COOP_ROWS + nw * (E * COOP_ROWS * W); // [2][TI][W]
+    const int ns = CAP ? CAP : nthr, na = CAP ? CAP : nw;       // request slots, warps with activation rows
+    T *items = reinterpret_cast<T *>(smem);                       // [slots][8]: sN, vN, ctx[4]
+    T *res = items + ns * COOP_ITEM;                              // [slots][6]
+    T *act = res + ns * COOP_ROWS + warp * (E * COOP_ROWS * W);   // this warp's [E][6][W] activation rows (updated in place)
+    T *tiles = res + ns * COOP_ROWS + na * (E * COOP_ROWS * W);   // [2][TI][W]
     T *bias = tiles + 2 * TI * W, *wlast = bias + MAX_MLP_LAYERS * W;   // [layers][W], [W]: staged once per call
-    int *list = reinterpret_cast<int *>(wlast + W), *wcnt = list + nthr;
+    int *list = reinterpret_cast<int *>(wlast + W), *wcnt = list + ns;
     coop_stage(P, bias, wlast);
-    for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
-    items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
+    if (CAP == 0 || warp < CAP)
+        for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
+    if constexpr (CAP == 0) {                                     // slot = thread
+        items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
 #pragma unroll
-    for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+        for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+    }
     // the valid requests in thread order
     const unsigned vm = __ballot_sync(0xffffffffu, valid);
     if (lane == 0) wcnt[warp] = __popc(vm);
     __syncthreads();
     int base = 0, nv = 0;
     for (int i = 0; i < nw; i++) { const int c = wcnt[i]; if (i < warp) base += c; nv += c; }
-    if (valid) list[base + __popc(vm & ((1u << lane) - 1u))] = tid;
-    __syncthreads();
-    coop_waves(P, items, res, act, tiles, bias, wlast, list, nv);
-    __syncthreads();
-    if (valid) {
+    if constexpr (CAP == 0) {
+        if (valid) list[base + __popc(vm & ((1u << lane) - 1u))] = tid;
+        __syncthreads();
+        coop_waves<CAP>(P, items, res, act, tiles, bias, wlast, list, nv);
+        __syncthreads();
+        if (valid) {
 #pragma unroll
-        for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];
+            for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];
+        }
+    } else {                                                      // slot = position in the list (at most CAP requests)
+        if (nv > CAP) __trap();                                   // (the caller's bound, see the file comment)
+        const int sl = base + __popc(vm & ((1u << lane) - 1u));
+        if (valid) {
+            items[sl * COOP_ITEM + 0] = sN; items[sl * COOP_ITEM + 1] = vN;
+#pragma unroll
+            for (int i = 0; i < 4; i++) items[sl * COOP_ITEM + 2 + i] = ctx[i];
+        }
+        if (tid < CAP) list[tid] = tid;
+        __syncthreads();
+        coop_waves<CAP>(P, items, res, act, tiles, bias, wlast, list, nv);
+        __syncthreads();
+        if (valid) {
+#pragma unroll
+            for (int r = 0; r < 6; r++) out[r] = res[sl * COOP_ROWS + r];
+        }
     }
     __syncthreads();
 }
 
+// one network group of the bank evaluation: nets[g] -> desc and the staged biases, then the waves of list[0 .. n)
+template <int CAP, typename T>
+__device__ __forceinline__ void coop_bank_group(const MlpNet<T> *nets, int g, MlpNet<T> *desc, const T *items, T *res, T *act,
+                                                T *tiles, T *bias, T *wlast, const int *list, int n)
+{
+    {   // descriptor -> shared memory (the previous group's waves are done with it: barrier at their end)
+        const int *src = reinterpret_cast<const int *>(nets + g);
+        int *dst = reinterpret_cast<int *>(desc);
+        for (int i = threadIdx.x; i < (int)(sizeof(MlpNet<T>) / 4); i += blockDim.x) dst[i] = src[i];
+    }
+    __syncthreads();
+    coop_stage(*desc, bias, wlast);
+    __syncthreads();
+    coop_waves<CAP>(*desc, items, res, act, tiles, bias, wlast, list, n);
+    __syncthreads();
+}
+
 // The same over a network bank: request t uses nets[net] (0 <= net < MAX_MLP_NETS, a loaded slot: the callers check).
-// Shared memory: mlp_coop_bank_smem_bytes.
-template <typename T>
+// Shared memory: mlp_coop_bank_smem_bytes<T, CAP>.
+template <typename T, int CAP = 0>
 __device__ __noinline__ void mlp_coop_eval_bank(const MlpNet<T> *nets, uint8_t *smem, bool valid, int net, T sN, T vN, const T *ctx, T *out)
 {
-    constexpr int W = MLP_COOP_W, E = COOP_E, TI = COOP_TI;
+    constexpr int W = MLP_COOP_W, E = CoopShape<CAP>::E, TI = CoopShape<CAP>::TI;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nthr = blockDim.x, nw = nthr >> 5;
+    const int ns = CAP ? CAP : nthr, na = CAP ? CAP : nw;
     T *items = reinterpret_cast<T *>(smem);
-    T *res = items + nthr * COOP_ITEM;
-    T *act = res + nthr * COOP_ROWS + warp * (E * COOP_ROWS * W);
-    T *tiles = res + nthr * COOP_ROWS + nw * (E * COOP_ROWS * W);
+    T *res = items + ns * COOP_ITEM;
+    T *act = res + ns * COOP_ROWS + warp * (E * COOP_ROWS * W);
+    T *tiles = res + ns * COOP_ROWS + na * (E * COOP_ROWS * W);
     T *bias = tiles + 2 * TI * W, *wlast = bias + MAX_MLP_LAYERS * W;   // staged once per group
     int *list = reinterpret_cast<int *>(wlast + W);
-    MlpNet<T> *desc = reinterpret_cast<MlpNet<T> *>(smem + mlp_coop_smem_bytes<T>(nthr));   // the current group's network
+    MlpNet<T> *desc = reinterpret_cast<MlpNet<T> *>(smem + mlp_coop_smem_bytes<T, CAP>(nthr));   // the current group's network
     int *gcnt = reinterpret_cast<int *>(reinterpret_cast<uint8_t *>(desc) + mlp_coop_desc_bytes<T>());   // [net][warp]
-    for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
-    items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
+    if (CAP == 0 || warp < CAP)
+        for (int idx = lane; idx < E * COOP_ROWS * W; idx += 32) act[idx] = T(0);
+    if constexpr (CAP == 0) {
+        items[tid * COOP_ITEM + 0] = sN; items[tid * COOP_ITEM + 1] = vN;
 #pragma unroll
-    for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+        for (int i = 0; i < 4; i++) items[tid * COOP_ITEM + 2 + i] = ctx[i];
+    }
     // counting sort of the valid requests by network: group g holds its requests in thread order
     int rank = 0;
     for (int g = 0; g < MAX_MLP_NETS; g++) {
@@ -275,32 +337,48 @@ __device__ __noinline__ void mlp_coop_eval_bank(const MlpNet<T> *nets, uint8_t *
         if (mine) rank = __popc(m & ((1u << lane) - 1u));
     }
     __syncthreads();
-    if (valid && (unsigned)net < (unsigned)MAX_MLP_NETS) {
-        int base = rank;
-        for (int g = 0; g <= net; g++)
-            for (int i = 0; i < nw; i++) if (g < net || i < warp) base += gcnt[g * nw + i];
-        list[base] = tid;
-    }
-    __syncthreads();
-    for (int g = 0, start = 0; g < MAX_MLP_NETS; g++) {           // CTA-uniform
-        int n = 0;
-        for (int i = 0; i < nw; i++) n += gcnt[g * nw + i];
-        if (n == 0) continue;
-        {   // descriptor -> shared memory (the previous group's waves are done with it: barrier at their end)
-            const int *src = reinterpret_cast<const int *>(nets + g);
-            int *dst = reinterpret_cast<int *>(desc);
-            for (int i = tid; i < (int)(sizeof(MlpNet<T>) / 4); i += nthr) dst[i] = src[i];
+    if constexpr (CAP == 0) {
+        if (valid && (unsigned)net < (unsigned)MAX_MLP_NETS) {
+            int base = rank;
+            for (int g = 0; g <= net; g++)
+                for (int i = 0; i < nw; i++) if (g < net || i < warp) base += gcnt[g * nw + i];
+            list[base] = tid;
         }
         __syncthreads();
-        coop_stage(*desc, bias, wlast);
-        __syncthreads();
-        coop_waves(*desc, items, res, act, tiles, bias, wlast, list + start, n);
-        __syncthreads();
-        start += n;
-    }
-    if (valid) {
+        for (int g = 0, start = 0; g < MAX_MLP_NETS; g++) {       // CTA-uniform
+            int n = 0;
+            for (int i = 0; i < nw; i++) n += gcnt[g * nw + i];
+            if (n == 0) continue;
+            coop_bank_group<CAP>(nets, g, desc, items, res, act, tiles, bias, wlast, list + start, n);
+            start += n;
+        }
+        if (valid) {
 #pragma unroll
-        for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];
+            for (int r = 0; r < 6; r++) out[r] = res[tid * COOP_ROWS + r];
+        }
+    } else {                                                      // slot = position in the sorted list (at most CAP requests)
+        const bool listed = valid && (unsigned)net < (unsigned)MAX_MLP_NETS;
+        int sl = rank;
+        if (listed) {
+            for (int g = 0; g <= net; g++)
+                for (int i = 0; i < nw; i++) if (g < net || i < warp) sl += gcnt[g * nw + i];
+            if (sl >= CAP) __trap();
+            items[sl * COOP_ITEM + 0] = sN; items[sl * COOP_ITEM + 1] = vN;
+#pragma unroll
+            for (int i = 0; i < 4; i++) items[sl * COOP_ITEM + 2 + i] = ctx[i];
+        }
+        if (tid < CAP) list[tid] = tid;
+        for (int g = 0, start = 0; g < MAX_MLP_NETS; g++) {       // CTA-uniform (the first group's barriers publish the items)
+            int n = 0;
+            for (int i = 0; i < nw; i++) n += gcnt[g * nw + i];
+            if (n == 0) continue;
+            coop_bank_group<CAP>(nets, g, desc, items, res, act, tiles, bias, wlast, list + start, n);
+            start += n;
+        }
+        if (listed) {
+#pragma unroll
+            for (int r = 0; r < 6; r++) out[r] = res[sl * COOP_ROWS + r];
+        }
     }
     __syncthreads();
 }

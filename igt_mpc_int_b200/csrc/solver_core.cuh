@@ -1857,10 +1857,11 @@ __device__ __forceinline__ int cta_list_build(bool need, long bound, const S &sv
 // which the translation unit defines.  BANK does not change what they compute: it only gives the bank kernels
 // instantiations of their own, so that each instantiation keeps a single calling kernel (NVVM then binds the work list
 // argument to that kernel's __shared__ NodeList instead of passing a generic pointer) and the other kernels compile as
-// they would without the bank.
+// they would without the bank.  OWN does the same for the latency kernels with the cooperative value term, whose
+// solver loop is otherwise the plain latency kernel's.
 template <typename T> struct ConstP;
 
-template <typename T, int PHASE, int STRIDE, bool OBCA, bool RSTG, bool BANK>
+template <typename T, int PHASE, int STRIDE, bool OBCA, bool RSTG, bool BANK, bool OWN = false>
 __device__ __noinline__ void phase_items(T *ws_base, const NodeList<T> *nl, int n, int n_spec)
 {
     const DevParams<T> &P = ConstP<T>::get(nl->cslot);
@@ -1888,12 +1889,12 @@ __device__ __noinline__ void phase_items(T *ws_base, const NodeList<T> *nl, int 
     }
 }
 
-template <typename T, int PHASE, int STRIDE, bool RSTG, typename S>
+template <typename T, int PHASE, int STRIDE, bool RSTG, typename S, bool OWN = false>
 __device__ __forceinline__ void node_phase_cta(const DevParams<T> &P, T *ws_base, const WsLayout &L, bool need,
                                                long bound, const S &sv, NodeList<T> &nl)
 {
     const int n = cta_list_build(need, bound, sv, nl);
-    if (n > 0) phase_items<T, PHASE, STRIDE, S::obca, RSTG, S::bank>(ws_base, &nl, n, 1);
+    if (n > 0) phase_items<T, PHASE, STRIDE, S::obca, RSTG, S::bank, OWN>(ws_base, &nl, n, 1);
     __syncthreads();
 }
 
@@ -1913,7 +1914,7 @@ __device__ long long g_mid_t;            // debug: end of the rollouts of CTA 0'
 #ifndef IGT_SPEC_BUDGET
 #define IGT_SPEC_BUDGET IGT_MAX_SOLVE_BLOCK
 #endif
-template <typename T, int STRIDE, bool RSTG, typename S>
+template <typename T, int STRIDE, bool RSTG, typename S, bool OWN = false>
 __device__ __forceinline__ int trial_phase_cta(const DevParams<T> &P, T *ws_base, const WsLayout &L, bool need,
                                                long bound, const S &sv, NodeList<T> &nl, bool speculate, int &n_out,
                                                int *my_idx = nullptr)
@@ -1924,10 +1925,10 @@ __device__ __forceinline__ int trial_phase_cta(const DevParams<T> &P, T *ws_base
     // IGT_SPEC_BUDGET: most candidates (problems x halvings) evaluated at once; the default fills the CTA's threads
     int n_spec = 1;
     if (speculate) { n_spec = IGT_SPEC_BUDGET / n; n_spec = n_spec < 1 ? 1 : (n_spec > P.n_alpha ? P.n_alpha : n_spec); }
-    phase_items<T, 3, STRIDE, S::obca, false, S::bank>(ws_base, &nl, n, n_spec);
+    phase_items<T, 3, STRIDE, S::obca, false, S::bank, OWN>(ws_base, &nl, n, n_spec);
     __syncthreads();
     IGT_MID_TICK();
-    phase_items<T, 4, STRIDE, S::obca, RSTG, S::bank>(ws_base, &nl, n, n_spec);
+    phase_items<T, 4, STRIDE, S::obca, RSTG, S::bank, OWN>(ws_base, &nl, n, n_spec);
     __syncthreads();
     return n_spec;
 }
@@ -1936,8 +1937,9 @@ __device__ __forceinline__ int trial_phase_cta(const DevParams<T> &P, T *ws_base
 // line-search candidates of the CTA in one CTA-wide evaluation -- thread t takes candidate t / n of the
 // t % n-th listed problem -- left in Tc(candidate buffer, 2..7) for the owner's accept_trials.
 // COOP: the same with the exact cooperative evaluation (mlp_coop.cuh) instead of the tensor cores; COOP + BANK: each
-// candidate with its problem's network, the index read here from io (not held by the solver loop).
-template <typename T, bool COOP, bool BANK, typename WS>
+// candidate with its problem's network, the index read here from io (not held by the solver loop).  CAP: the request
+// capacity of the cooperative buffers (mlp_coop.cuh).
+template <typename T, bool COOP, bool BANK, int CAP = 0, typename WS>
 __device__ __forceinline__ void tc_candidates(const DevParams<T> &P, const ProbIO &io, T *ws_base, const WS &wproto,
                                               const NodeList<T> &nl, int n, int n_spec, MlpTcCtx *tc, uint8_t *coop_smem,
                                               int jlo = 0, bool filter = false)
@@ -1963,8 +1965,8 @@ __device__ __forceinline__ void tc_candidates(const DevParams<T> &P, const ProbI
         if (BANK) net = bank_io<T>(io).net_idx[p];
     }
     if (__syncthreads_or(valid)) {
-        if constexpr (COOP && BANK) mlp_coop_eval_bank(bank_io<T>(io).nets, coop_smem, valid, net, sN, vN, cx, o);
-        else if constexpr (COOP) mlp_coop_eval(P, coop_smem, valid, sN, vN, cx, o);
+        if constexpr (COOP && BANK) mlp_coop_eval_bank<T, CAP>(bank_io<T>(io).nets, coop_smem, valid, net, sN, vN, cx, o);
+        else if constexpr (COOP) mlp_coop_eval<T, CAP>(P, coop_smem, valid, sN, vN, cx, o);
         else mlp_tc_eval(*tc, valid, sN, vN, cx, o);
         if (valid) {
 #pragma unroll
@@ -1990,7 +1992,8 @@ __device__ int g_round_mx[512][4];       // per loop pass, max over CTA 0's thre
 #endif
 
 // BANK: gt_mpc with the handle's network bank, each problem with network io.net_idx[p] (per-thread or, with COOP,
-// cooperative value term; not with TC)
+// cooperative value term; not with TC).  STRIDE 1 is the latency kernel's single-problem workspace: one problem per CTA,
+// so a CTA-wide evaluation has at most n_alpha requests and the cooperative buffers are sized for COOP_CAP of them.
 template <typename T, bool TC, int STRIDE = 32, bool OBCA = false, bool COOP = false, bool RSTG = false, bool BANK = false>
 __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const ProbIO &io, T *ws_base,
                                                  long slot, long B, const Sched &sc,
@@ -2012,6 +2015,9 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
     const long bound = slot;
     if (TC) sv.phi_noise = T(3e-7);
     constexpr bool CTA_MLP = TC || COOP;                          // value term evaluated CTA-wide at the two uniform points below
+    constexpr int CAP = STRIDE == 1 ? COOP_CAP : 0;
+    constexpr bool OWN = COOP && STRIDE == 1;                     // (phase_items)
+    using SV = decltype(sv);
 #ifdef IGT_PHASE_CLOCKS
     const bool clk_on = blockIdx.x == 0 && threadIdx.x == 0;
     long long clk[16] = { 0 }, clk_t = clock64(), round_t = clk_t;
@@ -2053,8 +2059,8 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
             if (__syncthreads_or(want)) {
                 T o[6];
                 const T sN = want ? sv.w.Z(sv.cur, P.N, IS) : T(0), vN = want ? sv.w.Z(sv.cur, P.N, IV) : T(0);
-                if constexpr (BANK) mlp_coop_eval_bank(bank_io<T>(io).nets, coop_smem, want, want ? bank_io<T>(io).net_idx[p] : 0, sN, vN, sv.ctx, o);
-                else mlp_coop_eval(P, coop_smem, want, sN, vN, sv.ctx, o);
+                if constexpr (BANK) mlp_coop_eval_bank<T, CAP>(bank_io<T>(io).nets, coop_smem, want, want ? bank_io<T>(io).net_idx[p] : 0, sN, vN, sv.ctx, o);
+                else mlp_coop_eval<T, CAP>(P, coop_smem, want, sN, vN, sv.ctx, o);
                 if (want) { sv.tcur.V = o[0]; sv.tcur.gs = o[1]; sv.tcur.gv = o[2]; sv.tcur.Hss = o[3]; sv.tcur.Hsv = o[4]; sv.tcur.Hvv = o[5]; }
             }
         }
@@ -2076,7 +2082,7 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
         IGT_TICK(0);
         // ---- phase 1: backward pass = CTA-wide node phases between the per-problem sweeps ----
         const bool back = active && sv.need_back;
-        node_phase_cta<T, 1, STRIDE, RSTG>(P, ws_base, sv.w.L, back && sv.need_back == 2, bound, sv, nl);
+        node_phase_cta<T, 1, STRIDE, RSTG, SV, OWN>(P, ws_base, sv.w.L, back && sv.need_back == 2, bound, sv, nl);
         IGT_TICK(1);
 #ifdef IGT_PHASE_CLOCKS
         __shared__ int s_round_i;
@@ -2090,7 +2096,7 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
         if (blockIdx.x == 0 && back && rnd_ < 512) atomicMax(&g_round_mx[rnd_][0], (int)((clock64() - ta_) >> 10));
 #endif
         IGT_TICK(2);
-        node_phase_cta<T, 2, STRIDE, RSTG>(P, ws_base, sv.w.L, p2, bound, sv, nl);
+        node_phase_cta<T, 2, STRIDE, RSTG, SV, OWN>(P, ws_base, sv.w.L, p2, bound, sv, nl);
         IGT_TICK(3);
         if (back && !sv.done) {                                  // Riccati sweep, step bound
 #ifdef IGT_PHASE_CLOCKS
@@ -2121,7 +2127,7 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
         const bool trying = active && !sv.done;
         int n_try = 0;
         int my_idx = 0;                                          // this owner's position in the trial phase's list
-        const int n_spec = trial_phase_cta<T, STRIDE, RSTG>(P, ws_base, sv.w.L, trying, bound, sv, nl, true, n_try, &my_idx);
+        const int n_spec = trial_phase_cta<T, STRIDE, RSTG, SV, OWN>(P, ws_base, sv.w.L, trying, bound, sv, nl, true, n_try, &my_idx);
 #ifdef IGT_PHASE_CLOCKS
         if (clk_on) { long long m_ = g_mid_t; clk[7] += m_ - clk_t; if (round_i < 512) g_round_ph[round_i][7] += (int)((m_ - clk_t) >> 10); clk_t = m_; }
 #endif
@@ -2131,14 +2137,14 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
             // first, accepted nine times out of ten); the speculative candidates only of the problems whose first
             // was rejected.  Same candidates judged in the same order: same iterates.
             const int left = P.n_alpha - sv.ls, nj = n_spec < left ? n_spec : left;
-            tc_candidates<T, COOP, BANK>(P, io, ws_base, sv.w, nl, n_try, 1, tc, coop_smem);
+            tc_candidates<T, COOP, BANK, CAP>(P, io, ws_base, sv.w, nl, n_try, 1, tc, coop_smem);
             int tried = 0, jacc = -1;
             if (trying) jacc = sv.judge_trials(0, 1, true, tried);
             const bool more = trying && jacc < 0 && nj > 1;
             if (trying) nl.more[my_idx] = more ? 1 : 0;
             if (__syncthreads_or(more)) {
                 // candidates 1 .. n_spec-1: (n_spec - 1) n <= blockDim.x requests, one pass
-                tc_candidates<T, COOP, BANK>(P, io, ws_base, sv.w, nl, n_try, n_spec, tc, coop_smem, 1, true);
+                tc_candidates<T, COOP, BANK, CAP>(P, io, ws_base, sv.w, nl, n_try, n_spec, tc, coop_smem, 1, true);
                 if (more) jacc = sv.judge_trials(1, nj, true, tried);
             }
             if (trying) sv.finish_trials(jacc, tried);

@@ -247,8 +247,12 @@ int igt_mlp_value_ex_host(igt_handle *h, int B, const double *sN, const double *
  * tcgen05 kernel (csrc/mlp_tc.cuh; 6-128-128-1 networks, bf16x3 = fp32-accurate): measured no faster than the exact
  * path on a B200 (DESIGN.md section 4) and it perturbs the merit at 1e-7, so closed-loop outcomes can differ from the
  * fp64 oracle's; kept as an option.
- * "latency_path" (default 1): 'mpc'-mode batches of at most one problem per SM (a closed-loop step solves the two
- * vehicles of an episode) run one CTA per problem with the workspace in shared memory; 0 = throughput kernel. */
+ * "latency_path" (default 1): batches of at most one problem per SM (a closed-loop step solves the two vehicles of an
+ * episode) run one CTA per problem with the workspace in shared memory; 0 = throughput kernel.  'mpc' mode, and gt_mpc
+ * with one network or a bank (net_idx): exact cooperative value term in circle mode (fp64, layers <= 128 wide), per-thread
+ * value term in OBCA mode, in fp32 and for wider networks.  Not with the tensor-core value term (tensor_core_mlp = 1),
+ * and only while the kernel's shared memory fits a block: with the cooperative value term up to N = 45 (a bank: N = 44)
+ * at n_cinf = 74 on a B200; longer horizons take the throughput kernel.  Results are the same bits either way. */
 int igt_set_option(igt_handle *h, const char *name, double value);
 
 /* Measured throughput (TFLOP/s, FMA = 2 flops) of dependent-free FMA chains in `precision` on
