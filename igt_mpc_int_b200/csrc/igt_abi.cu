@@ -15,6 +15,8 @@
 #include <vector>
 #include <new>
 #include <mutex>
+#include <atomic>
+#include <algorithm>
 
 #include "../../include/igt_mpc.h"
 #include "solver_core.cuh"
@@ -344,27 +346,22 @@ struct igt_handle {
     igt_params prm;
     DevParams<float> Pf;
     DevParams<double> Pd;
-    bool has_mlp = false;
     MlpTcWeights tc = {};              // tensor-core copy of the value network (6-128-128-1 only)
     int use_tc = 0;                    // igt_set_option("tensor_core_mlp", 1): fp32-accurate tcgen05 value term (6-128-128-1 nets)
-    bool coop_ok = false;              // every layer <= MLP_COOP_W wide: the exact CTA-cooperative evaluation applies
     int use_small = 1;                 // igt_set_option("latency_path", 0) keeps small batches on the throughput kernel
-    int mlp_width = 0;
-    // network bank (igt_set_mlp_at): slot 0 is also the network above (Pf / Pd, tc); a solve with net_idx reads the
-    // device table `bank` = [MAX_MLP_NETS] MlpNet<double>, then [MAX_MLP_NETS] MlpNet<float>
-    std::vector<void *> mlp_bufs[MAX_MLP_NETS];   // device weight buffers of each slot (both precisions)
+    // network bank (igt_set_mlp_at): slot 0 is also the network of the calls without net_idx (Pf / Pd, tc); a solve
+    // with net_idx reads the device table `bank` = [MAX_MLP_NETS] MlpNet<double>, then [MAX_MLP_NETS] MlpNet<float>
+    void *mlp_buf[MAX_MLP_NETS] = {};  // device image of each slot: its weights in both precisions (+ the tensor-core copy)
     MlpNet<double> netd[MAX_MLP_NETS] = {};
     MlpNet<float> netf[MAX_MLP_NETS] = {};
     int net_width[MAX_MLP_NETS] = {};  // widest layer of each slot, 0 = empty
     void *bank = nullptr;
     void *ws = nullptr; size_t ws_bytes = 0;
     void *mlp_scratch = nullptr; size_t mlp_scratch_bytes = 0;
-    void *stage = nullptr; size_t stage_bytes = 0;     // device staging for *_host calls
+    void *stage = nullptr; size_t stage_bytes = 0;     // device block of the *_host calls (see staged)
     void *guess = nullptr; size_t guess_bytes = 0;     // cold-start controls [B][N][2] + the work counter
-    void *episode = nullptr; size_t episode_bytes = 0; // igt_episode_run_host: state, records, solver inputs / outputs
     int n_sm = 0;
     int smem_optin = 0;                // shared memory a block may opt in to (the gt_mpc latency path's limit)
-    int small_static[8] = { -1, -1, -1, -1, -1, -1, -1, -1 };   // static shared memory of each k_small_gt kernel, -1: not read yet
     long long launches = 0;
     std::string err;
     int device = 0;
@@ -372,7 +369,7 @@ struct igt_handle {
     // streams -- the handle's workspace, guess buffer and work counter are shared by its calls
     std::mutex mu;                     // host-side: one call at a time per handle
     cudaStream_t hstream = nullptr;    // the *_host entry points run on a private non-blocking stream
-    void *pin = nullptr; size_t pin_bytes = 0;   // pinned staging block of igt_solve_host (small batches)
+    void *pin = nullptr; size_t pin_bytes = 0;   // pinned staging block of the *_host calls (small batches)
     cudaEvent_t last_use = nullptr;    // recorded after the last kernel of every call
     cudaStream_t last_stream = nullptr;
     bool used = false;
@@ -461,41 +458,268 @@ static int end_call(igt_handle *h, cudaStream_t st, int prec_used_mask)
     return IGT_OK;
 }
 
-// The gt_mpc instantiations of the latency kernel, by small_gt_variant: cooperative value term (circle mode, f64, every
-// layer <= MLP_COOP_W), then per-thread in f64 circle mode, OBCA and f32; each with one network and with the bank.
-static const void *const k_small_gt[8] = {
-    (const void *)solve_small_kernel<double, false, true, false>, (const void *)solve_small_kernel<double, false, true, true>,
-    (const void *)solve_small_kernel<double, false, false, false, true>, (const void *)solve_small_kernel<double, false, false, true>,
-    (const void *)solve_small_kernel<double, true, false, false, true>, (const void *)solve_small_kernel<double, true, false, true>,
-    (const void *)solve_small_kernel<float, false, false, false, true>, (const void *)solve_small_kernel<float, false, false, true>,
-};
-static int small_gt_variant(bool coop, bool bank, bool obca, bool f64) { return (coop ? 0 : obca ? 4 : f64 ? 2 : 6) + (bank ? 1 : 0); }
-
-// whether gt_mpc variant v fits one block's shared memory with `dyn` bytes of workspace and value-term buffers: the
-// kernel's static shared memory is read once per handle
-static int small_gt_fits(igt_handle *h, int v, size_t dyn, bool *fits)
+// Prologue of every *_host call: one call at a time per handle; the arguments are checked under the lock (bank
+// indices are read against the loaded slots, which igt_set_mlp_at changes under it) before anything is allocated or
+// copied; then `run` queues its work on the handle's private non-blocking stream.
+template <typename Check, typename Run>
+static int host_call(igt_handle *h, int B, Check &&check, Run &&run)
 {
-    if (h->small_static[v] < 0) {
-        cudaFuncAttributes a;
-        CK(cudaFuncGetAttributes(&a, k_small_gt[v]));
-        h->small_static[v] = (int)a.sharedSizeBytes;
+    if (!h) return IGT_EINVAL;
+    std::lock_guard<std::mutex> lk(h->mu);
+    int rc = check();
+    if (rc || B == 0) return rc;
+    CK(cudaSetDevice(h->device));
+    if (!h->hstream) CK(cudaStreamCreateWithFlags(&h->hstream, cudaStreamNonBlocking));
+    rc = begin_call(h, h->hstream);
+    return rc ? rc : run(h->hstream);
+}
+
+// One array of a *_host call: copied in from host memory, copied out to it, or on the device only.  An absent
+// (null) host array takes no bytes and gets a null device address.
+struct Staged { const void *in; void *out; size_t bytes; void **dev; };
+template <typename T, typename D> static Staged input(const T *p, size_t n, D **d) { return { p, nullptr, p ? n * sizeof(T) : 0, (void **)d }; }
+template <typename T> static Staged output(T *p, size_t n, T **d) { return { nullptr, p, p ? n * sizeof(T) : 0, (void **)d }; }
+template <typename T> static Staged device_only(size_t n, T **d) { return { nullptr, nullptr, n * sizeof(T), (void **)d }; }
+
+// Lays the arrays out in h->stage -- inputs, outputs, device-only arrays, each at a 256-byte boundary -- copies the
+// inputs in, calls `run` (which queues the call's kernels on `st`), copies the outputs back and synchronises.
+// Inputs and outputs of at most 1 MiB together (the closed-loop step: B = 2) travel in ONE copy each way through the
+// pinned block h->pin; larger ones are copied array by array straight from / to the caller's (ideally pinned)
+// memory -- packing 100 MB on the host would cost more than the copies.
+template <size_t n, typename Run>
+static int staged(igt_handle *h, cudaStream_t st, Staged (&a)[n], Run &&run)
+{
+    size_t off[n], top = 0, end[3];
+    for (int kind = 0; kind < 3; kind++) {
+        for (size_t i = 0; i < n; i++)
+            if ((a[i].in ? 0 : a[i].out ? 1 : 2) == kind) { off[i] = top; top += (a[i].bytes + 255) & ~(size_t)255; }
+        end[kind] = top;
     }
-    *fits = dyn + (size_t)h->small_static[v] <= (size_t)h->smem_optin;
+    int rc = grow(h, &h->stage, &h->stage_bytes, top, st);
+    if (rc) return rc;
+    char *d = (char *)h->stage, *pin = nullptr;
+    for (size_t i = 0; i < n; i++) *a[i].dev = a[i].bytes ? d + off[i] : nullptr;
+    if (end[1] <= (size_t)1 << 20) {
+        if (h->pin_bytes < end[1]) {
+            if (h->pin) { CK(cudaStreamSynchronize(st)); CK(cudaFreeHost(h->pin)); h->pin = nullptr; h->pin_bytes = 0; }
+            CK(cudaHostAlloc(&h->pin, end[1], cudaHostAllocDefault));
+            h->pin_bytes = end[1];
+        }
+        pin = (char *)h->pin;
+        for (size_t i = 0; i < n; i++) if (a[i].in && a[i].bytes) memcpy(pin + off[i], a[i].in, a[i].bytes);
+        if (end[0]) CK(cudaMemcpyAsync(d, pin, end[0], cudaMemcpyHostToDevice, st));
+    } else {
+        for (size_t i = 0; i < n; i++)
+            if (a[i].in && a[i].bytes) CK(cudaMemcpyAsync(d + off[i], a[i].in, a[i].bytes, cudaMemcpyHostToDevice, st));
+    }
+    if ((rc = run())) return rc;
+    if (pin) {
+        if (end[1] > end[0]) CK(cudaMemcpyAsync(pin + end[0], d + end[0], end[1] - end[0], cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        for (size_t i = 0; i < n; i++) if (a[i].out && a[i].bytes) memcpy(a[i].out, pin + off[i], a[i].bytes);
+    } else {
+        for (size_t i = 0; i < n; i++)
+            if (a[i].out && a[i].bytes) CK(cudaMemcpyAsync(a[i].out, d + off[i], a[i].bytes, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
     return IGT_OK;
 }
 
-template <typename T, bool OBCA, bool COOP, bool BANK>
-static int launch_small_gt(igt_handle *h, const ProbIONet<T> &iob, int B, Sched sc, const double *guess, T *scratch, int width,
-                           size_t smem, int cs, cudaStream_t st)
+// ------------------------------------------------------------------ solver variants -----
+// The solver configurations the library is built with, one row each.  A row names its throughput kernel
+// solve_kernel<T, TC, OBCA, COOP, BANK>, its cold-start kernel guess_kernel<T, OBCA> and, without TC, its latency
+// kernel solve_small_kernel<T, OBCA, COOP, BANK, GT>: these rows are the only instantiations of the three templates.
+// TC: tensor-core value term; COOP: the CTA-cooperative exact value term (f64, circle mode, every layer <= MLP_COOP_W);
+// BANK: network net_idx[p] of the handle's bank per problem; GT: gt_mpc (a value term at all).
+template <typename T_, bool OBCA_, bool TC_, bool COOP_, bool BANK_, bool GT_>
+struct Variant {
+    using T = T_;
+    static constexpr bool OBCA = OBCA_, TC = TC_, COOP = COOP_, BANK = BANK_, GT = GT_;
+};
+template <typename... V> struct VariantList {};
+using Variants = VariantList<
+    //      T       OBCA   TC     COOP   BANK   GT
+    Variant<double, false, false, false, false, false>,     // 'mpc'
+    Variant<float,  false, false, false, false, false>,
+    Variant<double, true,  false, false, false, false>,
+    Variant<double, false, false, true,  false, true>,      // gt_mpc, one network
+    Variant<double, false, true,  false, false, true>,
+    Variant<float,  false, true,  false, false, true>,
+    Variant<double, false, false, false, false, true>,
+    Variant<double, true,  false, false, false, true>,
+    Variant<float,  false, false, false, false, true>,
+    Variant<double, false, false, true,  true,  true>,      // gt_mpc, network bank
+    Variant<double, false, false, false, true,  true>,
+    Variant<double, true,  false, false, true,  true>,
+    Variant<float,  false, false, false, true,  true>>;
+
+// f(V()) for the row V with these flags (solve_dev_impl only asks for combinations that have a row)
+template <typename F, typename... V>
+static int with_variant(igt_handle *h, VariantList<V...>, bool f64, bool obca, bool tc, bool coop, bool bank, bool gt, F &&f)
 {
-    using IO = typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type;
-    SmallIO<IO, T> io;
-    static_cast<IO &>(io) = iob;
-    io.mlp_scratch = COOP ? nullptr : scratch;
-    io.mlp_width = width;
-    CK(cudaFuncSetAttribute(solve_small_kernel<T, OBCA, COOP, BANK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    solve_small_kernel<T, OBCA, COOP, BANK, true><<<B, SOLVE_BLOCK, smem, st>>>(io, B, sc, guess, cs);
+    int rc = IGT_OK;
+    const bool hit = ((std::is_same<typename V::T, double>::value == f64 && V::OBCA == obca && V::TC == tc && V::COOP == coop &&
+                       V::BANK == bank && V::GT == gt && (rc = f(V()), true)) || ...);
+    if (!hit) { h->err = "igt_solve: no solver variant for this combination"; return IGT_EINVAL; }
+    return rc;
+}
+
+// Widest network the value term of a call may meet: slot 0's, or the widest of the bank (0: nothing loaded).  It sizes
+// the per-thread scratch, and the cooperative evaluation applies when it is <= MLP_COOP_W.
+static int value_width(const igt_handle *h, bool bank)
+{
+    int w = h->net_width[0];
+    if (bank) for (int k = 1; k < MAX_MLP_NETS; k++) if (h->net_width[k] > w) w = h->net_width[k];
+    return w;
+}
+
+// Bank calls: every index names a loaded slot (checked on the host before anything is launched, under h->mu, so that
+// a concurrent igt_set_mlp_at cannot empty a slot between the check and the launch).
+static int check_net_idx(igt_handle *h, int n, const int *net_idx, const char *who)
+{
+    for (int i = 0; i < n; i++) {
+        const int k = net_idx[i];
+        if (k < 0 || k >= IGT_MAX_MLP_NETS || h->net_width[k] == 0) {
+            h->err = std::string(who) + ": net_idx[" + std::to_string(i) + "] = " + std::to_string(k) + " names no loaded network";
+            return IGT_EINVAL;
+        }
+    }
     return IGT_OK;
+}
+
+// arguments of igt_solve_ex_dev / igt_solve_ex_host (host_idx: net_idx is in host memory and is checked here; a device
+// index is checked in the kernel: IGT_STATUS_BAD_NET)
+static int check_solve(igt_handle *h, int B, const ProbIO &io, const int *net_idx, bool host_idx)
+{
+    if (B < 0 || !io.x0 || !io.u_prev || !io.curv || !io.obs || !io.x || !io.u || !io.cost || !io.viol || !io.status || !io.iters) {
+        h->err = "igt_solve: null argument"; return IGT_EINVAL;
+    }
+    if (net_idx && !io.ctx) { h->err = "igt_solve: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
+    if (net_idx && host_idx) { const int rc = check_net_idx(h, B, net_idx, "igt_solve"); if (rc) return rc; }
+    if (io.ctx && value_width(h, net_idx != nullptr) == 0) {
+        h->err = net_idx ? "igt_solve: net_idx given but no network was loaded" : "igt_solve: nn_ctx given but igt_set_mlp was never called";
+        return IGT_ENOMLP;
+    }
+    if (io.obs_psi && h->prm.precision != IGT_PREC_F64) { h->err = "igt_solve: the OBCA collision rows (obs_psi) need precision f64"; return IGT_EINVAL; }
+    return IGT_OK;
+}
+
+// io as the kernels of a row with BANK take it: with the bank's descriptor table in T (the f32 one follows the f64 one)
+template <typename T, bool BANK>
+static typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type io_for(const ProbIO &io, const int *net_idx, const igt_handle *h)
+{
+    typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type r;
+    static_cast<ProbIO &>(r) = io;
+    if constexpr (BANK) {
+        r.net_idx = net_idx;
+        r.nets = (const MlpNet<T> *)((const char *)h->bank + (sizeof(T) == 8 ? 0 : sizeof(h->netd)));
+    }
+    return r;
+}
+
+// Solve of checked arguments (device pointers) on `st`.
+static int solve_dev_impl(igt_handle *h, int B, const ProbIO &io, const int *net_idx, cudaStream_t st)
+{
+    if (B == 0) return IGT_OK;
+    int rc = begin_call(h, st);
+    if (rc) return rc;
+    const bool f64 = h->prm.precision == IGT_PREC_F64, obca = io.obs_psi != nullptr, gt = io.ctx != nullptr, bank = net_idx != nullptr;
+    WsLayout L; L.init(h->prm.N, h->prm.n_cinf, obca ? NGE_OBCA : NGE, obca ? NHE_OBCA : NHE);
+    // value term (OBCA + gt_mpc: per-thread value term; a bank: exact evaluation whatever tensor_core_mlp says)
+    const int width = value_width(h, bank);
+    const bool use_tc = gt && !bank && h->tc.enabled && h->use_tc && !obca;
+    const bool use_coop = gt && !use_tc && f64 && width <= MLP_COOP_W && !obca;
+    // persistent lanes: one CTA of SOLVE_BLOCK threads per SM.  A batch smaller than the machine is spread
+    // over all SMs, a whole number of warps each: `quota` threads per CTA fetch problems, the rest of
+    // the CTA only helps in the CTA-wide phases (and adopts stragglers in the tail).
+    const int bs = SOLVE_BLOCK;
+    long n_cta = ((long)B + 31) / 32;
+    if (n_cta > h->n_sm) n_cta = h->n_sm;
+    long per_cta = ((long)B + n_cta - 1) / n_cta;
+    int quota = (int)((per_cta + 31) / 32 * 32);
+    if (quota > bs) quota = bs;
+    const long n_slots = n_cta * bs;
+    return with_variant(h, Variants(), f64, obca, use_tc, use_coop, bank, gt, [&](auto v) -> int {
+        using V = decltype(v);
+        using T = typename V::T;
+        // latency path: at most one problem per SM and a workspace that fits shared memory next to the work lists; in
+        // gt_mpc (not with the tensor-core value term) the kernel's whole shared memory -- static, value-term buffers,
+        // workspace -- within the device's opt-in limit per block
+        const size_t small_smem = (size_t)L.total * sizeof(T) + small_coop_bytes<T, V::COOP, V::BANK>();
+        bool small = false;
+        if constexpr (!V::TC) {
+            if (h->use_small && B <= h->n_sm) {
+                if constexpr (V::GT) {
+                    static std::atomic<int> static_smem{ -1 };   // the latency kernel's static shared memory, read once
+                    if (static_smem < 0) {
+                        cudaFuncAttributes fa;
+                        CK(cudaFuncGetAttributes(&fa, solve_small_kernel<T, V::OBCA, V::COOP, V::BANK, V::GT>));
+                        static_smem = (int)fa.sharedSizeBytes;
+                    }
+                    small = small_smem + (size_t)static_smem <= (size_t)h->smem_optin;
+                } else {
+                    small = small_smem <= 200 * 1024;
+                }
+            }
+        }
+        int rc = small ? IGT_OK : grow(h, &h->ws, &h->ws_bytes, (size_t)L.total * n_slots * sizeof(T), st);
+        if (rc) return rc;
+        constexpr bool per_thread = V::GT && !V::TC && !V::COOP;      // per-thread value term: activations in HBM
+        if (per_thread) {                                                // (one slab per persistent lane, or per CTA on the latency path)
+            rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * (small ? B : n_slots) * sizeof(T), st);
+            if (rc) return rc;
+        }
+        T *scratch = per_thread ? (T *)h->mlp_scratch : nullptr;
+        // scheduler block (the work counter), then the cold-start guesses
+        const size_t off_guess = 256;
+        rc = grow(h, &h->guess, &h->guess_bytes, off_guess + (size_t)B * h->prm.N * 2 * sizeof(double), st);
+        if (rc) return rc;
+        char *sb = (char *)h->guess;
+        Sched sc;
+        sc.counter = (unsigned long long *)sb;
+        double *guess = (double *)(sb + off_guess);
+        int cs = 0;
+        rc = acquire_cslot(h, f64 ? 1 : 0, st, &cs);
+        if (rc) return rc;
+        CK(cudaMemsetAsync(sb, 0, 256, st));
+        if (!io.u_init || io.warm) {
+            guess_kernel<T, V::OBCA><<<(B + 127) / 128, 128, 0, st>>>(io, B, guess, cs);
+            h->launches++;
+        }
+        using IO = typename std::conditional<V::BANK, ProbIONet<T>, ProbIO>::type;
+        const IO iob = io_for<T, V::BANK>(io, net_idx, h);   // (a bank problem with a bad index gets IGT_STATUS_BAD_NET)
+        if constexpr (!V::TC) {
+            if (small) {
+                typename std::conditional<V::GT, SmallIO<IO, T>, IO>::type ios;
+                static_cast<IO &>(ios) = iob;
+                if constexpr (V::GT) { ios.mlp_scratch = scratch; ios.mlp_width = width; }
+                auto *k = solve_small_kernel<T, V::OBCA, V::COOP, V::BANK, V::GT>;
+                CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
+                k<<<B, bs, small_smem, st>>>(ios, B, sc, guess, cs);
+            }
+        }
+        if (!small) {
+            const int smem = V::TC ? TC_SMEM_BYTES
+                           : V::COOP ? (V::BANK ? mlp_coop_bank_smem_bytes<T>(SOLVE_BLOCK) : mlp_coop_smem_bytes<T>(SOLVE_BLOCK))
+                           : IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * (int)sizeof(T) : 0;
+            auto *k = solve_kernel<T, V::TC, V::OBCA, V::COOP, V::BANK>;
+            CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            k<<<(int)(n_slots / bs), bs, smem, st>>>(iob, (T *)h->ws, n_slots, B, sc, guess, scratch, width, h->tc, quota, cs);
+        }
+        h->launches++;
+        CK(cudaGetLastError());
+        return end_call(h, st, f64 ? 2 : 1);
+    });
+}
+
+// slot 0's network in the solver parameters (constant memory) of the single-network calls
+template <typename T>
+static void set_param_net(DevParams<T> &P, const MlpNet<T> &n)
+{
+    P.n_layers = n.n_layers;
+    memcpy(P.dims, n.dims, sizeof(P.dims)); memcpy(P.Wn, n.Wn, sizeof(P.Wn)); memcpy(P.mu_f, n.mu_f, sizeof(P.mu_f));
+    P.sigma_t = n.sigma_t; P.mu_t = n.mu_t;
+    memcpy(P.W, n.W, sizeof(P.W)); memcpy(P.b, n.b, sizeof(P.b)); memcpy(P.Wt, n.Wt, sizeof(P.Wt));
 }
 
 extern "C" {
@@ -543,7 +767,7 @@ void igt_destroy(igt_handle *h)
             for (int i = 0; i < N_CSLOTS; i++)
                 if (g_slots[dev][prec][i].owner == h) { g_slots[dev][prec][i].owner = nullptr; g_slots[dev][prec][i].version = 0; }
     }
-    for (auto &v : h->mlp_bufs) for (void *b : v) cudaFree(b);
+    for (void *b : h->mlp_buf) if (b) cudaFree(b);
     if (h->bank) cudaFree(h->bank);
     if (h->hstream) cudaStreamDestroy(h->hstream);
     if (h->pin) cudaFreeHost(h->pin);
@@ -551,7 +775,6 @@ void igt_destroy(igt_handle *h)
     if (h->mlp_scratch) cudaFree(h->mlp_scratch);
     if (h->stage) cudaFree(h->stage);
     if (h->guess) cudaFree(h->guess);
-    if (h->episode) cudaFree(h->episode);
     delete h;
 }
 
@@ -569,70 +792,32 @@ int igt_set_mlp_at(igt_handle *h, int net, int n_layers, const int *dims, const 
     int width = 6;
     for (int l = 0; l <= n_layers; l++) { if (dims[l] < 1 || dims[l] > 1024) { h->err = "igt_set_mlp: bad width"; return IGT_EINVAL; } if (dims[l] > width) width = dims[l]; }
     for (int l = 0; l < n_layers; l++) if (!W[l] || !b[l]) { h->err = "igt_set_mlp: null layer"; return IGT_EINVAL; }
-    std::lock_guard<std::mutex> lk(h->mu);
-    CK(cudaSetDevice(h->device));
-    if (h->last_use && h->used) CK(cudaEventSynchronize(h->last_use));   // no kernel of this handle reads the old network
-    if (!h->bank) CK(cudaMalloc(&h->bank, MAX_MLP_NETS * (sizeof(MlpNet<double>) + sizeof(MlpNet<float>))));
-    h->version[0]++; h->version[1]++;
-    for (void *q : h->mlp_bufs[net]) cudaFree(q);
-    h->mlp_bufs[net].clear();
-    h->net_width[net] = 0;
-    MlpNet<double> &nd = h->netd[net];
-    MlpNet<float> &nf = h->netf[net];
-    nd = MlpNet<double>(); nf = MlpNet<float>();
-    std::vector<void *> &bufs = h->mlp_bufs[net];
-    nf.n_layers = nd.n_layers = n_layers;
-    for (int l = 0; l <= n_layers; l++) nf.dims[l] = nd.dims[l] = dims[l];
+    // the slot's device image, built here and uploaded in one copy: per layer W, b in f64 and f32 and the transposed
+    // copies [in][out] for the cooperative evaluation (mlp_coop.cuh); for slot 0 of shape 6-128-128-1 also the
+    // tensor-core copy.  Every array starts at a 256-byte boundary, as a cudaMalloc of its own would.
+    std::vector<uint8_t> img;
+    auto put = [&img](const void *src, size_t bytes) {
+        const size_t o = img.size();
+        img.resize((o + bytes + 255) & ~(size_t)255);
+        memcpy(img.data() + o, src, bytes);
+        return o;
+    };
+    size_t o_net[IGT_MAX_MLP_LAYERS][6];
     for (int l = 0; l < n_layers; l++) {
-        size_t nw = (size_t)dims[l] * dims[l + 1], nb = dims[l + 1];
+        const size_t nw = (size_t)dims[l] * dims[l + 1], nb = dims[l + 1];
         std::vector<float> wf(nw), bf(nb);
         for (size_t i = 0; i < nw; i++) wf[i] = (float)W[l][i];
         for (size_t i = 0; i < nb; i++) bf[i] = (float)b[l][i];
-        void *dWd, *dbd, *dWf, *dbf;
-        CK(cudaMalloc(&dWd, nw * 8)); bufs.push_back(dWd);
-        CK(cudaMalloc(&dbd, nb * 8)); bufs.push_back(dbd);
-        CK(cudaMalloc(&dWf, nw * 4)); bufs.push_back(dWf);
-        CK(cudaMalloc(&dbf, nb * 4)); bufs.push_back(dbf);
-        CK(cudaMemcpy(dWd, W[l], nw * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dbd, b[l], nb * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dWf, wf.data(), nw * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dbf, bf.data(), nb * 4, cudaMemcpyHostToDevice));
-        nd.W[l] = (const double *)dWd; nd.b[l] = (const double *)dbd;
-        nf.W[l] = (const float *)dWf; nf.b[l] = (const float *)dbf;
-        // transposed copies [in][out] for the cooperative evaluation (mlp_coop.cuh)
         std::vector<double> wtd(nw); std::vector<float> wtf(nw);
         for (int o = 0; o < dims[l + 1]; o++)
             for (int i = 0; i < dims[l]; i++) { wtd[(size_t)i * dims[l + 1] + o] = W[l][(size_t)o * dims[l] + i]; wtf[(size_t)i * dims[l + 1] + o] = (float)W[l][(size_t)o * dims[l] + i]; }
-        void *dTd, *dTf;
-        CK(cudaMalloc(&dTd, nw * 8)); bufs.push_back(dTd);
-        CK(cudaMalloc(&dTf, nw * 4)); bufs.push_back(dTf);
-        CK(cudaMemcpy(dTd, wtd.data(), nw * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dTf, wtf.data(), nw * 4, cudaMemcpyHostToDevice));
-        nd.Wt[l] = (const double *)dTd; nf.Wt[l] = (const float *)dTf;
+        o_net[l][0] = put(W[l], nw * 8); o_net[l][1] = put(b[l], nb * 8);
+        o_net[l][2] = put(wf.data(), nw * 4); o_net[l][3] = put(bf.data(), nb * 4);
+        o_net[l][4] = put(wtd.data(), nw * 8); o_net[l][5] = put(wtf.data(), nw * 4);
     }
-    for (int i = 0; i < 36; i++) { nd.Wn[i] = Wn[i]; nf.Wn[i] = (float)Wn[i]; }
-    for (int i = 0; i < 6; i++) { nd.mu_f[i] = mu_f[i]; nf.mu_f[i] = (float)mu_f[i]; }
-    nd.sigma_t = sigma_t; nd.mu_t = mu_t; nf.sigma_t = (float)sigma_t; nf.mu_t = (float)mu_t;
-    h->net_width[net] = width;
-    // the whole descriptor table (empty slots: n_layers = 0); bank launches pass it to the kernels (ProbIONet::nets)
-    CK(cudaMemcpy(h->bank, h->netd, sizeof(h->netd), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy((char *)h->bank + sizeof(h->netd), h->netf, sizeof(h->netf), cudaMemcpyHostToDevice));
-    if (net != 0) return IGT_OK;
-    // slot 0 is the handle's network of the single-network calls: in DevParams (constant memory) and the tcgen05 copy
-    h->mlp_width = width;
-    h->Pf.n_layers = h->Pd.n_layers = n_layers;
-    for (int l = 0; l <= n_layers; l++) h->Pf.dims[l] = h->Pd.dims[l] = dims[l];
-    for (int l = 0; l < n_layers; l++) {
-        h->Pd.W[l] = nd.W[l]; h->Pd.b[l] = nd.b[l]; h->Pd.Wt[l] = nd.Wt[l];
-        h->Pf.W[l] = nf.W[l]; h->Pf.b[l] = nf.b[l]; h->Pf.Wt[l] = nf.Wt[l];
-    }
-    h->coop_ok = width <= MLP_COOP_W;
-    for (int i = 0; i < 36; i++) { h->Pd.Wn[i] = Wn[i]; h->Pf.Wn[i] = (float)Wn[i]; }
-    for (int i = 0; i < 6; i++) { h->Pd.mu_f[i] = mu_f[i]; h->Pf.mu_f[i] = (float)mu_f[i]; }
-    h->Pd.sigma_t = sigma_t; h->Pd.mu_t = mu_t; h->Pf.sigma_t = (float)sigma_t; h->Pf.mu_t = (float)mu_t;
-    h->has_mlp = true;
-    h->tc.enabled = 0;
-    if (n_layers == 3 && dims[1] == MLP_H && dims[2] == MLP_H) {
+    const bool tc = net == 0 && n_layers == 3 && dims[1] == MLP_H && dims[2] == MLP_H;
+    size_t o_tc[5] = {};
+    if (tc) {
         // tensor-core copy: W1eff = W1 Wn, b1eff = b1 - W1eff mu_f (fp32), W2 as bf16 hi/mid/lo in UMMA core-matrix order
         std::vector<float> w1eff(MLP_H * 6), b1eff(MLP_H), b2(MLP_H), w3(MLP_H);
         for (int o = 0; o < MLP_H; o++) {
@@ -656,19 +841,44 @@ int igt_set_mlp_at(igt_handle *h, int net, int n_layers, const int *dims, const 
                 int off = tc_elem_offset(n, k);
                 memcpy(&blob[off], &hi, 2); memcpy(&blob[TC_TILE_BYTES + off], &mid, 2); memcpy(&blob[2 * TC_TILE_BYTES + off], &lo, 2);
             }
-        void *dblob, *dw1, *db1, *db2, *dw3;
-        CK(cudaMalloc(&dblob, blob.size())); bufs.push_back(dblob);
-        CK(cudaMalloc(&dw1, w1eff.size() * 4)); bufs.push_back(dw1);
-        CK(cudaMalloc(&db1, MLP_H * 4)); bufs.push_back(db1);
-        CK(cudaMalloc(&db2, MLP_H * 4)); bufs.push_back(db2);
-        CK(cudaMalloc(&dw3, MLP_H * 4)); bufs.push_back(dw3);
-        CK(cudaMemcpy(dblob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dw1, w1eff.data(), w1eff.size() * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(db1, b1eff.data(), MLP_H * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(db2, b2.data(), MLP_H * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(dw3, w3.data(), MLP_H * 4, cudaMemcpyHostToDevice));
-        h->tc.w2_splits = (const uint8_t *)dblob; h->tc.w1eff = (const float *)dw1; h->tc.b1eff = (const float *)db1;
-        h->tc.b2 = (const float *)db2; h->tc.w3 = (const float *)dw3;
+        o_tc[0] = put(blob.data(), blob.size()); o_tc[1] = put(w1eff.data(), w1eff.size() * 4);
+        o_tc[2] = put(b1eff.data(), MLP_H * 4); o_tc[3] = put(b2.data(), MLP_H * 4); o_tc[4] = put(w3.data(), MLP_H * 4);
+    }
+    std::lock_guard<std::mutex> lk(h->mu);
+    CK(cudaSetDevice(h->device));
+    if (h->last_use && h->used) CK(cudaEventSynchronize(h->last_use));   // no kernel of this handle reads the old network
+    if (!h->bank) CK(cudaMalloc(&h->bank, MAX_MLP_NETS * (sizeof(MlpNet<double>) + sizeof(MlpNet<float>))));
+    h->version[0]++; h->version[1]++;
+    if (h->mlp_buf[net]) { cudaFree(h->mlp_buf[net]); h->mlp_buf[net] = nullptr; }
+    h->net_width[net] = 0;
+    if (net == 0) h->tc.enabled = 0;
+    MlpNet<double> &nd = h->netd[net];
+    MlpNet<float> &nf = h->netf[net];
+    nd = MlpNet<double>(); nf = MlpNet<float>();
+    CK(cudaMalloc(&h->mlp_buf[net], img.size()));
+    CK(cudaMemcpy(h->mlp_buf[net], img.data(), img.size(), cudaMemcpyHostToDevice));
+    const uint8_t *base = (const uint8_t *)h->mlp_buf[net];
+    nf.n_layers = nd.n_layers = n_layers;
+    for (int l = 0; l <= n_layers; l++) nf.dims[l] = nd.dims[l] = dims[l];
+    for (int l = 0; l < n_layers; l++) {
+        nd.W[l] = (const double *)(base + o_net[l][0]); nd.b[l] = (const double *)(base + o_net[l][1]);
+        nf.W[l] = (const float *)(base + o_net[l][2]); nf.b[l] = (const float *)(base + o_net[l][3]);
+        nd.Wt[l] = (const double *)(base + o_net[l][4]); nf.Wt[l] = (const float *)(base + o_net[l][5]);
+    }
+    for (int i = 0; i < 36; i++) { nd.Wn[i] = Wn[i]; nf.Wn[i] = (float)Wn[i]; }
+    for (int i = 0; i < 6; i++) { nd.mu_f[i] = mu_f[i]; nf.mu_f[i] = (float)mu_f[i]; }
+    nd.sigma_t = sigma_t; nd.mu_t = mu_t; nf.sigma_t = (float)sigma_t; nf.mu_t = (float)mu_t;
+    h->net_width[net] = width;
+    // the whole descriptor table (empty slots: n_layers = 0); bank launches pass it to the kernels (ProbIONet::nets)
+    CK(cudaMemcpy(h->bank, h->netd, sizeof(h->netd), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy((char *)h->bank + sizeof(h->netd), h->netf, sizeof(h->netf), cudaMemcpyHostToDevice));
+    if (net != 0) return IGT_OK;
+    // slot 0 is the handle's network of the single-network calls: in DevParams (constant memory) and the tcgen05 copy
+    set_param_net(h->Pd, nd);
+    set_param_net(h->Pf, nf);
+    if (tc) {
+        h->tc.w2_splits = base + o_tc[0]; h->tc.w1eff = (const float *)(base + o_tc[1]); h->tc.b1eff = (const float *)(base + o_tc[2]);
+        h->tc.b2 = (const float *)(base + o_tc[3]); h->tc.w3 = (const float *)(base + o_tc[4]);
         h->tc.b3 = (float)b[2][0]; h->tc.sigma_t = (float)sigma_t; h->tc.mu_t = (float)mu_t;
         h->tc.enabled = 1;
         CK(cudaFuncSetAttribute(mlp_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
@@ -682,41 +892,17 @@ int igt_set_mlp(igt_handle *h, int n_layers, const int *dims, const double *cons
     return igt_set_mlp_at(h, 0, n_layers, dims, W, b, Wn, mu_f, sigma_t, mu_t);
 }
 
-// Bank calls: every index names a loaded slot (checked on the host before anything is launched, under h->mu, so that
-// a concurrent igt_set_mlp_at cannot empty a slot between the check and the launch); the widest network
-// of the bank sizes the per-thread scratch, and the cooperative evaluation applies when every slot is <= 128 wide.
-static int check_net_idx(igt_handle *h, int n, const int *net_idx, const char *who)
+static int check_rollout(igt_handle *h, int B, const float *z0, const float *u, const float *curv, const float *z,
+                         const float *A, const float *Bm, int model)
 {
-    for (int i = 0; i < n; i++) {
-        const int k = net_idx[i];
-        if (k < 0 || k >= IGT_MAX_MLP_NETS || h->net_width[k] == 0) {
-            h->err = std::string(who) + ": net_idx[" + std::to_string(i) + "] = " + std::to_string(k) + " names no loaded network";
-            return IGT_EINVAL;
-        }
-    }
+    if (B < 0 || !z0 || !u || !z || (model == 0 && !curv) || ((A == nullptr) != (Bm == nullptr)) ||
+        (model != 0 && model != 1)) { h->err = "igt_rollout: bad argument"; return IGT_EINVAL; }
     return IGT_OK;
-}
-static ProbIONet<float> iob_f32(const ProbIONet<double> &io, const igt_handle *h)
-{
-    ProbIONet<float> r;
-    static_cast<ProbIO &>(r) = io;
-    r.net_idx = io.net_idx;
-    r.nets = (const MlpNet<float> *)((const char *)h->bank + sizeof(h->netd));
-    return r;
-}
-static int bank_width(const igt_handle *h)
-{
-    int w = 0;
-    for (int k = 0; k < MAX_MLP_NETS; k++) if (h->net_width[k] > w) w = h->net_width[k];
-    return w;
 }
 
 static int rollout_dev_impl(igt_handle *h, int B, const float *z0, const float *u, const float *curv, float *z,
                             float *A, float *Bm, int model, cudaStream_t st)
 {
-    if (B < 0 || !z0 || !u || !z || (model == 0 && !curv) || ((A == nullptr) != (Bm == nullptr)) ||
-        (model != 0 && model != 1)) { h->err = "igt_rollout: bad argument"; return IGT_EINVAL; }
-    if (B == 0) return IGT_OK;
     int rc = begin_call(h, st), cs = 0;
     if (rc) return rc;
     rc = acquire_cslot(h, 0, st, &cs);
@@ -734,189 +920,22 @@ int igt_rollout_dev(igt_handle *h, int B, const float *z0, const float *u, const
 {
     if (!h) return IGT_EINVAL;
     std::lock_guard<std::mutex> lk(h->mu);
+    const int rc = check_rollout(h, B, z0, u, curv, z, A, Bm, model);
+    if (rc || B == 0) return rc;
     return rollout_dev_impl(h, B, z0, u, curv, z, A, Bm, model, (cudaStream_t)stream);
 }
 
 int igt_rollout_host(igt_handle *h, int B, const float *z0, const float *u, const float *curv, float *z,
                      float *A, float *Bm, int model)
 {
-    if (!h) return IGT_EINVAL;
-    if (B < 0 || !z0 || !u || !z || (model == 0 && !curv)) { h->err = "igt_rollout: bad argument"; return IGT_EINVAL; }
-    if (B == 0) return IGT_OK;
-    std::lock_guard<std::mutex> lk(h->mu);
-    { int rc0 = begin_call(h, nullptr); if (rc0) return rc0; }
-    const int N = h->prm.N, nz = model == 0 ? 7 : 4;
-    size_t n_z0 = (size_t)B * nz, n_u = (size_t)B * N * 2, n_c = (size_t)B * 3, n_z = (size_t)B * (N + 1) * nz;
-    size_t n_A = A ? (size_t)B * N * nz * nz : 0, n_B = A ? (size_t)B * N * nz * 2 : 0;
-    size_t total = (n_z0 + n_u + n_c + n_z + n_A + n_B) * sizeof(float);
-    int rc = grow(h, &h->stage, &h->stage_bytes, total, nullptr);
-    if (rc) return rc;
-    float *d = (float *)h->stage;
-    float *dz0 = d, *du = dz0 + n_z0, *dc = du + n_u, *dz = dc + n_c, *dA = dz + n_z, *dB = dA + n_A;
-    CK(cudaMemcpy(dz0, z0, n_z0 * 4, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(du, u, n_u * 4, cudaMemcpyHostToDevice));
-    if (model == 0) CK(cudaMemcpy(dc, curv, n_c * 4, cudaMemcpyHostToDevice));
-    rc = rollout_dev_impl(h, B, dz0, du, dc, dz, A ? dA : nullptr, A ? dB : nullptr, model, nullptr);
-    if (rc) return rc;
-    CK(cudaMemcpy(z, dz, n_z * 4, cudaMemcpyDeviceToHost));
-    if (A) { CK(cudaMemcpy(A, dA, n_A * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(Bm, dB, n_B * 4, cudaMemcpyDeviceToHost)); }
-    return IGT_OK;
-}
-
-static int solve_dev_impl(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
-                          const double *obs_xy, const double *obs_psi, const double *nn_ctx, const double *u_init,
-                          double *x, double *u, double *cost, double *viol, int *status, int *iters, cudaStream_t st,
-                          const int *warm = nullptr, const int *net_idx = nullptr)
-{
-    if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !x || !u || !cost || !viol || !status || !iters) {
-        h->err = "igt_solve: null argument"; return IGT_EINVAL;
-    }
-    const bool bank = net_idx != nullptr;
-    if (bank && !nn_ctx) { h->err = "igt_solve: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
-    if (bank && bank_width(h) == 0) { h->err = "igt_solve: net_idx given but no network was loaded"; return IGT_ENOMLP; }
-    if (nn_ctx && !bank && !h->has_mlp) { h->err = "igt_solve: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
-    const bool f64 = h->prm.precision == IGT_PREC_F64, obca = obs_psi != nullptr;
-    if (obca && !f64) { h->err = "igt_solve: the OBCA collision rows (obs_psi) need precision f64"; return IGT_EINVAL; }
-    if (B == 0) return IGT_OK;
-    int rc = begin_call(h, st), cs = 0;
-    if (rc) return rc;
-    WsLayout L; L.init(h->prm.N, h->prm.n_cinf, obca ? NGE_OBCA : NGE, obca ? NHE_OBCA : NHE);
-    size_t esz = f64 ? 8 : 4;
-    // value term (OBCA + gt_mpc: per-thread value term; a bank: exact evaluation whatever tensor_core_mlp says)
-    const bool use_tc = nn_ctx && !bank && h->tc.enabled && h->use_tc && !obca;
-    const int width = bank ? bank_width(h) : h->mlp_width;
-    const bool use_coop = nn_ctx && !use_tc && f64 && (bank ? width <= MLP_COOP_W : h->coop_ok) && !obca;
-    // latency path: at most one problem per SM and a workspace that fits shared memory next to the work lists; in
-    // gt_mpc (not with the tensor-core value term) the kernel's whole shared memory -- static, value-term buffers,
-    // workspace -- within the device's opt-in limit per block
-    const int small_v = small_gt_variant(use_coop, bank, obca, f64);
-    size_t small_smem = (size_t)L.total * esz;
-    bool small = h->use_small && !nn_ctx && B <= h->n_sm && small_smem <= 200 * 1024;
-    if (h->use_small && nn_ctx && !use_tc && B <= h->n_sm) {
-        if (use_coop) small_smem += bank ? small_coop_bytes<double, true, true>() : small_coop_bytes<double, true, false>();
-        rc = small_gt_fits(h, small_v, small_smem, &small);
-        if (rc) return rc;
-    }
-    // persistent lanes: one CTA of SOLVE_BLOCK threads per SM.  A batch smaller than the machine is spread
-    // over all SMs, a whole number of warps each: `quota` threads per CTA fetch problems, the rest of
-    // the CTA only helps in the CTA-wide phases (and adopts stragglers in the tail).
-    const int bs = SOLVE_BLOCK;
-    long n_cta = ((long)B + 31) / 32;
-    if (n_cta > h->n_sm) n_cta = h->n_sm;
-    long per_cta = ((long)B + n_cta - 1) / n_cta;
-    int quota = (int)((per_cta + 31) / 32 * 32);
-    if (quota > bs) quota = bs;
-    long n_slots = n_cta * bs;
-    rc = small ? IGT_OK : grow(h, &h->ws, &h->ws_bytes, (size_t)L.total * n_slots * esz, st);
-    if (rc) return rc;
-    if (nn_ctx && !use_tc && !use_coop) {                                 // per-thread evaluation: activations in HBM
-        // (one slab per persistent lane, or per CTA on the latency path)
-        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * (small ? B : n_slots) * esz, st);
-        if (rc) return rc;
-    }
-    // scheduler block (the work counter), then the cold-start guesses
-    const size_t off_guess = 256;
-    rc = grow(h, &h->guess, &h->guess_bytes, off_guess + (size_t)B * h->prm.N * 2 * sizeof(double), st);
-    if (rc) return rc;
-    char *sb = (char *)h->guess;
-    Sched sc;
-    sc.counter = (unsigned long long *)sb;
-    double *guess = (double *)(sb + off_guess);
-    rc = acquire_cslot(h, f64 ? 1 : 0, st, &cs);
-    if (rc) return rc;
-    CK(cudaMemsetAsync(sb, 0, 256, st));
-    ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters };
-    io.obs_psi = obs_psi;
-    io.warm = warm;
-    ProbIONet<double> iob;   // (the bank kernels' inputs: the f32 one reinterprets nets, same layout)
-    static_cast<ProbIO &>(iob) = io;
-    iob.net_idx = net_idx;
-    iob.nets = (const MlpNet<double> *)h->bank;
-    if (!u_init || warm) {
-        int gbs = 128, ggs = (B + gbs - 1) / gbs;
-        if (obca) guess_kernel<double, true><<<ggs, gbs, 0, st>>>(io, B, guess, cs);
-        else if (f64) guess_kernel<double, false><<<ggs, gbs, 0, st>>>(io, B, guess, cs);
-        else guess_kernel<float, false><<<ggs, gbs, 0, st>>>(io, B, guess, cs);
-        h->launches++;
-    }
-    int gs = (int)(n_slots / bs);
-    if (small && nn_ctx) {
-        // gt_mpc: the latency kernel's value-term instantiations (a bank problem with a bad index gets IGT_STATUS_BAD_NET)
-        double *scr = (double *)h->mlp_scratch;
-        float *scr_f = (float *)h->mlp_scratch;
-        switch (small_v) {
-        case 0: rc = launch_small_gt<double, false, true, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 1: rc = launch_small_gt<double, false, true, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 2: rc = launch_small_gt<double, false, false, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 3: rc = launch_small_gt<double, false, false, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 4: rc = launch_small_gt<double, true, false, false>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 5: rc = launch_small_gt<double, true, false, true>(h, iob, B, sc, guess, scr, width, small_smem, cs, st); break;
-        case 6: rc = launch_small_gt<float, false, false, false>(h, iob_f32(iob, h), B, sc, guess, scr_f, width, small_smem, cs, st); break;
-        default: rc = launch_small_gt<float, false, false, true>(h, iob_f32(iob, h), B, sc, guess, scr_f, width, small_smem, cs, st); break;
-        }
-        if (rc) return rc;
-    } else if (small) {
-        if (obca) {
-            CK(cudaFuncSetAttribute(solve_small_kernel<double, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
-            solve_small_kernel<double, true><<<B, bs, small_smem, st>>>(io, B, sc, guess, cs);
-        } else if (f64) {
-            CK(cudaFuncSetAttribute(solve_small_kernel<double, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
-            solve_small_kernel<double, false><<<B, bs, small_smem, st>>>(io, B, sc, guess, cs);
-        } else {
-            CK(cudaFuncSetAttribute(solve_small_kernel<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem));
-            solve_small_kernel<float, false><<<B, bs, small_smem, st>>>(io, B, sc, guess, cs);
-        }
-    } else if (bank) {
-        // gt_mpc with the network bank: the same kernels' BANK instantiations (problems with a bad index get
-        // IGT_STATUS_BAD_NET); cooperative value term where every network fits it, else per thread
-        double *scr = (double *)h->mlp_scratch;
-        const int rsm = IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * (int)esz : 0;
-        if (use_coop) {
-            const int sm = mlp_coop_bank_smem_bytes<double>(SOLVE_BLOCK);
-            CK(cudaFuncSetAttribute(solve_kernel<double, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-            solve_kernel<double, false, false, true, true><<<gs, bs, sm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, nullptr, width, h->tc, quota, cs);
-        } else if (obca) {
-            CK(cudaFuncSetAttribute(solve_kernel<double, false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-            solve_kernel<double, false, true, false, true><<<gs, bs, rsm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, scr, width, h->tc, quota, cs);
-        } else if (f64) {
-            CK(cudaFuncSetAttribute(solve_kernel<double, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-            solve_kernel<double, false, false, false, true><<<gs, bs, rsm, st>>>(iob, (double *)h->ws, n_slots, B, sc, guess, scr, width, h->tc, quota, cs);
-        } else {
-            CK(cudaFuncSetAttribute(solve_kernel<float, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-            solve_kernel<float, false, false, false, true><<<gs, bs, rsm, st>>>(iob_f32(iob, h), (float *)h->ws, n_slots, B, sc, guess, (float *)h->mlp_scratch, width, h->tc, quota, cs);
-        }
-    } else if (use_tc) {
-        if (f64) {
-            CK(cudaFuncSetAttribute(solve_kernel<double, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
-            solve_kernel<double, true, false><<<gs, bs, TC_SMEM_BYTES, st>>>(io, (double *)h->ws, n_slots, B, sc, guess, nullptr, h->mlp_width, h->tc, quota, cs);
-        } else {
-            CK(cudaFuncSetAttribute(solve_kernel<float, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
-            solve_kernel<float, true, false><<<gs, bs, TC_SMEM_BYTES, st>>>(io, (float *)h->ws, n_slots, B, sc, guess, nullptr, h->mlp_width, h->tc, quota, cs);
-        }
-    } else if (use_coop) {
-        // gt_mpc, exact value term: CTA-cooperative evaluation, one warp per evaluation (mlp_coop.cuh)
-        const int sm = mlp_coop_smem_bytes<double>(SOLVE_BLOCK);
-        CK(cudaFuncSetAttribute(solve_kernel<double, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-        solve_kernel<double, false, false, true><<<gs, bs, sm, st>>>(io, (double *)h->ws, n_slots, B, sc, guess, nullptr, h->mlp_width, h->tc, quota, cs);
-    } else if (obca) {
-        const int rsm = IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * 8 : 0;
-        CK(cudaFuncSetAttribute(solve_kernel<double, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-        solve_kernel<double, false, true><<<gs, bs, rsm, st>>>(io, (double *)h->ws, n_slots, B, sc, guess,
-                                                               nn_ctx ? (double *)h->mlp_scratch : nullptr, h->mlp_width, h->tc, quota, cs);
-    } else if (f64) {
-        const int rsm = IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * 8 : 0;
-        CK(cudaFuncSetAttribute(solve_kernel<double, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-        solve_kernel<double, false, false><<<gs, bs, rsm, st>>>(io, (double *)h->ws, n_slots, B, sc, guess,
-                                                                nn_ctx ? (double *)h->mlp_scratch : nullptr, h->mlp_width, h->tc, quota, cs);
-    } else {
-        const int rsm = IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * 4 : 0;
-        CK(cudaFuncSetAttribute(solve_kernel<float, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, rsm));
-        solve_kernel<float, false, false><<<gs, bs, rsm, st>>>(io, (float *)h->ws, n_slots, B, sc, guess,
-                                                               nn_ctx ? (float *)h->mlp_scratch : nullptr, h->mlp_width, h->tc, quota, cs);
-    }
-    h->launches++;
-    CK(cudaGetLastError());
-    return end_call(h, st, f64 ? 2 : 1);
+    return host_call(h, B, [&] { return check_rollout(h, B, z0, u, curv, z, A, Bm, model); }, [&](cudaStream_t st) {
+        const size_t N = h->prm.N, nb = B, nz = model == 0 ? 7 : 4;
+        const float *dz0, *du, *dc;
+        float *dz, *dA, *dB;
+        Staged a[] = { input(z0, nb * nz, &dz0), input(u, nb * N * 2, &du), input(model == 0 ? curv : nullptr, nb * 3, &dc),
+                       output(z, nb * (N + 1) * nz, &dz), output(A, nb * N * nz * nz, &dA), output(Bm, nb * N * nz * 2, &dB) };
+        return staged(h, st, a, [&] { return rollout_dev_impl(h, B, dz0, du, dc, dz, dA, dB, model, st); });
+    });
 }
 
 int igt_solve_ex_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
@@ -924,9 +943,10 @@ int igt_solve_ex_dev(igt_handle *h, int B, const double *x0, const double *u_pre
                      double *x, double *u, double *cost, double *viol, int *status, int *iters, void *stream)
 {
     if (!h) return IGT_EINVAL;
+    const ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters, obs_psi };
     std::lock_guard<std::mutex> lk(h->mu);
-    return solve_dev_impl(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, u_init, x, u, cost, viol, status, iters,
-                          (cudaStream_t)stream, nullptr, net_idx);
+    const int rc = check_solve(h, B, io, net_idx, false);
+    return rc ? rc : solve_dev_impl(h, B, io, net_idx, (cudaStream_t)stream);
 }
 
 int igt_solve_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
@@ -936,90 +956,22 @@ int igt_solve_dev(igt_handle *h, int B, const double *x0, const double *u_prev, 
     return igt_solve_ex_dev(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, nullptr, u_init, x, u, cost, viol, status, iters, stream);
 }
 
-// Host-pointer solve.  All inputs travel in ONE host-to-device copy and all outputs in ONE device-to-host copy on
-// the handle's own non-blocking stream: small batches (a closed-loop step solves B = 2) are packed into pinned
-// staging blocks first; large batches are copied array by array straight from the caller's (ideally pinned)
-// memory -- packing 100 MB on the host would cost more than the copies.
 int igt_solve_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
                       const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx, const double *u_init,
                       double *x, double *u, double *cost, double *viol, int *status, int *iters)
 {
-    if (!h) return IGT_EINVAL;
-    if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !x || !u || !cost || !viol || !status || !iters) {
-        h->err = "igt_solve: null argument"; return IGT_EINVAL;
-    }
-    if (net_idx && !nn_ctx) { h->err = "igt_solve: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
-    if (B == 0) return IGT_OK;
-    std::lock_guard<std::mutex> lk(h->mu);
-    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_solve"); if (rc0) return rc0; }
-    CK(cudaSetDevice(h->device));
-    if (!h->hstream) CK(cudaStreamCreateWithFlags(&h->hstream, cudaStreamNonBlocking));
-    cudaStream_t st = h->hstream;
-    int rc = begin_call(h, st);
-    if (rc) return rc;
-    const int N = h->prm.N;
-    size_t nb = (size_t)B;
-    size_t n_x0 = nb * 7, n_up = nb * 2, n_c = nb * 3, n_o = nb * (N + 1) * 2, n_ctx = nn_ctx ? nb * 4 : 0;
-    size_t n_ui = u_init ? nb * N * 2 : 0, n_x = nb * (N + 1) * 7, n_u = nb * N * 2, n_op = obs_psi ? nb * (N + 1) : 0;
-    size_t n_in = n_x0 + n_up + n_c + n_o + n_ctx + n_ui + n_op, n_out = n_x + n_u + 2 * nb;
-    size_t in_bytes = n_in * 8, out_bytes = n_out * 8 + 2 * nb * 4, total = in_bytes + out_bytes;
-    rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), st);
-    if (rc) return rc;
-    int *dnet = (int *)((char *)h->stage + total);                     // net_idx: after the outputs, copied on its own
-    if (net_idx) CK(cudaMemcpyAsync(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice, st));
-    double *d = (double *)h->stage;
-    double *dx0 = d, *dup = dx0 + n_x0, *dc = dup + n_up, *dob = dc + n_c, *dctx = dob + n_o, *dui = dctx + n_ctx;
-    double *dop = dui + n_ui;
-    double *dx = dop + n_op, *du = dx + n_x, *dcost = du + n_u, *dviol = dcost + nb;
-    int *dst = (int *)(dviol + nb), *dit = dst + nb;
-    const bool packed = total <= (size_t)1 << 20;
-    if (packed) {
-        if (h->pin_bytes < total) {
-            if (h->pin) { CK(cudaStreamSynchronize(st)); CK(cudaFreeHost(h->pin)); h->pin = nullptr; h->pin_bytes = 0; }
-            CK(cudaHostAlloc(&h->pin, total, cudaHostAllocDefault));
-            h->pin_bytes = total;
-        }
-        double *p = (double *)h->pin;
-        memcpy(p, x0, n_x0 * 8); p += n_x0;
-        memcpy(p, u_prev, n_up * 8); p += n_up;
-        memcpy(p, curv, n_c * 8); p += n_c;
-        memcpy(p, obs_xy, n_o * 8); p += n_o;
-        if (nn_ctx) { memcpy(p, nn_ctx, n_ctx * 8); p += n_ctx; }
-        if (u_init) { memcpy(p, u_init, n_ui * 8); p += n_ui; }
-        if (obs_psi) { memcpy(p, obs_psi, n_op * 8); p += n_op; }
-        CK(cudaMemcpyAsync(dx0, h->pin, in_bytes, cudaMemcpyHostToDevice, st));
-    } else {
-        CK(cudaMemcpyAsync(dx0, x0, n_x0 * 8, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dup, u_prev, n_up * 8, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dc, curv, n_c * 8, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dob, obs_xy, n_o * 8, cudaMemcpyHostToDevice, st));
-        if (nn_ctx) CK(cudaMemcpyAsync(dctx, nn_ctx, n_ctx * 8, cudaMemcpyHostToDevice, st));
-        if (u_init) CK(cudaMemcpyAsync(dui, u_init, n_ui * 8, cudaMemcpyHostToDevice, st));
-        if (obs_psi) CK(cudaMemcpyAsync(dop, obs_psi, n_op * 8, cudaMemcpyHostToDevice, st));
-    }
-    rc = solve_dev_impl(h, B, dx0, dup, dc, dob, obs_psi ? dop : nullptr, nn_ctx ? dctx : nullptr, u_init ? dui : nullptr,
-                        dx, du, dcost, dviol, dst, dit, st, nullptr, net_idx ? dnet : nullptr);
-    if (rc) return rc;
-    if (packed) {
-        char *q = (char *)h->pin + in_bytes;
-        CK(cudaMemcpyAsync(q, dx, out_bytes, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        memcpy(x, q, n_x * 8); q += n_x * 8;
-        memcpy(u, q, n_u * 8); q += n_u * 8;
-        memcpy(cost, q, nb * 8); q += nb * 8;
-        memcpy(viol, q, nb * 8); q += nb * 8;
-        memcpy(status, q, nb * 4); q += nb * 4;
-        memcpy(iters, q, nb * 4);
-    } else {
-        CK(cudaMemcpyAsync(x, dx, n_x * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(u, du, n_u * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(cost, dcost, nb * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(viol, dviol, nb * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(status, dst, nb * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(iters, dit, nb * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    }
-    return IGT_OK;
+    const ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters, obs_psi };
+    return host_call(h, B, [&] { return check_solve(h, B, io, net_idx, true); }, [&](cudaStream_t st) {
+        const size_t N = h->prm.N, nb = B;
+        ProbIO d = {};
+        const int *dnet;
+        Staged a[] = { input(x0, nb * 7, &d.x0), input(u_prev, nb * 2, &d.u_prev), input(curv, nb * 3, &d.curv),
+                       input(obs_xy, nb * (N + 1) * 2, &d.obs), input(nn_ctx, nb * 4, &d.ctx), input(u_init, nb * N * 2, &d.u_init),
+                       input(obs_psi, nb * (N + 1), &d.obs_psi), input(net_idx, nb, &dnet),
+                       output(x, nb * (N + 1) * 7, &d.x), output(u, nb * N * 2, &d.u), output(cost, nb, &d.cost), output(viol, nb, &d.viol),
+                       output(status, nb, &d.status), output(iters, nb, &d.iters) };
+        return staged(h, st, a, [&] { return solve_dev_impl(h, B, d, dnet, st); });
+    });
 }
 
 int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
@@ -1033,53 +985,34 @@ int igt_eval_ex_host(igt_handle *h, int B, const double *x0, const double *u_pre
                      const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx, const double *u,
                      double *cost, double *viol, double *z)
 {
-    if (!h) return IGT_EINVAL;
-    if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !u || !cost || !viol) { h->err = "igt_eval: null argument"; return IGT_EINVAL; }
-    if (net_idx && !nn_ctx) { h->err = "igt_eval: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
-    if (nn_ctx && !net_idx && !h->has_mlp) { h->err = "igt_eval: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
-    if (B == 0) return IGT_OK;
-    std::lock_guard<std::mutex> lk(h->mu);
-    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_eval"); if (rc0) return rc0; }
-    int cs = 0;
-    { int rc0 = begin_call(h, nullptr); if (rc0) return rc0; }
-    const int N = h->prm.N;
-    size_t nb = (size_t)B;
-    size_t n_x0 = nb * 7, n_up = nb * 2, n_c = nb * 3, n_o = nb * (N + 1) * 2, n_ctx = nn_ctx ? nb * 4 : 0;
-    size_t n_u = nb * N * 2, n_z = nb * (N + 1) * 7, n_op = obs_psi ? nb * (N + 1) : 0;
-    size_t total = (n_x0 + n_up + n_c + n_o + n_ctx + n_u + n_z + 2 * nb + n_op) * 8;
-    int rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), nullptr);
-    if (rc) return rc;
-    const int width = net_idx ? bank_width(h) : h->mlp_width;
-    if (nn_ctx) { rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * B * 8, nullptr); if (rc) return rc; }
-    int *dnet = (int *)((char *)h->stage + total);
-    if (net_idx) CK(cudaMemcpy(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice));
-    double *d = (double *)h->stage;
-    double *dx0 = d, *dup = dx0 + n_x0, *dc = dup + n_up, *dob = dc + n_c, *dctx = dob + n_o, *du = dctx + n_ctx;
-    double *dz = du + n_u, *dcost = dz + n_z, *dviol = dcost + nb, *dop = dviol + nb;
-    if (obs_psi) CK(cudaMemcpy(dop, obs_psi, n_op * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dx0, x0, n_x0 * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dup, u_prev, n_up * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dc, curv, n_c * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dob, obs_xy, n_o * 8, cudaMemcpyHostToDevice));
-    if (nn_ctx) CK(cudaMemcpy(dctx, nn_ctx, n_ctx * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(du, u, n_u * 8, cudaMemcpyHostToDevice));
-    rc = acquire_cslot(h, 1, nullptr, &cs);
-    if (rc) return rc;
-    int bs = 128, gs = (B + bs - 1) / bs;
-    if (net_idx)
-        eval_kernel<true><<<gs, bs>>>(B, dx0, dup, dc, dob, dctx, du, dcost, dviol, dz, (double *)h->mlp_scratch, width, cs,
-                                      obs_psi ? dop : nullptr, dnet, (const MlpNet<double> *)h->bank);
-    else
-        eval_kernel<false><<<gs, bs>>>(B, dx0, dup, dc, dob, nn_ctx ? dctx : nullptr, du, dcost, dviol, dz,
-                                       nn_ctx ? (double *)h->mlp_scratch : nullptr, h->mlp_width, cs, obs_psi ? dop : nullptr, nullptr, nullptr);
-    h->launches++;
-    CK(cudaGetLastError());
-    rc = end_call(h, nullptr, 2);
-    if (rc) return rc;
-    CK(cudaMemcpy(cost, dcost, nb * 8, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(viol, dviol, nb * 8, cudaMemcpyDeviceToHost));
-    if (z) CK(cudaMemcpy(z, dz, n_z * 8, cudaMemcpyDeviceToHost));
-    return IGT_OK;
+    auto check = [&]() -> int {
+        if (B < 0 || !x0 || !u_prev || !curv || !obs_xy || !u || !cost || !viol) { h->err = "igt_eval: null argument"; return IGT_EINVAL; }
+        if (net_idx && !nn_ctx) { h->err = "igt_eval: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
+        if (nn_ctx && !net_idx && value_width(h, false) == 0) { h->err = "igt_eval: nn_ctx given but igt_set_mlp was never called"; return IGT_ENOMLP; }
+        return net_idx ? check_net_idx(h, B, net_idx, "igt_eval") : IGT_OK;
+    };
+    return host_call(h, B, check, [&](cudaStream_t st) {
+        const size_t N = h->prm.N, nb = B;
+        const double *dx0, *dup, *dc, *dob, *dctx, *du, *dop;
+        const int *dnet;
+        double *dcost, *dviol, *dz;
+        Staged a[] = { input(x0, nb * 7, &dx0), input(u_prev, nb * 2, &dup), input(curv, nb * 3, &dc), input(obs_xy, nb * (N + 1) * 2, &dob),
+                       input(nn_ctx, nb * 4, &dctx), input(u, nb * N * 2, &du), input(obs_psi, nb * (N + 1), &dop), input(net_idx, nb, &dnet),
+                       output(cost, nb, &dcost), output(viol, nb, &dviol), output(z, nb * (N + 1) * 7, &dz) };
+        return staged(h, st, a, [&] {
+            const int width = value_width(h, net_idx != nullptr);
+            if (nn_ctx) { const int rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * nb * 8, st); if (rc) return rc; }
+            int cs = 0;
+            const int rc = acquire_cslot(h, 1, st, &cs);
+            if (rc) return rc;
+            auto *k = net_idx ? eval_kernel<true> : eval_kernel<false>;
+            k<<<(B + 127) / 128, 128, 0, st>>>(B, dx0, dup, dc, dob, dctx, du, dcost, dviol, dz, nn_ctx ? (double *)h->mlp_scratch : nullptr,
+                                               width, cs, dop, dnet, (const MlpNet<double> *)h->bank);
+            h->launches++;
+            CK(cudaGetLastError());
+            return end_call(h, st, 2);
+        });
+    });
 }
 
 int igt_eval_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
@@ -1122,64 +1055,48 @@ int igt_measure_fma_peak(igt_handle *h, int precision, double *tflops)
 int igt_mlp_value_ex_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx, const int *net_idx,
                           double *out, int use_tensor_cores)
 {
-    if (!h) return IGT_EINVAL;
-    if (B < 0 || !sN || !vN || !nn_ctx || !out) { h->err = "igt_mlp_value: null argument"; return IGT_EINVAL; }
-    if (net_idx && use_tensor_cores != 0 && use_tensor_cores != 2) {
-        h->err = "igt_mlp_value: with net_idx the mode must be 0 (per thread) or 2 (cooperative)"; return IGT_EINVAL;
-    }
-    std::lock_guard<std::mutex> lk(h->mu);   // (the bank state below is read under the lock: igt_set_mlp_at takes it)
-    const int width = net_idx ? bank_width(h) : h->mlp_width;
-    if (net_idx ? width == 0 : !h->has_mlp) { h->err = "igt_mlp_value: igt_set_mlp was never called"; return IGT_ENOMLP; }
-    if (use_tensor_cores == 1 && !h->tc.enabled) { h->err = "igt_mlp_value: tensor-core path needs a 6-128-128-1 network"; return IGT_EINVAL; }
-    if (use_tensor_cores == 2 && (net_idx ? width > MLP_COOP_W : !h->coop_ok)) {
-        h->err = "igt_mlp_value: the cooperative evaluation needs layers <= 128 wide"; return IGT_EINVAL;
-    }
-    if (B == 0) return IGT_OK;
-    if (net_idx) { const int rc0 = check_net_idx(h, B, net_idx, "igt_mlp_value"); if (rc0) return rc0; }
-    int cs = 0;
-    int rc = begin_call(h, nullptr);
-    if (rc) return rc;
-    size_t nb = (size_t)B, total = (nb * 2 + nb * 4 + nb * 6) * 8;
-    rc = grow(h, &h->stage, &h->stage_bytes, total + (net_idx ? nb * 4 : 0), nullptr);
-    if (rc) return rc;
-    double *ds = (double *)h->stage, *dv = ds + nb, *dc = dv + nb, *dout = dc + nb * 4;
-    int *dnet = (int *)((char *)h->stage + total);
-    if (net_idx) CK(cudaMemcpy(dnet, net_idx, nb * 4, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(ds, sN, nb * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dv, vN, nb * 8, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dc, nn_ctx, nb * 32, cudaMemcpyHostToDevice));
-    if (use_tensor_cores == 2) {
-        rc = acquire_cslot(h, 1, nullptr, &cs);
-        if (rc) return rc;
-        int grid = (int)((nb + 255) / 256);
-        if (grid > h->n_sm) grid = h->n_sm;
-        if (net_idx) {
-            const int sm = mlp_coop_bank_smem_bytes<double>(256);
-            CK(cudaFuncSetAttribute(mlp_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-            mlp_coop_kernel<true><<<grid, 256, sm>>>(B, ds, dv, dc, dout, cs, dnet, (const MlpNet<double> *)h->bank);
-        } else {
-            const int sm = mlp_coop_smem_bytes<double>(256);
-            CK(cudaFuncSetAttribute(mlp_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-            mlp_coop_kernel<false><<<grid, 256, sm>>>(B, ds, dv, dc, dout, cs, nullptr, nullptr);
+    const int mode = use_tensor_cores;
+    auto check = [&]() -> int {
+        if (B < 0 || !sN || !vN || !nn_ctx || !out) { h->err = "igt_mlp_value: null argument"; return IGT_EINVAL; }
+        if (net_idx && mode != 0 && mode != 2) {
+            h->err = "igt_mlp_value: with net_idx the mode must be 0 (per thread) or 2 (cooperative)"; return IGT_EINVAL;
         }
-    } else if (use_tensor_cores) {
-        int grid = (int)((nb + 255) / 256);
-        if (grid > h->n_sm) grid = h->n_sm;
-        mlp_tc_kernel<<<grid, 256, TC_SMEM_BYTES>>>(h->tc, B, ds, dv, dc, dout);
-    } else {
-        rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * nb * 8, nullptr);
-        if (rc) return rc;
-        rc = acquire_cslot(h, 1, nullptr, &cs);
-        if (rc) return rc;
-        if (net_idx) mlp_ref_kernel<true><<<(int)((nb + 127) / 128), 128>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, width, cs, dnet, (const MlpNet<double> *)h->bank);
-        else mlp_ref_kernel<false><<<(int)((nb + 127) / 128), 128>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, width, cs, nullptr, nullptr);
-    }
-    h->launches++;
-    CK(cudaGetLastError());
-    rc = end_call(h, nullptr, use_tensor_cores == 1 ? 0 : 2);
-    if (rc) return rc;
-    CK(cudaMemcpy(out, dout, nb * 48, cudaMemcpyDeviceToHost));
-    return IGT_OK;
+        const int width = value_width(h, net_idx != nullptr);
+        if (width == 0) { h->err = "igt_mlp_value: igt_set_mlp was never called"; return IGT_ENOMLP; }
+        if (mode == 1 && !h->tc.enabled) { h->err = "igt_mlp_value: tensor-core path needs a 6-128-128-1 network"; return IGT_EINVAL; }
+        if (mode == 2 && width > MLP_COOP_W) { h->err = "igt_mlp_value: the cooperative evaluation needs layers <= 128 wide"; return IGT_EINVAL; }
+        return net_idx ? check_net_idx(h, B, net_idx, "igt_mlp_value") : IGT_OK;
+    };
+    return host_call(h, B, check, [&](cudaStream_t st) {
+        const size_t nb = B;
+        const double *ds, *dv, *dc;
+        const int *dnet;
+        double *dout;
+        Staged a[] = { input(sN, nb, &ds), input(vN, nb, &dv), input(nn_ctx, nb * 4, &dc), input(net_idx, nb, &dnet), output(out, nb * 6, &dout) };
+        return staged(h, st, a, [&] {
+            const int grid = (int)std::min<size_t>((nb + 255) / 256, (size_t)h->n_sm);
+            const MlpNet<double> *nets = (const MlpNet<double> *)h->bank;
+            int cs = 0, rc;
+            if (mode == 2) {
+                if ((rc = acquire_cslot(h, 1, st, &cs))) return rc;
+                const int sm = net_idx ? mlp_coop_bank_smem_bytes<double>(256) : mlp_coop_smem_bytes<double>(256);
+                auto *k = net_idx ? mlp_coop_kernel<true> : mlp_coop_kernel<false>;
+                CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+                k<<<grid, 256, sm, st>>>(B, ds, dv, dc, dout, cs, dnet, nets);
+            } else if (mode) {
+                mlp_tc_kernel<<<grid, 256, TC_SMEM_BYTES, st>>>(h->tc, B, ds, dv, dc, dout);
+            } else {
+                const int width = value_width(h, net_idx != nullptr);
+                if ((rc = grow(h, &h->mlp_scratch, &h->mlp_scratch_bytes, (size_t)12 * width * nb * 8, st))) return rc;
+                if ((rc = acquire_cslot(h, 1, st, &cs))) return rc;
+                auto *k = net_idx ? mlp_ref_kernel<true> : mlp_ref_kernel<false>;
+                k<<<(int)((nb + 127) / 128), 128, 0, st>>>(B, ds, dv, dc, dout, (double *)h->mlp_scratch, width, cs, dnet, nets);
+            }
+            h->launches++;
+            CK(cudaGetLastError());
+            return end_call(h, st, mode == 1 ? 0 : 2);
+        });
+    });
 }
 
 int igt_mlp_value_host(igt_handle *h, int B, const double *sN, const double *vN, const double *nn_ctx, double *out,
@@ -1236,94 +1153,66 @@ int igt_episode_run_ex_host(igt_handle *h, int E, int steps, int mode, const dou
                             const double *z0, const double *u_prev0, const double *enc, const int *net_idx, double *z_cl,
                             double *u_cl, int *solved, float *step_ms)
 {
-    if (!h) return IGT_EINVAL;
-    if (E < 0 || steps < 1 || !route_desc || !curv || !z0 || !u_prev0 || !enc || !z_cl || !u_cl || !solved) {
-        h->err = "igt_episode_run: bad argument"; return IGT_EINVAL;
-    }
-    if (mode & ~(IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)) {
-        h->err = "igt_episode_run: unknown mode bits (IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)"; return IGT_EINVAL;
-    }
     const int gt_mpc = (mode & IGT_EPISODE_GT_MPC) != 0;
     const bool obca = (mode & IGT_EPISODE_OBCA) != 0;
-    if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_episode_run: needs precision f64"; return IGT_EINVAL; }
-    if (net_idx && !gt_mpc) { h->err = "igt_episode_run: net_idx needs the IGT_EPISODE_GT_MPC mode bit"; return IGT_EINVAL; }
-    if (gt_mpc && !net_idx && !h->has_mlp) { h->err = "igt_episode_run: gt_mpc needs igt_set_mlp"; return IGT_ENOMLP; }
-    if (E == 0) return IGT_OK;
-    std::lock_guard<std::mutex> lk(h->mu);
-    if (net_idx) { const int rc0 = check_net_idx(h, E, net_idx, "igt_episode_run"); if (rc0) return rc0; }
-    CK(cudaSetDevice(h->device));
-    if (!h->hstream) CK(cudaStreamCreateWithFlags(&h->hstream, cudaStreamNonBlocking));
-    cudaStream_t st = h->hstream;
-    int rc = begin_call(h, st);
-    if (rc) return rc;
-    const int N = h->prm.N, B = 2 * E, T = steps;
-    const size_t nb = (size_t)B;
-    // one device block: state, records, solver inputs and two sets of solver outputs (the plans of t and t-1)
-    const size_t n_z = nb * 7, n_up = nb * 2, n_cv = nb * 3, n_rd = nb * ROUTE_DESC, n_en = nb, n_obs = nb * (N + 1) * 2,
-                 n_ctx = nb * 4, n_ui = nb * N * 2, n_zcl = nb * (T + 1) * 7, n_ucl = nb * T * 2, n_x = nb * (N + 1) * 7,
-                 n_u = nb * N * 2, n_op = obca ? nb * (N + 1) : 0;
-    const size_t n_dbl = n_z + n_up + n_cv + n_rd + n_en + n_obs + n_ctx + n_ui + n_zcl + n_ucl + 2 * (n_x + n_u + 2 * nb) + n_op;
-    const size_t n_int = nb /*warm*/ + nb /*prev_ok*/ + nb * T /*solved*/ + 2 * 2 * nb /*status, iters x2*/ + (net_idx ? nb : 0);
-    rc = grow(h, &h->episode, &h->episode_bytes, n_dbl * 8 + n_int * 4, st);
-    if (rc) return rc;
-    double *d = (double *)h->episode;
-    EpisodeBufs eb;
-    eb.z = d; d += n_z; eb.u_prev = d; d += n_up;
-    double *dcv = d; d += n_cv; double *drd = d; d += n_rd; double *den = d; d += n_en;
-    eb.curv = dcv; eb.rd = drd; eb.enc = den;
-    eb.obs = d; d += n_obs; eb.ctx = d; d += n_ctx; eb.u_init = d; d += n_ui;
-    eb.z_cl = d; d += n_zcl; eb.u_cl = d; d += n_ucl;
-    double *px[2], *pu[2], *pcost[2], *pviol[2];
-    for (int i = 0; i < 2; i++) { px[i] = d; d += n_x; pu[i] = d; d += n_u; pcost[i] = d; d += nb; pviol[i] = d; d += nb; }
-    eb.obs_psi = obca ? d : nullptr; d += n_op;
-    int *ip = (int *)d;
-    eb.warm = ip; ip += nb; eb.prev_ok = ip; ip += nb; eb.solved = ip; ip += nb * T;
-    int *pst[2], *pit[2];
-    for (int i = 0; i < 2; i++) { pst[i] = ip; ip += nb; pit[i] = ip; ip += nb; }
-    int *dnet = net_idx ? ip : nullptr;
-    std::vector<int> veh_net;
-    if (net_idx) {   // both vehicles of episode e plan with network net_idx[e]: expanded once, the glue kernels never see it
-        veh_net.resize(nb);
-        for (int b = 0; b < B; b++) veh_net[b] = net_idx[b / 2];
-        CK(cudaMemcpyAsync(dnet, veh_net.data(), nb * 4, cudaMemcpyHostToDevice, st));
-    }
-    CK(cudaMemcpyAsync(eb.z, z0, n_z * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(eb.u_prev, u_prev0, n_up * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(dcv, curv, n_cv * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(drd, route_desc, n_rd * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(den, enc, n_en * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(eb.prev_ok, 0, nb * 4, st));
-    // z_cl[:, :, 0] = z0
-    CK(cudaMemcpy2DAsync(eb.z_cl, (size_t)(T + 1) * 7 * 8, eb.z, 7 * 8, 7 * 8, nb, cudaMemcpyDeviceToDevice, st));
+    auto check = [&]() -> int {
+        if (E < 0 || steps < 1 || !route_desc || !curv || !z0 || !u_prev0 || !enc || !z_cl || !u_cl || !solved) {
+            h->err = "igt_episode_run: bad argument"; return IGT_EINVAL;
+        }
+        if (mode & ~(IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)) {
+            h->err = "igt_episode_run: unknown mode bits (IGT_EPISODE_GT_MPC | IGT_EPISODE_OBCA)"; return IGT_EINVAL;
+        }
+        if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_episode_run: needs precision f64"; return IGT_EINVAL; }
+        if (net_idx && !gt_mpc) { h->err = "igt_episode_run: net_idx needs the IGT_EPISODE_GT_MPC mode bit"; return IGT_EINVAL; }
+        if (gt_mpc && !net_idx && value_width(h, false) == 0) { h->err = "igt_episode_run: gt_mpc needs igt_set_mlp"; return IGT_ENOMLP; }
+        return net_idx ? check_net_idx(h, E, net_idx, "igt_episode_run") : IGT_OK;
+    };
     std::vector<cudaEvent_t> ev;
-    if (step_ms) { ev.resize(T + 1); for (auto &e : ev) CK(cudaEventCreate(&e)); CK(cudaEventRecord(ev[0], st)); }
-    const int bs = 128, gs = (B + bs - 1) / bs;
-    int cs = 0;
-    for (int t = 0; t < T; t++) {
-        const int cur = t & 1, prv = cur ^ 1;
-        if (obca) episode_pre_kernel<true><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
-        else episode_pre_kernel<false><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
-        h->launches++;
-        rc = solve_dev_impl(h, B, eb.z, eb.u_prev, eb.curv, eb.obs, eb.obs_psi, gt_mpc ? eb.ctx : nullptr, eb.u_init, px[cur], pu[cur],
-                            pcost[cur], pviol[cur], pst[cur], pit[cur], st, eb.warm, dnet);
-        if (rc) return rc;
-        rc = acquire_cslot(h, 1, st, &cs);
-        if (rc) return rc;
-        episode_post_kernel<<<gs, bs, 0, st>>>(eb, B, N, T, t, h->prm.a_min, px[cur], pu[cur], pst[cur], cs);
-        h->launches++;
-        if (step_ms) CK(cudaEventRecord(ev[t + 1], st));
-    }
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(z_cl, eb.z_cl, n_zcl * 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(u_cl, eb.u_cl, n_ucl * 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(solved, eb.solved, nb * T * 4, cudaMemcpyDeviceToHost, st));
-    rc = end_call(h, st, 2);
-    if (rc) return rc;
-    CK(cudaStreamSynchronize(st));
-    if (step_ms) {
-        for (int t = 0; t < T; t++) CK(cudaEventElapsedTime(&step_ms[t], ev[t], ev[t + 1]));
-        for (auto &e : ev) cudaEventDestroy(e);
-    }
+    const int rc = host_call(h, E, check, [&](cudaStream_t st) {
+        const int N = h->prm.N, B = 2 * E, T = steps;
+        const size_t nb = B;
+        std::vector<int> veh_net;   // both vehicles of episode e plan with network net_idx[e]: expanded once, the glue kernels never see it
+        if (net_idx) { veh_net.resize(nb); for (int b = 0; b < B; b++) veh_net[b] = net_idx[b / 2]; }
+        // one device block: state, records, solver inputs and two sets of solver outputs (the plans of t and t-1)
+        EpisodeBufs eb;
+        const int *dnet;
+        double *px[2], *pu[2], *pcost[2], *pviol[2];
+        int *pst[2], *pit[2];
+        Staged a[] = { input(z0, nb * 7, &eb.z), input(u_prev0, nb * 2, &eb.u_prev), input(curv, nb * 3, &eb.curv),
+                       input(route_desc, nb * ROUTE_DESC, &eb.rd), input(enc, nb, &eb.enc), input(net_idx ? veh_net.data() : nullptr, nb, &dnet),
+                       output(z_cl, nb * (T + 1) * 7, &eb.z_cl), output(u_cl, nb * T * 2, &eb.u_cl), output(solved, nb * T, &eb.solved),
+                       device_only(nb * (N + 1) * 2, &eb.obs), device_only(nb * 4, &eb.ctx), device_only(nb * N * 2, &eb.u_init),
+                       device_only(obca ? nb * (N + 1) : 0, &eb.obs_psi), device_only(nb, &eb.warm), device_only(nb, &eb.prev_ok),
+                       device_only(nb * (N + 1) * 7, &px[0]), device_only(nb * N * 2, &pu[0]), device_only(nb, &pcost[0]), device_only(nb, &pviol[0]),
+                       device_only(nb * (N + 1) * 7, &px[1]), device_only(nb * N * 2, &pu[1]), device_only(nb, &pcost[1]), device_only(nb, &pviol[1]),
+                       device_only(nb, &pst[0]), device_only(nb, &pit[0]), device_only(nb, &pst[1]), device_only(nb, &pit[1]) };
+        return staged(h, st, a, [&] {
+            CK(cudaMemsetAsync(eb.prev_ok, 0, nb * 4, st));
+            // z_cl[:, :, 0] = z0
+            CK(cudaMemcpy2DAsync(eb.z_cl, (size_t)(T + 1) * 7 * 8, eb.z, 7 * 8, 7 * 8, nb, cudaMemcpyDeviceToDevice, st));
+            if (step_ms) { ev.resize(T + 1); for (auto &e : ev) CK(cudaEventCreate(&e)); CK(cudaEventRecord(ev[0], st)); }
+            const int bs = 128, gs = (B + bs - 1) / bs;
+            int cs = 0, rc;
+            for (int t = 0; t < T; t++) {
+                const int cur = t & 1, prv = cur ^ 1;
+                if (obca) episode_pre_kernel<true><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
+                else episode_pre_kernel<false><<<gs, bs, 0, st>>>(eb, B, N, h->prm.dt, t, gt_mpc, px[prv], pu[prv]);
+                h->launches++;
+                const ProbIO io = { eb.z, eb.u_prev, eb.curv, eb.obs, gt_mpc ? eb.ctx : nullptr, eb.u_init, px[cur], pu[cur],
+                                    pcost[cur], pviol[cur], pst[cur], pit[cur], eb.obs_psi, eb.warm };
+                if ((rc = solve_dev_impl(h, B, io, dnet, st))) return rc;
+                if ((rc = acquire_cslot(h, 1, st, &cs))) return rc;
+                episode_post_kernel<<<gs, bs, 0, st>>>(eb, B, N, T, t, h->prm.a_min, px[cur], pu[cur], pst[cur], cs);
+                h->launches++;
+                if (step_ms) CK(cudaEventRecord(ev[t + 1], st));
+            }
+            CK(cudaGetLastError());
+            return end_call(h, st, 2);
+        });
+    });
+    if (rc || ev.empty()) return rc;
+    for (int t = 0; t < steps; t++) CK(cudaEventElapsedTime(&step_ms[t], ev[t], ev[t + 1]));
+    for (auto &e : ev) cudaEventDestroy(e);
     return IGT_OK;
 }
 
@@ -1344,4 +1233,3 @@ int igt_set_option(igt_handle *h, const char *name, double value)
 }
 
 }  // extern "C"
-

@@ -286,15 +286,13 @@ def run_closed_loop_device(solver, specs, steps=150, N=40, d_min=5.6, mode="mpc"
     z_cl = np.zeros((E, 2, steps + 1, 7)); u_cl = np.zeros((E, 2, steps, 2)); solved = np.zeros((E, 2, steps), dtype=np.int32)
     ms = np.zeros(steps, dtype=np.float32)
     vp = lambda a: C.c_void_p(a.ctypes.data)
-    if net_idx is None:
-        rc = solver.lib.igt_episode_run_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
-                                             vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
-        solver._check(rc, "igt_episode_run_host")
-    else:
+    nets = None
+    if net_idx is not None:
         nets = np.ascontiguousarray(net_idx, dtype=np.int32)
         if nets.shape != (E,):
             raise ValueError("net_idx: one bank slot per episode, expected shape (%d,), got %s" % (E, nets.shape))
-        rc = solver.lib.igt_episode_run_ex_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
-                                                vp(nets), vp(z_cl), vp(u_cl), vp(solved), vp(ms) if record_latency else None)
-        solver._check(rc, "igt_episode_run_ex_host")
+    rc = solver.lib.igt_episode_run_ex_host(solver._h, E, steps, flags, vp(rd), vp(curv), vp(z), vp(u_prev), vp(enc),
+                                            None if nets is None else vp(nets), vp(z_cl), vp(u_cl), vp(solved),
+                                            vp(ms) if record_latency else None)
+    solver._check(rc, "igt_episode_run_ex_host")
     return _outcome(z_cl, u_cl, solved.astype(bool), d_min, ca_type, [float(v) for v in ms] if record_latency else [])

@@ -149,13 +149,9 @@ class BatchSolver:
         sN = _f64(sN).ravel(); B = sN.shape[0]
         vN = _f64(vN, (B,)); nn_ctx = _f64(nn_ctx, (B, 4))
         out = np.empty((B, 6))
-        if net_idx is None:
-            rc = self.lib.igt_mlp_value_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(out), int(tensor_cores))
-            self._check(rc, "igt_mlp_value_host")
-        else:
-            rc = self.lib.igt_mlp_value_ex_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(_net_idx(net_idx, B)), _hp(out),
-                                                int(tensor_cores))
-            self._check(rc, "igt_mlp_value_ex_host")
+        rc = self.lib.igt_mlp_value_ex_host(self._h, B, _hp(sN), _hp(vN), _hp(nn_ctx), _hp(_net_idx(net_idx, B)), _hp(out),
+                                            int(tensor_cores))
+        self._check(rc, "igt_mlp_value_ex_host")
         return out
 
     # -- host-pointer calls (copies inside) ---------------------------------------------------
@@ -175,16 +171,10 @@ class BatchSolver:
         if out is None:
             out = dict(x=np.empty((B, N + 1, 7)), u=np.empty((B, N, 2)), cost=np.empty(B), viol=np.empty(B),
                        status=np.empty(B, dtype=np.int32), iters=np.empty(B, dtype=np.int32))
-        if net_idx is None:
-            rc = self.lib.igt_solve_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                         _hp(u_init), _hp(out["x"]), _hp(out["u"]), _hp(out["cost"]),
-                                         _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
-            self._check(rc, "igt_solve_host")
-        else:
-            rc = self.lib.igt_solve_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                            _hp(_net_idx(net_idx, B)), _hp(u_init), _hp(out["x"]), _hp(out["u"]),
-                                            _hp(out["cost"]), _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
-            self._check(rc, "igt_solve_ex_host")
+        rc = self.lib.igt_solve_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                        _hp(_net_idx(net_idx, B)), _hp(u_init), _hp(out["x"]), _hp(out["u"]),
+                                        _hp(out["cost"]), _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
+        self._check(rc, "igt_solve_ex_host")
         return out
 
     def evaluate(self, x0, u_prev, curv, obs_xy, u, nn_ctx=None, obs_psi=None, net_idx=None):
@@ -197,14 +187,9 @@ class BatchSolver:
         nn_ctx = None if nn_ctx is None else _f64(nn_ctx, (B, 4))
         obs_psi = None if obs_psi is None else _f64(obs_psi, (B, N + 1))
         cost, viol, z = np.empty(B), np.empty(B), np.empty((B, N + 1, 7))
-        if net_idx is None:
-            rc = self.lib.igt_eval_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                        _hp(u), _hp(cost), _hp(viol), _hp(z))
-            self._check(rc, "igt_eval_host")
-        else:
-            rc = self.lib.igt_eval_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
-                                           _hp(_net_idx(net_idx, B)), _hp(u), _hp(cost), _hp(viol), _hp(z))
-            self._check(rc, "igt_eval_ex_host")
+        rc = self.lib.igt_eval_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
+                                       _hp(_net_idx(net_idx, B)), _hp(u), _hp(cost), _hp(viol), _hp(z))
+        self._check(rc, "igt_eval_ex_host")
         return dict(cost=cost, viol=viol, x=z)
 
     def rollout(self, z0, u, curv=None, jac=False, model=0):
@@ -260,16 +245,10 @@ class BatchSolver:
                 check(out[k], shp, dt, "out[%r]" % k)
         st = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
         p = lambda t: None if t is None else _vp(t.data_ptr())
-        if net_idx is None:
-            rc = self.lib.igt_solve_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(u_init),
-                                        p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]), p(out["status"]),
-                                        p(out["iters"]), _vp(st))
-            self._check(rc, "igt_solve_dev")
-        else:
-            rc = self.lib.igt_solve_ex_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(net_idx),
-                                           p(u_init), p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]),
-                                           p(out["status"]), p(out["iters"]), _vp(st))
-            self._check(rc, "igt_solve_ex_dev")
+        rc = self.lib.igt_solve_ex_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(net_idx),
+                                       p(u_init), p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]),
+                                       p(out["status"]), p(out["iters"]), _vp(st))
+        self._check(rc, "igt_solve_ex_dev")
         return out
 
 

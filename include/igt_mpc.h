@@ -9,7 +9,8 @@
  * Conventions: plain pointers and sizes only; every array is contiguous, batch-major
  * ("problem b" first).  `*_dev` entry points take DEVICE pointers and enqueue work on `stream`
  * (a cudaStream_t passed as void*; NULL = legacy default stream) without synchronising;
- * `*_host` entry points take HOST pointers, copy in, run, copy out and synchronise.
+ * `*_host` entry points take HOST pointers, copy in, run, copy out and synchronise; they run on a
+ * private non-blocking stream of the handle, not on the legacy default stream.
  * Every function returns 0 on success or a negative IGT_E* code; igt_last_error() gives text.
  * No C++ exception crosses this boundary.
  *
