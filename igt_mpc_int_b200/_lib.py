@@ -70,7 +70,8 @@ EXPORTS = ("igt_version", "igt_default_params", "igt_create", "igt_destroy", "ig
            "igt_set_mlp", "igt_rollout_dev", "igt_rollout_host", "igt_eval_host", "igt_solve_dev",
            "igt_solve_host", "igt_launch_count", "igt_measure_fma_peak", "igt_mlp_value_host", "igt_set_option",
            "igt_episode_run_host", "igt_set_mlp_at", "igt_solve_ex_dev", "igt_solve_ex_host", "igt_eval_ex_host",
-           "igt_mlp_value_ex_host", "igt_episode_run_ex_host")
+           "igt_mlp_value_ex_host", "igt_episode_run_ex_host", "igt_row_count", "igt_solve_duals_ex_dev",
+           "igt_solve_duals_ex_host", "igt_solve_vjp_dev", "igt_solve_vjp_host")
 
 
 def load():
@@ -112,8 +113,14 @@ def load():
     lib.igt_eval_ex_host.argtypes = [vp, C.c_int] + [vp] * 11
     lib.igt_mlp_value_ex_host.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp, C.c_int]
     lib.igt_episode_run_ex_host.argtypes = [vp, C.c_int, C.c_int, C.c_int] + [vp] * 10
+    lib.igt_row_count.argtypes = [vp]
+    lib.igt_solve_duals_ex_dev.argtypes = [vp, C.c_int] + [vp] * 16 + [vp]
+    lib.igt_solve_duals_ex_host.argtypes = [vp, C.c_int] + [vp] * 16
+    lib.igt_solve_vjp_dev.argtypes = [vp, C.c_int] + [vp] * 17 + [vp]
+    lib.igt_solve_vjp_host.argtypes = [vp, C.c_int] + [vp] * 17
     for f in ("igt_set_mlp_at", "igt_solve_ex_dev", "igt_solve_ex_host", "igt_eval_ex_host", "igt_mlp_value_ex_host",
-              "igt_episode_run_ex_host"):
+              "igt_episode_run_ex_host", "igt_row_count", "igt_solve_duals_ex_dev", "igt_solve_duals_ex_host",
+              "igt_solve_vjp_dev", "igt_solve_vjp_host"):
         getattr(lib, f).restype = C.c_int
     for f in ("igt_default_params", "igt_create", "igt_set_mlp", "igt_rollout_dev", "igt_rollout_host",
               "igt_eval_host", "igt_solve_dev", "igt_solve_host"):

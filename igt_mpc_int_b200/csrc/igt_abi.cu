@@ -7,6 +7,7 @@
 //                         accumulation); replaces kinematic_bicycle_model_frenet.py:69-185
 //   rollout_euler_kernel  fp32 Cartesian Euler rollout + Jacobians; kinematic_bicycle_model.py:15-50
 //   eval_kernel           fp64 cost / max-row-violation of given controls; mpc.py:177-373
+//   vjp_kernel            fp64 vector-Jacobian product of a solve through its converged KKT system (sens.cuh)
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstdlib>
@@ -20,6 +21,7 @@
 
 #include "../../include/igt_mpc.h"
 #include "solver_core.cuh"
+#include "sens.cuh"
 #include "params_host.hpp"
 #include "mlp_tc.cuh"
 
@@ -62,8 +64,12 @@ __global__ void __launch_bounds__(128) guess_kernel(ProbIO io, long B, double *g
 #define IGT_RSTG 1     // row staging in the node phases of the plain throughput kernels (solver_core.cuh, Ws RSTG)
 #endif
 // BANK: gt_mpc with the handle's network bank, network io.net_idx[p] per problem (not with TC)
-template <typename T, bool TC, bool OBCA, bool COOP = false, bool BANK = false>
-__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type io, T *ws, long n_slots, long B, Sched sc,
+// DUALS: io is a DualsIO, and every problem also writes the final slack and multiplier of each row
+template <typename T, bool BANK, bool DUALS>
+using SolveIO = typename std::conditional<DUALS, DualsIO<typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type>,
+                                          typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type>::type;
+template <typename T, bool TC, bool OBCA, bool COOP = false, bool BANK = false, bool DUALS = false>
+__global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(SolveIO<T, BANK, DUALS> io, T *ws, long n_slots, long B, Sched sc,
                                                                const double *guess, T *mlp_scratch, int mlp_width,
                                                                MlpTcWeights wt, int quota, int cs)
 {
@@ -75,7 +81,7 @@ __global__ void __launch_bounds__(SOLVE_BLOCK, 1) solve_kernel(typename std::con
     constexpr bool RSTG = IGT_RSTG && !TC && !COOP;                 // (TC fills shared memory itself; with COOP the value term's
                                                                     //  weight reads need the L1 more: measured 120 -> 146 ms per batch)
     // dynamic shared memory: [cooperative value-term buffers (COOP)] [row staging (RSTG)]
-    solve_persistent<T, TC, 32, OBCA, COOP, RSTG, BANK>(P, io, ws, slot, B, sc, guess,
+    solve_persistent<T, TC, 32, OBCA, COOP, RSTG, BANK, DUALS>(P, io, ws, slot, B, sc, guess,
                             mlp_scratch ? mlp_scratch + slot * 12 * (long)mlp_width : nullptr, mlp_width, &tc, quota, cs, dyn_smem,
                             RSTG ? dyn_smem + (COOP ? mlp_coop_smem_bytes<T>(SOLVE_BLOCK) : 0) : nullptr);
     if (TC) mlp_tc_teardown(tc);
@@ -327,6 +333,18 @@ __global__ void __launch_bounds__(256, 1) mlp_coop_kernel(long B, const double *
     }
 }
 
+// VJP of a solve (sens.cuh), one problem per thread; ws: [sens_ws_size(N)][B] (element-major, so that a warp's 32
+// problems touch consecutive words); mlp_scratch: [B][2][6][mlp_width] (gt_mpc)
+template <bool BANK>
+__global__ void __launch_bounds__(128) vjp_kernel(SensIO io, long B, double *ws, double *mlp_scratch, int mlp_width, int cs)
+{
+    const long p = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= B) return;
+    const DevParams<double> &P = c_Pd[cs];
+    const SensWs w = { ws + p, B, P.N };
+    vjp_problem<BANK>(P, io, p, w, mlp_scratch ? mlp_scratch + p * 12 * (long)mlp_width : nullptr, mlp_width);
+}
+
 // dependent-free FMA chains: the CUDA-core roofline denominator that MEASURED_PEAKS.json lacks
 template <typename T>
 __global__ void __launch_bounds__(256) fma_peak_kernel(T *out, int iters)
@@ -360,6 +378,7 @@ struct igt_handle {
     void *mlp_scratch = nullptr; size_t mlp_scratch_bytes = 0;
     void *stage = nullptr; size_t stage_bytes = 0;     // device block of the *_host calls (see staged)
     void *guess = nullptr; size_t guess_bytes = 0;     // cold-start controls [B][N][2] + the work counter
+    void *sens = nullptr; size_t sens_bytes = 0;       // VJP scratch (vjp_kernel)
     int n_sm = 0;
     int smem_optin = 0;                // shared memory a block may opt in to (the gt_mpc latency path's limit)
     long long launches = 0;
@@ -530,28 +549,30 @@ static int staged(igt_handle *h, cudaStream_t st, Staged (&a)[n], Run &&run)
 // solve_kernel<T, TC, OBCA, COOP, BANK>, its cold-start kernel guess_kernel<T, OBCA> and, without TC, its latency
 // kernel solve_small_kernel<T, OBCA, COOP, BANK, GT>: these rows are the only instantiations of the three templates.
 // TC: tensor-core value term; COOP: the CTA-cooperative exact value term (f64, circle mode, every layer <= MLP_COOP_W);
-// BANK: network net_idx[p] of the handle's bank per problem; GT: gt_mpc (a value term at all).
-template <typename T_, bool OBCA_, bool TC_, bool COOP_, bool BANK_, bool GT_>
+// BANK: network net_idx[p] of the handle's bank per problem; GT: gt_mpc (a value term at all); DUALS: the row also
+// builds solve_kernel<..., DUALS = true>, the throughput kernel that exports every row's final slack and multiplier
+// (igt_solve_duals_*: f64 circle mode with the exact value term; these are the inputs of the VJP, sens.cuh).
+template <typename T_, bool OBCA_, bool TC_, bool COOP_, bool BANK_, bool GT_, bool DUALS_>
 struct Variant {
     using T = T_;
-    static constexpr bool OBCA = OBCA_, TC = TC_, COOP = COOP_, BANK = BANK_, GT = GT_;
+    static constexpr bool OBCA = OBCA_, TC = TC_, COOP = COOP_, BANK = BANK_, GT = GT_, DUALS = DUALS_;
 };
 template <typename... V> struct VariantList {};
 using Variants = VariantList<
-    //      T       OBCA   TC     COOP   BANK   GT
-    Variant<double, false, false, false, false, false>,     // 'mpc'
-    Variant<float,  false, false, false, false, false>,
-    Variant<double, true,  false, false, false, false>,
-    Variant<double, false, false, true,  false, true>,      // gt_mpc, one network
-    Variant<double, false, true,  false, false, true>,
-    Variant<float,  false, true,  false, false, true>,
-    Variant<double, false, false, false, false, true>,
-    Variant<double, true,  false, false, false, true>,
-    Variant<float,  false, false, false, false, true>,
-    Variant<double, false, false, true,  true,  true>,      // gt_mpc, network bank
-    Variant<double, false, false, false, true,  true>,
-    Variant<double, true,  false, false, true,  true>,
-    Variant<float,  false, false, false, true,  true>>;
+    //      T       OBCA   TC     COOP   BANK   GT     DUALS
+    Variant<double, false, false, false, false, false, true>,      // 'mpc'
+    Variant<float,  false, false, false, false, false, false>,
+    Variant<double, true,  false, false, false, false, false>,
+    Variant<double, false, false, true,  false, true,  true>,      // gt_mpc, one network
+    Variant<double, false, true,  false, false, true,  false>,
+    Variant<float,  false, true,  false, false, true,  false>,
+    Variant<double, false, false, false, false, true,  true>,
+    Variant<double, true,  false, false, false, true,  false>,
+    Variant<float,  false, false, false, false, true,  false>,
+    Variant<double, false, false, true,  true,  true,  true>,      // gt_mpc, network bank
+    Variant<double, false, false, false, true,  true,  true>,
+    Variant<double, true,  false, false, true,  true,  false>,
+    Variant<float,  false, false, false, true,  true,  false>>;
 
 // f(V()) for the row V with these flags (solve_dev_impl only asks for combinations that have a row)
 template <typename F, typename... V>
@@ -617,8 +638,11 @@ static typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type io_for(const 
     return r;
 }
 
-// Solve of checked arguments (device pointers) on `st`.
-static int solve_dev_impl(igt_handle *h, int B, const ProbIO &io, const int *net_idx, cudaStream_t st)
+// Solve of checked arguments (device pointers) on `st`.  slack / mult [B][M] (both or neither): a dual-exporting solve
+// (checked by check_duals), always on the throughput kernel: the latency kernel gives the same bits, so the small
+// batches it would take are exported from the throughput kernel without a latency twin of each dual-exporting row.
+static int solve_dev_impl(igt_handle *h, int B, const ProbIO &io, const int *net_idx, cudaStream_t st,
+                          double *slack = nullptr, double *mult = nullptr)
 {
     if (B == 0) return IGT_OK;
     int rc = begin_call(h, st);
@@ -648,7 +672,7 @@ static int solve_dev_impl(igt_handle *h, int B, const ProbIO &io, const int *net
         const size_t small_smem = (size_t)L.total * sizeof(T) + small_coop_bytes<T, V::COOP, V::BANK>();
         bool small = false;
         if constexpr (!V::TC) {
-            if (h->use_small && B <= h->n_sm) {
+            if (h->use_small && B <= h->n_sm && !slack) {
                 if constexpr (V::GT) {
                     static std::atomic<int> static_smem{ -1 };   // the latency kernel's static shared memory, read once
                     if (static_smem < 0) {
@@ -698,10 +722,22 @@ static int solve_dev_impl(igt_handle *h, int B, const ProbIO &io, const int *net
                 k<<<B, bs, small_smem, st>>>(ios, B, sc, guess, cs);
             }
         }
-        if (!small) {
-            const int smem = V::TC ? TC_SMEM_BYTES
-                           : V::COOP ? (V::BANK ? mlp_coop_bank_smem_bytes<T>(SOLVE_BLOCK) : mlp_coop_smem_bytes<T>(SOLVE_BLOCK))
-                           : IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * (int)sizeof(T) : 0;
+        const int smem = V::TC ? TC_SMEM_BYTES
+                       : V::COOP ? (V::BANK ? mlp_coop_bank_smem_bytes<T>(SOLVE_BLOCK) : mlp_coop_smem_bytes<T>(SOLVE_BLOCK))
+                       : IGT_RSTG ? RSTG_SLOTS * SOLVE_BLOCK * (int)sizeof(T) : 0;
+        if (slack) {
+            if constexpr (V::DUALS) {
+                SolveIO<T, V::BANK, true> iod;
+                static_cast<IO &>(iod) = iob;
+                iod.slack = slack; iod.mult = mult;
+                auto *k = solve_kernel<T, V::TC, V::OBCA, V::COOP, V::BANK, true>;
+                CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+                k<<<(int)(n_slots / bs), bs, smem, st>>>(iod, (T *)h->ws, n_slots, B, sc, guess, scratch, width, h->tc, quota, cs);
+            } else {
+                h->err = "igt_solve_duals: no dual-exporting solver for this combination";
+                return IGT_EINVAL;
+            }
+        } else if (!small) {
             auto *k = solve_kernel<T, V::TC, V::OBCA, V::COOP, V::BANK>;
             CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             k<<<(int)(n_slots / bs), bs, smem, st>>>(iob, (T *)h->ws, n_slots, B, sc, guess, scratch, width, h->tc, quota, cs);
@@ -775,6 +811,7 @@ void igt_destroy(igt_handle *h)
     if (h->mlp_scratch) cudaFree(h->mlp_scratch);
     if (h->stage) cudaFree(h->stage);
     if (h->guess) cudaFree(h->guess);
+    if (h->sens) cudaFree(h->sens);
     delete h;
 }
 
@@ -979,6 +1016,115 @@ int igt_solve_host(igt_handle *h, int B, const double *x0, const double *u_prev,
                    double *u, double *cost, double *viol, int *status, int *iters)
 {
     return igt_solve_ex_host(h, B, x0, u_prev, curv, obs_xy, obs_psi, nn_ctx, nullptr, u_init, x, u, cost, viol, status, iters);
+}
+
+int igt_row_count(const igt_handle *h) { return h ? row_total(h->prm.N, h->prm.n_cinf) : IGT_EINVAL; }
+
+// the further conditions of a dual-exporting solve (after check_solve)
+static int check_duals(igt_handle *h, const ProbIO &io, const double *slack, const double *mult)
+{
+    if (!slack || !mult) { h->err = "igt_solve_duals: null argument"; return IGT_EINVAL; }
+    if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_solve_duals: needs precision f64"; return IGT_EINVAL; }
+    if (io.obs_psi) { h->err = "igt_solve_duals: not in the OBCA collision mode (obs_psi)"; return IGT_EINVAL; }
+    if (io.ctx && h->use_tc) { h->err = "igt_solve_duals: not with the tensor-core value term (tensor_core_mlp = 1)"; return IGT_EINVAL; }
+    return IGT_OK;
+}
+
+int igt_solve_duals_ex_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                           const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                           const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters,
+                           double *slack, double *mult, void *stream)
+{
+    if (!h) return IGT_EINVAL;
+    const ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters, obs_psi };
+    std::lock_guard<std::mutex> lk(h->mu);
+    int rc = check_solve(h, B, io, net_idx, false);
+    if (!rc) rc = check_duals(h, io, slack, mult);
+    return rc ? rc : solve_dev_impl(h, B, io, net_idx, (cudaStream_t)stream, slack, mult);
+}
+
+int igt_solve_duals_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                            const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                            const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters,
+                            double *slack, double *mult)
+{
+    const ProbIO io = { x0, u_prev, curv, obs_xy, nn_ctx, u_init, x, u, cost, viol, status, iters, obs_psi };
+    return host_call(h, B, [&] { int rc = check_solve(h, B, io, net_idx, true); return rc ? rc : check_duals(h, io, slack, mult); },
+                     [&](cudaStream_t st) {
+        const size_t N = h->prm.N, nb = B, M = row_total(h->prm.N, h->prm.n_cinf);
+        ProbIO d = {};
+        const int *dnet;
+        double *dy, *ds;
+        Staged a[] = { input(x0, nb * 7, &d.x0), input(u_prev, nb * 2, &d.u_prev), input(curv, nb * 3, &d.curv),
+                       input(obs_xy, nb * (N + 1) * 2, &d.obs), input(nn_ctx, nb * 4, &d.ctx), input(u_init, nb * N * 2, &d.u_init),
+                       input(net_idx, nb, &dnet),
+                       output(x, nb * (N + 1) * 7, &d.x), output(u, nb * N * 2, &d.u), output(cost, nb, &d.cost), output(viol, nb, &d.viol),
+                       output(status, nb, &d.status), output(iters, nb, &d.iters), output(slack, nb * M, &dy), output(mult, nb * M, &ds) };
+        return staged(h, st, a, [&] { return solve_dev_impl(h, B, d, dnet, st, dy, ds); });
+    });
+}
+
+// arguments of igt_solve_vjp_dev / _host (host_idx: as in check_solve)
+static int check_vjp(igt_handle *h, int B, const SensIO &io, bool host_idx)
+{
+    if (B < 0 || !io.x0 || !io.u_prev || !io.curv || !io.obs || !io.u || !io.slack || !io.mult || !io.status || !io.gx0 ||
+        !io.gu_prev || !io.gobs || !io.ok) { h->err = "igt_solve_vjp: null argument"; return IGT_EINVAL; }
+    if (h->prm.precision != IGT_PREC_F64) { h->err = "igt_solve_vjp: needs precision f64"; return IGT_EINVAL; }
+    if (io.ctx && h->use_tc) { h->err = "igt_solve_vjp: not with the tensor-core value term (tensor_core_mlp = 1)"; return IGT_EINVAL; }
+    if (io.net_idx && !io.ctx) { h->err = "igt_solve_vjp: net_idx needs nn_ctx (gt_mpc)"; return IGT_EINVAL; }
+    if (io.net_idx && host_idx) { const int rc = check_net_idx(h, B, io.net_idx, "igt_solve_vjp"); if (rc) return rc; }
+    if (io.ctx && value_width(h, io.net_idx != nullptr) == 0) { h->err = "igt_solve_vjp: nn_ctx given but no network was loaded"; return IGT_ENOMLP; }
+    return IGT_OK;
+}
+
+static int vjp_dev_impl(igt_handle *h, int B, SensIO io, cudaStream_t st)
+{
+    if (B == 0) return IGT_OK;
+    int rc = begin_call(h, st), cs = 0;
+    if (rc) return rc;
+    const int width = value_width(h, io.net_idx != nullptr);
+    const size_t ws = (size_t)B * sens_ws_size(h->prm.N), scr = io.ctx ? (size_t)B * 12 * width : 0;
+    if ((rc = grow(h, &h->sens, &h->sens_bytes, (ws + scr) * sizeof(double), st))) return rc;
+    if ((rc = acquire_cslot(h, 1, st, &cs))) return rc;
+    io.nets = (const MlpNet<double> *)h->bank;
+    double *base = (double *)h->sens;
+    auto *k = io.net_idx ? vjp_kernel<true> : vjp_kernel<false>;
+    k<<<(B + 127) / 128, 128, 0, st>>>(io, B, base, io.ctx ? base + ws : nullptr, width, cs);
+    h->launches++;
+    CK(cudaGetLastError());
+    return end_call(h, st, 2);
+}
+
+int igt_solve_vjp_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv, const double *obs_xy,
+                      const double *nn_ctx, const int *net_idx, const double *u, const double *slack, const double *mult,
+                      const int *status, const double *gx, const double *gu, const double *gcost, double *gx0, double *gu_prev,
+                      double *gobs, int *ok, void *stream)
+{
+    if (!h) return IGT_EINVAL;
+    SensIO io = { x0, u_prev, curv, obs_xy, nn_ctx, net_idx, nullptr, u, slack, mult, status, gx, gu, gcost, gx0, gu_prev, gobs, ok };
+    std::lock_guard<std::mutex> lk(h->mu);
+    const int rc = check_vjp(h, B, io, false);
+    return rc ? rc : vjp_dev_impl(h, B, io, (cudaStream_t)stream);
+}
+
+int igt_solve_vjp_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv, const double *obs_xy,
+                       const double *nn_ctx, const int *net_idx, const double *u, const double *slack, const double *mult,
+                       const int *status, const double *gx, const double *gu, const double *gcost, double *gx0, double *gu_prev,
+                       double *gobs, int *ok)
+{
+    const SensIO io = { x0, u_prev, curv, obs_xy, nn_ctx, net_idx, nullptr, u, slack, mult, status, gx, gu, gcost, gx0, gu_prev, gobs, ok };
+    return host_call(h, B, [&] { return check_vjp(h, B, io, true); }, [&](cudaStream_t st) {
+        const size_t N = h->prm.N, nb = B, M = row_total(h->prm.N, h->prm.n_cinf);
+        SensIO d = {};
+        Staged a[] = { input(x0, nb * 7, &d.x0), input(u_prev, nb * 2, &d.u_prev), input(curv, nb * 3, &d.curv),
+                       input(obs_xy, nb * (N + 1) * 2, &d.obs), input(nn_ctx, nb * 4, &d.ctx), input(net_idx, nb, &d.net_idx),
+                       input(u, nb * N * 2, &d.u), input(slack, nb * M, &d.slack), input(mult, nb * M, &d.mult),
+                       input(status, nb, &d.status), input(gx, nb * (N + 1) * 7, &d.gx), input(gu, nb * N * 2, &d.gu),
+                       input(gcost, nb, &d.gcost),
+                       output(gx0, nb * 7, &d.gx0), output(gu_prev, nb * 2, &d.gu_prev), output(gobs, nb * (N + 1) * 2, &d.gobs),
+                       output(ok, nb, &d.ok) };
+        return staged(h, st, a, [&] { return vjp_dev_impl(h, B, d, st); });
+    });
 }
 
 int igt_eval_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,

@@ -252,6 +252,12 @@ struct ProbIONet : ProbIO {
 // (only for an io that is a ProbIONet<T>: the BANK code paths)
 template <typename T>
 IGT_HD const ProbIONet<T> &bank_io(const ProbIO &io) { return static_cast<const ProbIONet<T> &>(io); }
+// outputs of a dual-exporting solve (the DUALS throughput kernels): IO plus the final slack y and multiplier s of every
+// inequality row, [B][row_total(N, n_cinf)] each, rows in workspace order (row_off)
+template <typename IO>
+struct DualsIO : IO {
+    double *slack = nullptr, *mult = nullptr;
+};
 
 // ------------------------------------------------------------------ dynamics -----------
 IGT_HD void sincos_t(float x, float *s, float *c) { sincosf(x, s, c); }
@@ -324,8 +330,9 @@ struct StepK {
     T b0, b1, kv;
 };
 
-template <typename T>
-IGT_HD StepK<T> step_setup(const DevParams<T> &P, const T *z0, const T *u, const T *curv)
+// (PT: DevParams<T>, or DevParams<double> with the forward-mode Dual of sens.cuh as T)
+template <typename T, typename PT>
+IGT_HD StepK<T> step_setup(const PT &P, const T *z0, const T *u, const T *curv)
 {
     StepK<T> c;
     c.h = P.h; c.a = u[0];
@@ -405,8 +412,8 @@ enum { SX = 0, SY = 4, SS = 8, SEY = 13, SEP = 18, SPS = 23 };
 // sensitivities; the state arithmetic is the same expression for expression, so both variants
 // return bit-identical states (the solver relies on it: a trial point rolled out with or without
 // sensitivities is the same point).
-template <typename T, bool SENS>
-IGT_HD void rk4_core(const DevParams<T> &P, const T *z0, const T *u_in, const T *curv_in, T *zn, T *Sc)
+template <typename T, bool SENS, typename PT>
+IGT_HD void rk4_core(const PT &P, const T *z0, const T *u_in, const T *curv_in, T *zn, T *Sc)
 {
     const StepK<T> c = step_setup(P, z0, u_in, curv_in);
     const T h = c.h, hh = h * T(0.5), h6 = h / T(6), a = c.a;
@@ -1717,6 +1724,18 @@ struct Solver : SolverNet<T, BANK> {
         accept_trials(1);
     }
 
+    // slack and multiplier of every row of the returned iterate (buffer cur) to y[p][M], s[p][M]; NaN for a problem
+    // that was never solved (status 2, 7)
+    IGT_HD void write_duals(double *y, double *s, long p) const
+    {
+        const int M = w.L.M;
+        const bool none = status == 2 || (BANK && status == 7);
+        for (int r = 0; r < M; r++) {
+            y[p * M + r] = none ? NAN : double(w.Y(cur, r));
+            s[p * M + r] = none ? NAN : double(w.S(cur, r));
+        }
+    }
+
     // write the outputs of this problem (x, u, cost, max row violation in reference units)
     IGT_HD void write_out(const ProbIO &io, long p)
     {
@@ -1994,7 +2013,17 @@ __device__ int g_round_mx[512][4];       // per loop pass, max over CTA 0's thre
 // BANK: gt_mpc with the handle's network bank, each problem with network io.net_idx[p] (per-thread or, with COOP,
 // cooperative value term; not with TC).  STRIDE 1 is the latency kernel's single-problem workspace: one problem per CTA,
 // so a CTA-wide evaluation has at most n_alpha requests and the cooperative buffers are sized for COOP_CAP of them.
-template <typename T, bool TC, int STRIDE = 32, bool OBCA = false, bool COOP = false, bool RSTG = false, bool BANK = false>
+// the duals of problem p, for an io that is a DualsIO (the DUALS kernels)
+template <typename T, bool BANK, typename S>
+__device__ __forceinline__ void write_duals_io(const S &sv, const ProbIO &io, long p)
+{
+    const auto &d = static_cast<const DualsIO<typename std::conditional<BANK, ProbIONet<T>, ProbIO>::type> &>(io);
+    sv.write_duals(d.slack, d.mult, p);
+}
+
+// DUALS: io is a DualsIO; every finished problem also writes its final slacks and multipliers
+template <typename T, bool TC, int STRIDE = 32, bool OBCA = false, bool COOP = false, bool RSTG = false, bool BANK = false,
+          bool DUALS = false>
 __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const ProbIO &io, T *ws_base,
                                                  long slot, long B, const Sched &sc,
                                                  const double *guess, T *mlp_scratch, int mlp_width, MlpTcCtx *tc,
@@ -2043,6 +2072,7 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
                     fresh = true;
                 } else {
                     sv.write_out(io, p);
+                    if constexpr (DUALS) write_duals_io<T, BANK>(sv, io, p);
                 }
             }
         }
@@ -2153,7 +2183,11 @@ __device__ __forceinline__ void solve_persistent(const DevParams<T> &P, const Pr
             sv.accept_trials(n_spec < left ? n_spec : left, false);
         }
         IGT_TICK(8);
-        if (active && sv.done) { sv.write_out(io, p); active = false; }
+        if (active && sv.done) {
+            sv.write_out(io, p);
+            if constexpr (DUALS) write_duals_io<T, BANK>(sv, io, p);
+            active = false;
+        }
         IGT_TICK(10);
     }
 #ifdef IGT_PHASE_CLOCKS

@@ -155,11 +155,19 @@ class BatchSolver:
         return out
 
     # -- host-pointer calls (copies inside) ---------------------------------------------------
-    def solve_batch(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, obs_psi=None, net_idx=None):
+    @property
+    def n_rows(self):
+        """M: inequality rows per problem, the width of the slack / mult outputs (order: include/igt_mpc.h)"""
+        return int(self.lib.igt_row_count(self._h))
+
+    def solve_batch(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, obs_psi=None, net_idx=None,
+                    duals=False):
         """numpy in / numpy out.  Returns dict(x[B,N+1,7], u[B,N,2], cost, viol, status, iters).
         obs_psi[B,N+1] (obstacle heading forecast) selects the OBCA collision rows (mpc.py:211-221).
         net_idx[B] (with nn_ctx): the bank slot of each problem's value network; an index that names no loaded
-        network raises IgtError before anything runs."""
+        network raises IgtError before anything runs.
+        duals: also slack[B,M] and mult[B,M], every row's final slack and multiplier (igt_solve_duals_ex_host: f64,
+        circle rows, exact value term) -- the inputs of vjp()."""
         N = self.N
         x0 = _f64(x0)
         B = x0.shape[0]
@@ -171,6 +179,15 @@ class BatchSolver:
         if out is None:
             out = dict(x=np.empty((B, N + 1, 7)), u=np.empty((B, N, 2)), cost=np.empty(B), viol=np.empty(B),
                        status=np.empty(B, dtype=np.int32), iters=np.empty(B, dtype=np.int32))
+        if duals:
+            M = self.n_rows
+            out.setdefault("slack", np.empty((B, M))); out.setdefault("mult", np.empty((B, M)))
+            rc = self.lib.igt_solve_duals_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi),
+                                                  _hp(nn_ctx), _hp(_net_idx(net_idx, B)), _hp(u_init), _hp(out["x"]),
+                                                  _hp(out["u"]), _hp(out["cost"]), _hp(out["viol"]), _hp(out["status"]),
+                                                  _hp(out["iters"]), _hp(out["slack"]), _hp(out["mult"]))
+            self._check(rc, "igt_solve_duals_ex_host")
+            return out
         rc = self.lib.igt_solve_ex_host(self._h, B, _hp(x0), _hp(u_prev), _hp(curv), _hp(obs_xy), _hp(obs_psi), _hp(nn_ctx),
                                         _hp(_net_idx(net_idx, B)), _hp(u_init), _hp(out["x"]), _hp(out["u"]),
                                         _hp(out["cost"]), _hp(out["viol"]), _hp(out["status"]), _hp(out["iters"]))
@@ -212,10 +229,11 @@ class BatchSolver:
 
     # -- device-pointer call (torch tensors already in HBM; no copies, no sync) ---------------
     def solve_batch_device(self, x0, u_prev, curv, obs_xy, nn_ctx=None, u_init=None, out=None, stream=None, obs_psi=None,
-                           net_idx=None):
+                           net_idx=None, duals=False):
         """torch CUDA float64 tensors in / out; enqueues on the current torch stream.
         net_idx: int32 device tensor [B] of bank slots (with nn_ctx); checked in the kernel: a problem whose index
-        names no loaded network gets status 7 (STATUS_BAD_NET) and NaN outputs."""
+        names no loaded network gets status 7 (STATUS_BAD_NET) and NaN outputs.
+        duals: also slack[B,M] and mult[B,M] (see solve_batch)."""
         import torch
         N = self.N
         B = x0.shape[0]
@@ -245,10 +263,81 @@ class BatchSolver:
                 check(out[k], shp, dt, "out[%r]" % k)
         st = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
         p = lambda t: None if t is None else _vp(t.data_ptr())
+        if duals:
+            M = self.n_rows
+            for k in ("slack", "mult"):
+                if k not in out:
+                    out[k] = torch.empty((B, M), dtype=torch.float64, device=dev)
+                check(out[k], (B, M), torch.float64, "out[%r]" % k)
+            rc = self.lib.igt_solve_duals_ex_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx),
+                                                 p(net_idx), p(u_init), p(out["x"]), p(out["u"]), p(out["cost"]),
+                                                 p(out["viol"]), p(out["status"]), p(out["iters"]), p(out["slack"]),
+                                                 p(out["mult"]), _vp(st))
+            self._check(rc, "igt_solve_duals_ex_dev")
+            return out
         rc = self.lib.igt_solve_ex_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(obs_psi), p(nn_ctx), p(net_idx),
                                        p(u_init), p(out["x"]), p(out["u"]), p(out["cost"]), p(out["viol"]),
                                        p(out["status"]), p(out["iters"]), _vp(st))
         self._check(rc, "igt_solve_ex_dev")
+        return out
+
+    # -- gradients through the solve (csrc/sens.cuh) ---------------------------------------------
+    def vjp(self, x0, u_prev, curv, obs_xy, u, slack, mult, status, gx=None, gu=None, gcost=None, nn_ctx=None,
+            net_idx=None):
+        """Vector-Jacobian product of a solve through its converged KKT system (numpy in / out).
+        The solve's inputs and its outputs u, slack, mult, status (solve_batch(..., duals=True)); cotangents gx[B,N+1,7],
+        gu[B,N,2], gcost[B] on x, u, cost (None = zero).  Returns dict(gx0[B,7], gu_prev[B,2], gobs[B,N+1,2] (row 0 is
+        0: mpc.py:224 does not use it), ok[B] int32); a problem with ok = 0 (status != 0, or a stage Hessian that is not
+        positive definite) gets exact zeros."""
+        N = self.N
+        x0 = _f64(x0)
+        B = x0.shape[0]
+        M = self.n_rows
+        args = [_f64(x0, (B, 7)), _f64(u_prev, (B, 2)), _f64(curv, (B, 3)), _f64(obs_xy, (B, N + 1, 2)),
+                None if nn_ctx is None else _f64(nn_ctx, (B, 4))]
+        net = _net_idx(net_idx, B)
+        sol = [_f64(u, (B, N, 2)), _f64(slack, (B, M)), _f64(mult, (B, M))]
+        status = np.ascontiguousarray(status, dtype=np.int32)
+        if status.shape != (B,):
+            raise ValueError("status: expected shape (%d,)" % B)
+        cot = [None if gx is None else _f64(gx, (B, N + 1, 7)), None if gu is None else _f64(gu, (B, N, 2)),
+               None if gcost is None else _f64(gcost, (B,))]
+        out = dict(gx0=np.empty((B, 7)), gu_prev=np.empty((B, 2)), gobs=np.empty((B, N + 1, 2)), ok=np.empty(B, dtype=np.int32))
+        rc = self.lib.igt_solve_vjp_host(self._h, B, *[_hp(a) for a in args], _hp(net), *[_hp(a) for a in sol], _hp(status),
+                                         *[_hp(a) for a in cot], _hp(out["gx0"]), _hp(out["gu_prev"]), _hp(out["gobs"]),
+                                         _hp(out["ok"]))
+        self._check(rc, "igt_solve_vjp_host")
+        return out
+
+    def vjp_device(self, x0, u_prev, curv, obs_xy, u, slack, mult, status, gx=None, gu=None, gcost=None, nn_ctx=None,
+                   net_idx=None, stream=None):
+        """vjp() on torch CUDA tensors (float64; status and net_idx int32), enqueued on the current torch stream.
+        A device net_idx is checked in the kernel: a bad index gives ok = 0."""
+        import torch
+        N = self.N
+        B = x0.shape[0]
+        M = self.n_rows
+        dev = x0.device
+        shapes = (("x0", x0, (B, 7)), ("u_prev", u_prev, (B, 2)), ("curv", curv, (B, 3)), ("obs_xy", obs_xy, (B, N + 1, 2)),
+                  ("nn_ctx", nn_ctx, (B, 4)), ("u", u, (B, N, 2)), ("slack", slack, (B, M)), ("mult", mult, (B, M)),
+                  ("gx", gx, (B, N + 1, 7)), ("gu", gu, (B, N, 2)), ("gcost", gcost, (B,)), ("status", status, (B,)),
+                  ("net_idx", net_idx, (B,)))
+        for name, t, shp in shapes:
+            if t is None:
+                continue
+            dt = torch.int32 if name in ("status", "net_idx") else torch.float64
+            if not (t.is_cuda and t.device == dev and t.dtype == dt and t.is_contiguous() and tuple(t.shape) == shp):
+                raise ValueError("%s: expected a contiguous %s tensor of shape %s on %s" % (name, dt, shp, dev))
+        out = dict(gx0=torch.empty((B, 7), dtype=torch.float64, device=dev),
+                   gu_prev=torch.empty((B, 2), dtype=torch.float64, device=dev),
+                   gobs=torch.empty((B, N + 1, 2), dtype=torch.float64, device=dev),
+                   ok=torch.empty(B, dtype=torch.int32, device=dev))
+        st = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        p = lambda t: None if t is None else _vp(t.data_ptr())
+        rc = self.lib.igt_solve_vjp_dev(self._h, B, p(x0), p(u_prev), p(curv), p(obs_xy), p(nn_ctx), p(net_idx), p(u),
+                                        p(slack), p(mult), p(status), p(gx), p(gu), p(gcost), p(out["gx0"]),
+                                        p(out["gu_prev"]), p(out["gobs"]), p(out["ok"]), _vp(st))
+        self._check(rc, "igt_solve_vjp_dev")
         return out
 
 

@@ -195,6 +195,54 @@ int igt_solve_ex_host(igt_handle *h, int B, const double *x0, const double *u_pr
                       const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
                       const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters);
 
+/* Gradients through the solve (csrc/sens.cuh; DESIGN.md section 10).
+ *
+ * Inequality rows of one problem, M = igt_row_count(h) = 8 + 13 (N - 1) + n_cinf + 3 of them, in the solver's order:
+ *   node 0:            a <= a_max, a >= a_min, df <= df_max, df >= -df_max, the four rate rows (a - a_prev <= da_max,
+ *                      a_prev - a <= da_max, df - df_prev <= ddf_max, df_prev - df <= ddf_max)          -- 8 rows
+ *   node k = 1..N-1:   v <= v_max, v >= v_min, ey <= ey_lim, ey >= -ey_lim, collision (d_min - |p - o| <= 0), then
+ *                      the 8 input rows of node 0's order                                                -- 13 rows
+ *   after node N-1:    the n_cinf terminal-set rows C_inf.A [v_{N-1}; a_{N-1}] <= C_inf.b
+ *   node N:            ey <= ey_lim, ey >= -ey_lim, collision                                            -- 3 rows
+ * Each row is c(u) <= 0 with slack y = -c > 0 and multiplier s > 0 at the returned point. */
+int igt_row_count(const igt_handle *h);
+
+/* igt_solve_ex_* that also writes the final slack[B,M] and multiplier mult[B,M] of every row (the iterate the solve
+ * returned; NaN for a problem that was never solved, status 2 / 7).  x, u, cost, viol, status, iters are the same bits as
+ * igt_solve_ex_*.  Supported: precision f64, circle rows, 'mpc' and gt_mpc with one network or a bank, exact value term.
+ * IGT_EINVAL: obs_psi (OBCA: Gauss-Newton rows with a piecewise Hessian), precision f32, and gt_mpc with
+ * tensor_core_mlp = 1 (it perturbs the merit at 1e-7).  Always runs the throughput kernel, whatever latency_path says
+ * (the latency kernel gives the same bits). */
+int igt_solve_duals_ex_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                           const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                           const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters,
+                           double *slack, double *mult, void *stream);
+int igt_solve_duals_ex_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                            const double *obs_xy, const double *obs_psi, const double *nn_ctx, const int *net_idx,
+                            const double *u_init, double *x, double *u, double *cost, double *viol, int *status, int *iters,
+                            double *slack, double *mult);
+
+/* Vector-Jacobian product of a solve through its converged KKT system: the implicit function theorem on
+ * grad_u L = 0, c + y = 0, s_i y_i = const_i at the returned (u, y, s), theta = (x0, u_prev, obs_xy), the rollout
+ * included, with the exact Hessian of the Lagrangian (stage cost, value term, circle rows, second derivatives of the
+ * discrete RK4 step).  One problem per thread, fp64.
+ * In : the solve's inputs x0, u_prev, curv, obs_xy, nn_ctx (or NULL), net_idx (or NULL; as in igt_solve_ex_*) and its
+ *      outputs u[B,N,2], slack[B,M], mult[B,M], status[B] (igt_solve_duals_ex_*); cotangents gx[B,N+1,7], gu[B,N,2],
+ *      gcost[B] on x, u, cost, each may be NULL (zero).
+ * Out: gx0[B,7], gu_prev[B,2], gobs[B,N+1,2] (row 0 is 0: mpc.py:224 does not use it), ok[B] (int32).
+ *      ok = 0 with exact zero gradients (never NaN) when status != 0, when a slack or multiplier is not positive, when a
+ *      stage's Quu of the Riccati sweep is not positive definite (no regularisation), or when a result is not finite.
+ * Needs precision f64; gt_mpc with tensor_core_mlp = 1 is IGT_EINVAL.  A device net_idx naming no loaded slot gives
+ * ok = 0; the _host call checks the indices as igt_solve_ex_host does.  _dev and _host give the same bits. */
+int igt_solve_vjp_dev(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                      const double *obs_xy, const double *nn_ctx, const int *net_idx, const double *u, const double *slack,
+                      const double *mult, const int *status, const double *gx, const double *gu, const double *gcost,
+                      double *gx0, double *gu_prev, double *gobs, int *ok, void *stream);
+int igt_solve_vjp_host(igt_handle *h, int B, const double *x0, const double *u_prev, const double *curv,
+                       const double *obs_xy, const double *nn_ctx, const int *net_idx, const double *u, const double *slack,
+                       const double *mult, const int *status, const double *gx, const double *gu, const double *gcost,
+                       double *gx0, double *gu_prev, double *gobs, int *ok);
+
 /* Replaces the per-timestep loop of evaluate.py:451-564 ('mpc') / :198-312 ('gt_mpc') for E independent two-vehicle
  * episodes: `steps` closed-loop steps entirely on the device -- per step one kernel for the glue before the solve
  * (constant-acceleration forecast constant_acceleration_model.py:18-82, shared plans utils.py:339-352, filter_preds
